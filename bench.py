@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- closed-loop MPC steps/s on B200 (BASELINE.json metric), roofline and CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--horizon-steps T]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--horizon-steps T] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: BASELINE config 2 -- B = 1024 trajectories per GPU,
 spline / sinusoidal references, N = 20, Ts = 0.01, T = 1200 closed-loop MPC steps each (1.23 M MPC steps),
@@ -28,6 +28,7 @@ sys.path.insert(0, ROOT)
 
 N_HORIZON, TS = 20, 0.01
 METRIC = "closed-loop MPC steps/sec (batched QP solves/sec)"
+DUMP_BYTES = 64 * 10 ** 6       # --dump-outputs writes at most this much in all
 
 
 def make_workload(gen, B, traj_id0=0):
@@ -268,6 +269,23 @@ def measure_widened_rows(stream, hbm_peak):
     return out, launches
 
 
+def dump_outputs(out_dir, outputs, traj_id0):
+    """--dump-outputs: the device arrays one tg_closed_loop launch returned (dict name -> tensor [B, ...]) as <name>.npy in
+    float64, for a fixed, seeded sample of the B trajectories (all of them when they fit in DUMP_BYTES), plus their global ids
+    as traj_ids.npy.  The workload is a function of the trajectory ids alone, so two builds run with the same arguments can be
+    compared output for output."""
+    import torch
+    B = outputs["clean"].shape[0]
+    per_traj = 8 * (1 + sum(a[0].numel() for a in outputs.values()))
+    n = min(B, max(1, (DUMP_BYTES - 4096) // per_traj))            # 4096: room for the .npy headers
+    rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    idx = torch.from_numpy(rows).to(outputs["clean"].device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "traj_ids.npy"), (traj_id0 + rows).astype(np.float64))
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.index_select(0, idx).to(torch.float64).cpu().numpy())
+
+
 def run_gpu(args, rank, world, local_rank):
     import torch
     import trajectory_generation_b200 as tg
@@ -339,6 +357,7 @@ def run_gpu(args, rank, world, local_rank):
     barrier()
     kern_ms = [a.elapsed_time(b) for a, b in evs]
     gpu_launches = gen.kernel_launches() - launches0
+    timed_launches = gpu_launches                                    # counted by the library: one per timed step
     total_ms = float(np.sum(kern_ms))
     tm = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -373,6 +392,9 @@ def run_gpu(args, rank, world, local_rank):
     e2e_ok = bool(np.array_equal(out["clean"], d_clean.cpu().numpy()))
     gpu_launches += args.steps + 1
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:          # the e2e calls above use their own buffers: d_* still hold the last timed step
+        dump_outputs(args.dump_outputs, {"clean": d_clean, "noisy": d_noisy, "U": d_U, "status_counts": d_sc, "iters_total": d_it},
+                     traj_id0)
 
     # ---- p50 latency of one batched mpc_step call (device-resident, B problems, cold start): on the initial states of the
     # workload (large offsets: most problems have active rows) and on its states at mid-run (t = T/2: the typical case)
@@ -458,7 +480,7 @@ def run_gpu(args, rank, world, local_rank):
             "e2e": {"value": e2e_value, "unit": "MPC steps/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h),
                     "api": "ClosedLoopGenerator.generate (host arrays in, page-locked result arrays out; tg_closed_loop_host)",
                     "matches_resident_run": e2e_ok},
-            "gpu_launches": int(gpu_launches),
+            "gpu_launches": int(gpu_launches), "timed_launches": int(timed_launches),
             "parity": parity,
             # the binding roofline of this path is the fp64 CUDA-core FMA rate (SURVEY.md 8(d): neither HBM nor tensor cores;
             # the only dense contraction is a 40 x 40 SPD inversion per problem); algorithmic flops per MPC step by the
@@ -497,7 +519,12 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the side measurements of the widened rows (open-loop generators)")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity sample against the golden oracle loops (development runs)")
     ap.add_argument("--solver-opt", action="append", default=[], help="development: key=value override of a tg_config solver field")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="GPU path only: write the last timed step's outputs (clean, noisy, U, "
+                    "status_counts, iters_total of rank 0's trajectories; a fixed sample of them beyond 64 MB) as DIR/<name>.npy "
+                    "in float64")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs the GPU path (--impl b200) and at least one timed step (--steps >= 1)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -15,6 +15,9 @@ Parity status ("pinned" means checked against genuine reference outputs):
   (``oracle/refload.py``); ``tests/golden/make_golden.py`` ran it and committed the
   outputs under ``tests/golden/``; ``tests/test_oracle_vs_golden.py`` checks every
   restated function against them.
+* the consumer's loader (``KalmanNet/data_loader.py``, restated in ``oracle/dataset.py``)  --
+  restated from the cited lines; ``tests/golden/make_golden.py`` checks the restatement
+  against the reference's own loader whenever it regenerates the fixtures.
 * the QP (``MPC/mpc_6stati.py:180-262``: CVXPY problem -> OSQP)  -- PARITY UNPINNED.
   ``cvxpy`` and ``osqp`` are un-pinned third-party dependencies
   (``README.md:70``, ``MPC/README.md:84``: "pip install cvxpy osqp", no version) that are

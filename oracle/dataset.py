@@ -1,8 +1,10 @@
-"""Oracle: the generators' dataset shell -- x0 sampling, noisy/clean rows, CSV (fp64, pandas).
+"""Oracle: the generators' dataset shell -- x0 sampling, noisy/clean rows, CSV (fp64, pandas) -- and
+the consumer's loader.
 
 Test infrastructure -- see ``oracle/__init__.py``.  Restates generation_type2.py:162-220,309-322
 and generation_type1.py:139-158,260-339 (x0 ranges, clean/noisy DataFrames, CSV schema
-``t,X,Y,[phi],vx,vy,omega,d,delta,trajectory_id``; last row's d,delta = NaN -> empty field).
+``t,X,Y,[phi],vx,vy,omega,d,delta,trajectory_id``; last row's d,delta = NaN -> empty field), and
+KalmanNet/data_loader.py:5-109 (CSV pair -> shuffled float32 tensors).
 The sensor noise values come from ``oracle/philox.py`` (the B200 path's Philox stream) or, for
 pinning the shell itself against the reference, from NumPy PCG64 exactly as the reference does.
 """
@@ -63,3 +65,25 @@ def write_csv(clean_frames, noisy_frames, clean_path, noisy_path):
     """pd.concat(..., ignore_index=True).to_csv(index=False).  generation_type2.py:218,319-322."""
     pd.concat(clean_frames, ignore_index=True).to_csv(clean_path, index=False)
     pd.concat(noisy_frames, ignore_index=True).to_csv(noisy_path, index=False)
+
+
+def load_vehicle_dataset(noisy_path, clean_path, T_steps):
+    """KalmanNet/data_loader.py:5-109 (load_vehicle_dataset) on a clean / noisy CSV pair -> (y[n,5,T], u[n,2,T], x[n,6,T],
+    n_train): both files read with pandas' default parser (:22-23); n = number of distinct trajectory_id (:29); trajectory i =
+    the group with id i (:44-47, so ids must be 0..n-1), its first T_steps rows (:51-53); y = noisy X,Y,vx,vy,omega,
+    u = the noisy file's d,delta, x = clean X,Y,phi,vx,vy,omega (:14-18), float32, laid out [n, channel, T].  Trajectories
+    come in the loader's shuffled order (default_rng(42), :60-62), i.e. its train, validation and test tensors concatenated;
+    the first n_train = int(0.7 n) of them are the training split.  The loader's None returns on missing data
+    (:24-26, :54-56) are not restated."""
+    noisy, clean = pd.read_csv(noisy_path), pd.read_csv(clean_path)
+    n = clean["trajectory_id"].nunique()
+    gn, gc = noisy.groupby("trajectory_id"), clean.groupby("trajectory_id")
+    y, u, x = [], [], []
+    for i in range(n):
+        a, b = gn.get_group(i).iloc[:T_steps], gc.get_group(i).iloc[:T_steps]
+        y.append(a[["X", "Y", "vx", "vy", "omega"]].to_numpy().T)
+        u.append(a[["d", "delta"]].to_numpy().T)
+        x.append(b[["X", "Y", "phi", "vx", "vy", "omega"]].to_numpy().T)
+    perm = np.arange(n)
+    np.random.default_rng(42).shuffle(perm)
+    return tuple(np.stack(v).astype(np.float32)[perm] for v in (y, u, x)) + (int(0.7 * n),)

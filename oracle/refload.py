@@ -1,10 +1,9 @@
 """Oracle helper: import the reference's own importable Python (build container only).
 
-Test infrastructure -- see ``oracle/__init__.py``.  ``/root/reference`` exists only in
-the build container, never on the GPU box, so nothing at run time of the ``-m gpu``
-tests, ``smoke()`` or ``bench.py`` may call this; it is used by
-``tests/golden/make_golden.py`` (to produce the committed fixtures) and by CPU tests that
-``pytest.skip`` when the tree is absent.
+Test infrastructure -- see ``oracle/__init__.py``.  The reference tree (``REFERENCE_ROOT``)
+is not part of this repository, so no test, ``smoke()`` or ``bench.py`` calls this; only
+``tests/golden/make_golden.py`` does, to produce the committed fixtures and to check the
+oracle's loader restatement against the reference's own loader.
 
 ``MPC/mpc_6stati.py:6`` does ``import cvxpy as cp`` and uses ``cp.OSQP`` as a default
 argument (``:141``); neither cvxpy nor osqp is installed or installable offline, so a

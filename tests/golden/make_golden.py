@@ -191,6 +191,21 @@ def reference_estimator_fixtures():
     print("reference estimator fixtures written")
 
 
+def reference_loader_check():
+    """oracle/dataset.py's load_vehicle_dataset (which the tests read the package's CSVs with) against the reference's own
+    KalmanNet/data_loader.py on the committed gen2 CSVs: the same tensors in the same order, the same training split."""
+    dl = refload.load_data_loader()
+    from oracle import dataset as odata
+    c, n = os.path.join(HERE, "reference_gen2_clean.csv"), os.path.join(HERE, "reference_gen2_noisy.csv")
+    splits = dl.load_vehicle_dataset(n, c, T_steps=50)
+    mine = odata.load_vehicle_dataset(n, c, T_steps=50)
+    for k in range(3):                                                  # y, u, x
+        ref = np.concatenate([s[k].numpy() for s in splits])
+        assert ref.dtype == mine[k].dtype and np.array_equal(ref, mine[k], equal_nan=True), k
+    assert len(splits[0][0]) == mine[3]
+    print("loader restatement agrees with the reference loader")
+
+
 def oracle_qp_fixtures():
     rng = np.random.default_rng(7)
     cases = []
@@ -244,5 +259,6 @@ if __name__ == "__main__":
     reference_fixtures()
     reference_openloop_fixtures()
     reference_estimator_fixtures()
+    reference_loader_check()
     oracle_qp_fixtures()
     oracle_closed_loop_fixtures()

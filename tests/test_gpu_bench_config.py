@@ -66,3 +66,28 @@ def test_benchmarked_configuration_is_batch_and_shard_invariant(golden):
     small = gen.generate(x0[:n], u0[:n], sc.slice(0, n), 300)
     assert np.array_equal(big["clean"][:n], small["clean"]) and np.array_equal(big["U"][:n], small["U"])
     assert np.array_equal(big["noisy"][:n], small["noisy"])
+
+
+def test_dump_outputs_are_the_timed_launch_results(tmp_path):
+    """bench.py --dump-outputs at the benchmarked size: --steps sets the number of launches the library counts in the timed
+    window, and the dump is a seeded sample of the B = 1024 trajectories (all of them would exceed 64 MB) in float64,
+    bit-identical to the rows the public API returns for the same workload."""
+    import json
+    import subprocess
+    import sys
+    out = tmp_path / "dump"
+    p = subprocess.run([sys.executable, os.path.join(bench.ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-cpu", "--no-extra",
+                        "--no-parity", "--dump-outputs", str(out)], capture_output=True, text=True, check=True)
+    line = json.loads(p.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["timed_launches"] == 2 and line["warmup"] == 3
+    d = {f.stem: np.load(f) for f in out.glob("*.npy")}
+    assert set(d) == {"traj_ids", "clean", "noisy", "U", "status_counts", "iters_total"}
+    assert all(a.dtype == np.float64 for a in d.values())
+    assert sum(f.stat().st_size for f in out.glob("*.npy")) <= bench.DUMP_BYTES
+    ids = d["traj_ids"].astype(np.int64)
+    assert 32 <= len(ids) < 1024 and (np.diff(ids) > 0).all() and ids[-1] < 1024
+    gen = tg.ClosedLoopGenerator(**bench.GEN_KW)
+    x0, u0, sc = bench.make_workload(gen, 1024)
+    ref = gen.generate(x0, u0, sc, 1200)
+    for k in ("clean", "noisy", "U", "status_counts", "iters_total"):
+        assert np.array_equal(d[k], ref[k][ids].astype(np.float64)), k

@@ -64,22 +64,19 @@ def test_config3_mixed_references_generator_plant_csv_and_loader(tmp_path):
         Xo, Uo, st, _ = ompc.closed_loop(x0[i], u0[i], 25, Ts, 20, path_kind=kind, path_prm=tuple(sc.spec["path"][i]), spline=spline,
                                          vref_kind=R.VREF_RAMP, vref_prm=(0.8, 2.0, 2.0), vref_advance=True, plant=dyn.PLANT_GEN2)
         assert np.abs(res["clean"][i, :26] - Xo).max() < 1e-3 and np.abs(res["U"][i, :25] - Uo).max() < 1e-3
-    # dataset files through the native writer, read back through the reference's own loader when it is mounted
+    # dataset files through the native writer, read back through the loader (oracle/dataset.py restates KalmanNet/data_loader.py)
     tg.write_csv(res, Ts, tmp_path / "clean.csv", tmp_path / "noisy.csv")
     import pandas as pd
     c = pd.read_csv(tmp_path / "clean.csv", float_precision="round_trip")
     assert list(c.columns) == tg.CLEAN_COLS and len(c) == B * (T + 1)
     np.testing.assert_array_equal(c[["X", "Y", "phi", "vx", "vy", "omega"]].values.reshape(B, T + 1, 6), res["clean"])   # text round-trips exactly
-    from oracle import refload
-    if refload.available():
-        dl = refload.load_data_loader()
-        tr, va, te = dl.load_vehicle_dataset(str(tmp_path / "noisy.csv"), str(tmp_path / "clean.csv"), T_steps=T)
-        y, u, x = tg.to_loader_tensors(res, T)
-        perm = np.arange(B); np.random.default_rng(42).shuffle(perm)
-        allx = np.concatenate([tr[2].numpy(), va[2].numpy(), te[2].numpy()])
-        allu = np.concatenate([tr[1].numpy(), va[1].numpy(), te[1].numpy()])
-        np.testing.assert_array_equal(allx, x[perm]); np.testing.assert_array_equal(allu, u[perm])
-        assert tr[0].shape == (int(B * 0.7), 5, T)
+    from oracle import dataset as odata
+    ally, allu, allx, n_train = odata.load_vehicle_dataset(str(tmp_path / "noisy.csv"), str(tmp_path / "clean.csv"), T_steps=T)
+    y, u, x = tg.to_loader_tensors(res, T)
+    perm = np.arange(B); np.random.default_rng(42).shuffle(perm)
+    np.testing.assert_array_equal(allx, x[perm]); np.testing.assert_array_equal(allu, u[perm])
+    np.testing.assert_array_equal(ally, y[perm])
+    assert n_train == int(B * 0.7) and ally.shape == (B, 5, T)
 
 
 def _oracle_hard_loop(x0, u0, T, Ts, N):

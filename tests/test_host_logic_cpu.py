@@ -58,21 +58,30 @@ def test_native_float_formatting_equals_python_repr(tmp_path):
 
 
 def test_loader_tensors_match_reference_loader(tmp_path):
+    """the reference's rows written by the package's writer, read back by the loader (oracle/dataset.py's restatement of
+    KalmanNet/data_loader.py), give the tensors to_loader_tensors hands over without the CSV round trip."""
+    from oracle import dataset as odata
     res = _reference_rows()
     tg.write_csv(res, 0.01, tmp_path / "c.csv", tmp_path / "n.csv")
     y, u, x = tg.to_loader_tensors(res, 50)
     assert y.shape == (3, 5, 50) and u.shape == (3, 2, 50) and x.shape == (3, 6, 50) and y.dtype == np.float32
-    from oracle import refload
-    if not refload.available():
-        pytest.skip("reference tree not mounted")
-    dl = refload.load_data_loader()
-    tr, va, te = dl.load_vehicle_dataset(str(tmp_path / "n.csv"), str(tmp_path / "c.csv"), T_steps=50)
-    allx = np.concatenate([tr[2].numpy(), va[2].numpy(), te[2].numpy()])
-    ally = np.concatenate([tr[0].numpy(), va[0].numpy(), te[0].numpy()])
+    ally, allu, allx, n_train = odata.load_vehicle_dataset(str(tmp_path / "n.csv"), str(tmp_path / "c.csv"), T_steps=50)
     perm = np.arange(3); np.random.default_rng(42).shuffle(perm)      # KalmanNet/data_loader.py:60-62
     np.testing.assert_array_equal(allx, x[perm])
     np.testing.assert_array_equal(ally, y[perm])
-    assert not np.isnan(allx).any()
+    np.testing.assert_array_equal(allu, u[perm])
+    assert n_train == 2 and not np.isnan(allx).any()
+
+
+@pytest.mark.parametrize("args", [["--impl", "reference"], ["--steps", "0"]])
+def test_bench_refuses_dump_outputs_without_a_timed_gpu_step(tmp_path, args):
+    """--dump-outputs writes the timed GPU launch's results: with the CPU arm or no timed step there is nothing to write."""
+    import subprocess
+    import sys
+    from conftest import ROOT
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "d")] + args,
+                       capture_output=True, text=True)
+    assert p.returncode == 2 and "--dump-outputs needs" in p.stderr and not (tmp_path / "d").exists()
 
 
 def test_sample_x0_is_the_reference_draw():
