@@ -17,14 +17,11 @@
  * thread-safe; use one handle per thread/stream.
  *
  * Environment variables read by the library (development / measurement knobs; none is needed in production and none changes
- * results beyond rounding -- the GPU tests pin that for TRAJGEN_PPC and TRAJGEN_HOST_OUTPUT):
- *   TRAJGEN_PPC=<p>            problems per CTA of the fused kernels (default: chosen per launch, 1-4); read by tg_create
- *   TRAJGEN_GRID=<g>           cap on the number of CTAs of a fused launch (default: resident CTAs x SMs); read per launch
- *   TRAJGEN_SHAPE=<W>,<S>      warps per problem and register-tile slots per thread (must fit the horizon); read by tg_create
- *   TRAJGEN_DYNAMIC_N=1        use the run-time-horizon kernel where a compile-time-horizon instance (N = 20) exists
+ * results beyond rounding -- the GPU tests pin that for TRAJGEN_PPC).  tg_create reads them: a handle keeps what they were
+ * when it was created.
+ *   TRAJGEN_PPC=<p>            problems per CTA of the fused kernels (default: chosen per launch, 1-4)
+ *   TRAJGEN_DYNAMIC_N=1        use the run-time-horizon kernel where a compile-time-horizon instance (N = 10, 20, 40, 50) exists
  *   TRAJGEN_NO_TYRE_TABLE=1    evaluate the tyre curve / slip-angle atan with libdevice instead of the handle's tables
- *   TRAJGEN_HOST_OUTPUT=staged tg_closed_loop_host: stage the rows through device memory even when the caller's buffers are
- *                              page-locked (default: the kernel stores straight into page-locked result buffers)
  *   TRAJGEN_LIB=<path>         (Python layer only) load this shared library instead of the in-tree libtrajgen.so
  */
 #ifndef TRAJGEN_H

@@ -301,3 +301,24 @@ def test_state_row_instances_ignore_the_problems_per_cta_knob(monkeypatch):
     assert np.array_equal(ref["status_counts"], dyn_["status_counts"])
     np.testing.assert_allclose(ref["clean"], dyn_["clean"], atol=1e-6)      # different instruction order, same algorithm
     np.testing.assert_allclose(ref["U"], dyn_["U"], atol=1e-6)
+
+
+def test_kernel_instances_are_fixed_when_the_handle_is_created(monkeypatch):
+    """tg_create chooses a handle's kernel instances once: TRAJGEN_DYNAMIC_N set after the handles exist must not move them
+    to the run-time-horizon instances.  The batch is large enough for several problems per CTA, whose shared memory
+    (4 x 25 KB at N = 20) needs the opt-in that tg_create gives the chosen instances."""
+    B, T = 600, 30
+    x0 = tg.sample_x0(B, seed=13); x0[:, 1:3] = 0.0; x0[:, 3] += 0.4
+    u0 = np.stack([tg.d_steady_state(x0[:, 3]), np.zeros(B)], 1)
+    sc = tg.Scenarios(B); sc.set_sine(slice(0, B, 2), A=0.4, k=0.7)
+    monkeypatch.delenv("TRAJGEN_DYNAMIC_N", raising=False)
+    gen = tg.ClosedLoopGenerator(N=20, Ts=0.01, plant=tg.PLANT_GEN1)
+    ctl = tg.BatchedMPC(N=20, Ts=0.01)                          # warm start off: repeated calls are independent
+    pr, vr = gen.ref_window(x0, sc)
+    loop0, step0 = gen.generate(x0, u0, sc, T), ctl.step(x0, u0, pr, vr)
+    monkeypatch.setenv("TRAJGEN_DYNAMIC_N", "1")
+    loop1, step1 = gen.generate(x0, u0, sc, T), ctl.step(x0, u0, pr, vr)
+    for k in ("clean", "noisy", "U", "status_counts", "iters_total"):
+        np.testing.assert_array_equal(loop1[k], loop0[k], err_msg=k)
+    for k in step0:
+        np.testing.assert_array_equal(step1[k], step0[k], err_msg=k)

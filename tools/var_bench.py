@@ -1,15 +1,14 @@
-"""Development: time bench.py for library variants (tools/_var/*.so via TRAJGEN_LIB), kernel shapes (TRAJGEN_SHAPE = W,S) and
-problems per CTA (TRAJGEN_PPC).  usage: python tools/var_bench.py lib:shape:ppc:batch[:extra-env=val] ..."""
+"""Development: time bench.py for library variants (tools/_var/*.so via TRAJGEN_LIB) and problems per CTA (TRAJGEN_PPC).
+usage: python tools/var_bench.py lib:ppc:batch[:extra-env=val] ..."""
 import json, os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for spec in sys.argv[1:]:
     f = spec.split(":")
-    lib, shape, ppc, batch = f[0], f[1], f[2], f[3]
+    lib, ppc, batch = f[0], f[1], f[2]
     env = dict(os.environ)
     if lib: env["TRAJGEN_LIB"] = os.path.join(ROOT, "tools", "_var", lib)
-    if shape: env["TRAJGEN_SHAPE"] = shape
     if ppc: env["TRAJGEN_PPC"] = ppc
-    for kv in f[4:]:
+    for kv in f[3:]:
         k, v = kv.split("="); env[k] = v
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--no-cpu", "--no-extra", "--batch", batch, "--steps", "3"],
                        env=env, capture_output=True, text=True)

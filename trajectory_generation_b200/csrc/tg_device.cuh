@@ -47,21 +47,13 @@ enum { P_Cm1 = 0, P_Cm2, P_Cr0, P_Cr2, P_Br, P_Cr, P_Dr, P_Bf, P_Cf, P_Df, P_m, 
 
 __device__ __forceinline__ double tg_clamp(double v, double lo, double hi) { return fmin(fmax(v, lo), hi); }
 
-// One copy of each fp64 transcendental per kernel: the libdevice bodies are 120-350 SASS instructions each, and
-// the step body calls them from eight places; inlining every call made the per-step instruction footprint
-// several times the 32 KB L1.5 instruction cache (ncu: stall_no_instruction 3.6 cycles per issue).
-#ifndef TG_NOINLINE_MATH
-#define TG_NOINLINE_MATH 0
-#endif
-#if TG_NOINLINE_MATH
-#define TG_MATH_ATTR __noinline__
-#else
-#define TG_MATH_ATTR __forceinline__
-#endif
-__device__ TG_MATH_ATTR double2 tg_sincos2(double x) { double s_, c_; sincos(x, &s_, &c_); return make_double2(s_, c_); }
-__device__ TG_MATH_ATTR double tg_atan2(double y, double x) { return atan2(y, x); }
-__device__ TG_MATH_ATTR double tg_atan(double x) { return atan(x); }
-__device__ TG_MATH_ATTR double tg_sin(double x) { return sin(x); }
+// The fp64 transcendentals are inlined at every call.  One out-of-line copy of each per kernel shrinks the step from 11.1 k to
+// 9.3 k SASS instructions but measured 2.3 % slower (DESIGN.md section 8): with the problems of a CTA walking the code
+// together, instruction fetch no longer limits the step.
+__device__ __forceinline__ double2 tg_sincos2(double x) { double s_, c_; sincos(x, &s_, &c_); return make_double2(s_, c_); }
+__device__ __forceinline__ double tg_atan2(double y, double x) { return atan2(y, x); }
+__device__ __forceinline__ double tg_atan(double x) { return atan(x); }
+__device__ __forceinline__ double tg_sin(double x) { return sin(x); }
 __device__ __forceinline__ void TG_SINCOS(double x_, double &s_, double &c_) { const double2 r_ = tg_sincos2(x_); s_ = r_.x; c_ = r_.y; }
 
 // ------------------------------------------------------------------------------------------------

@@ -61,20 +61,17 @@ struct LoopArgs {
 // block (and, for W > 1, its own named barrier).  Problems of a CTA are re-aligned at every step boundary (barrier 15) so that
 // they fetch the same instruction lines at the same time (the step body is ~100 KB of mostly straight-line code).
 #define TW_CTA_THREADS 512
-// register budget: S = 2 tiles take 64 registers -> 128-register kernels; S = 1 tiles take 32 -> TW_REGS_S1 registers
-#ifndef TW_REGS_S1
-#define TW_REGS_S1 128
-#endif
-#define TW_REGS(S) ((S) == 1 ? TW_REGS_S1 : 128)
-// shapes that have a single-problem-per-CTA instance (see tw_mpc_step_kernel): the one- and two-warp kernels, where four CTAs
-// per SM would leave most of the register file and shared memory unused
-#define TW_HAS_P1(W, NC, HS) ((W) <= 2 && ((NC) == 0 || (HS)))
+// register budget: 128 per thread on every shape (the tile takes 32 of them with S = 1, 64 with S = 2).  The kernels state it
+// next to __launch_bounds__, so that ptxas gets both .maxntid and .maxnreg (without .maxntid the single-problem instances
+// compile to different code, without .maxnreg all of them do); nvcc accepts the two qualifiers together only with a value
+// that depends on a template parameter, hence the function template.
+template <int S> constexpr int tw_regs() { return 128; }
 
 // P1 = true: the single-problem-per-CTA instance.  Its only barrier id is the constant 1, so the kernel is built with 2
 // hardware barriers instead of 16 (a barrier id held in a register makes ptxas reserve all 16, and an SM has 64: four
 // resident CTAs at most, whatever the registers and the shared memory would allow).
 template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0)>
-__global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(TW_REGS(S))
+__global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(tw_regs<S>())
 tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLayout L, const __grid_constant__ StepArgs a)
 {
     extern __shared__ __align__(16) double sm_all[];
@@ -171,7 +168,7 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
 }
 
 template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0)>
-__global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(TW_REGS(S))
+__global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(tw_regs<S>())
 tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLayout L, const __grid_constant__ LoopArgs a)
 {
     extern __shared__ __align__(16) double sm_all[];
@@ -406,6 +403,15 @@ static double build_atan_table(double *tab /*[TG_ATAN_ROWS][NC]*/)
     return build_cheb_table(f, df, -(long double)TG_ATAN_T0, (long double)TG_ATAN_T0, TG_ATAN_NI, tab, nullptr);
 }
 
+// the warp-per-problem kernel instances of a handle: several problems per CTA, and P1 (one problem per CTA); null where the
+// instance is not compiled
+typedef void (*TwStepKernel)(DevCfg, WLayout, StepArgs);
+typedef void (*TwLoopKernel)(DevCfg, WLayout, LoopArgs);
+struct TwKernels {
+    TwStepKernel step, step_p1;
+    TwLoopKernel loop, loop_p1;
+};
+
 struct tg_handle {
     tg_config cfg;
     DevCfg dc;
@@ -413,6 +419,7 @@ struct tg_handle {
     int ppc_max, ppc_env;     // closed-loop kernel: most problems per CTA that fit / TRAJGEN_PPC override (0 = automatic)
     // warp-per-problem kernels (tw_solver.cuh): W warps per problem, S tile blocks per thread
     int W, S;
+    TwKernels kern;
     WLayout WL;
     WLayout Lref;             // layout of the reference-window tap kernel (no state rows, one warp)
     size_t smem_optin;
@@ -430,13 +437,6 @@ struct tg_handle {
 
 static bool pick_tw_shape(int N, int &W, int &S)
 {
-    if (const char *e = getenv("TRAJGEN_SHAPE")) {   // development knob: "W,S" (must fit the horizon)
-        int w = 0, s_ = 0;
-        if (sscanf(e, "%d,%d", &w, &s_) == 2 && w >= 1 && s_ >= 1) {
-            const int nb = (2 * N + 3) / 4;
-            if (nb * (nb + 1) / 2 <= 32 * w * s_ && N <= 32 * w && 2 * N <= 64 * w) { W = w; S = s_; return true; }
-        }
-    }
     if (N <= 14) { W = 1; S = 1; }          // 28 blocks on one warp
     else if (N <= 20) { W = 2; S = 1; }     // 55 blocks on two warps
     else if (N <= 30) { W = 4; S = 1; }     // 120 blocks
@@ -453,42 +453,83 @@ static bool tw_standard_controller(const DevCfg &d)
 {
     return d.model == TG_MODEL_MPC && d.jacobian == TG_JAC_ANALYTIC && d.tyre_tab && d.atan_tab;
 }
-template <typename F>
-static int dispatch_tw(int W, int S, const DevCfg &d, F &&f)
+// the kernels of one (W, S, NC, HS).  Single-problem-per-CTA instances exist for the one- and two-warp shapes, where four CTAs
+// per SM would leave most of the register file and shared memory unused, except for a compile-time horizon without state-bound
+// rows.  A compile-time horizon with state-bound rows on those shapes has only that instance (problems with state-bound rows
+// always run one per CTA, choose_tw_ppc).
+template <int W, int S, int NC, bool HS>
+static TwKernels tw_instance()
 {
-    using std::integral_constant;
-    typedef integral_constant<bool, false> no_rows;
-    typedef integral_constant<bool, true> rows;
-    const int N = d.N;
-    if (tw_standard_controller(d) && !getenv("TRAJGEN_DYNAMIC_N")) {   // mpc_step's default horizon (20), MPC/main.py's (40), BASELINE config 4's (10, 50)
-        if (d.ms == 0) {
-            if (W == 2 && S == 1 && N == 20) return f(integral_constant<int, 2>(), integral_constant<int, 1>(), integral_constant<int, 20>(), no_rows());
-#ifndef TG_DEV_SHAPES_ONLY
-            if (W == 1 && S == 1 && N == 10) return f(integral_constant<int, 1>(), integral_constant<int, 1>(), integral_constant<int, 10>(), no_rows());
-            if (W == 8 && S == 1 && N == 40) return f(integral_constant<int, 8>(), integral_constant<int, 1>(), integral_constant<int, 40>(), no_rows());
-            if (W == 8 && S == 2 && N == 50) return f(integral_constant<int, 8>(), integral_constant<int, 2>(), integral_constant<int, 50>(), no_rows());
-#endif
-        } else {
-            if (W == 2 && S == 1 && N == 20) return f(integral_constant<int, 2>(), integral_constant<int, 1>(), integral_constant<int, 20>(), rows());
-#ifndef TG_DEV_SHAPES_ONLY
-            if (W == 1 && S == 1 && N == 10) return f(integral_constant<int, 1>(), integral_constant<int, 1>(), integral_constant<int, 10>(), rows());
-            if (W == 8 && S == 2 && N == 50) return f(integral_constant<int, 8>(), integral_constant<int, 2>(), integral_constant<int, 50>(), rows());
-#endif
-        }
+    TwKernels k = {};
+    if constexpr (!(HS && NC > 0 && W <= 2)) {
+        k.step = tw_mpc_step_kernel<W, S, NC, false, HS>;
+        k.loop = tw_closed_loop_kernel<W, S, NC, false, HS>;
     }
-    if (W == 1 && S == 1) return f(integral_constant<int, 1>(), integral_constant<int, 1>(), integral_constant<int, 0>(), rows());
-    if (W == 2 && S == 1) return f(integral_constant<int, 2>(), integral_constant<int, 1>(), integral_constant<int, 0>(), rows());
-#ifndef TG_DEV_SHAPES_ONLY
-    if (W == 4 && S == 1) return f(integral_constant<int, 4>(), integral_constant<int, 1>(), integral_constant<int, 0>(), rows());
-    if (W == 8 && S == 1) return f(integral_constant<int, 8>(), integral_constant<int, 1>(), integral_constant<int, 0>(), rows());
-    if (W == 8 && S == 2) return f(integral_constant<int, 8>(), integral_constant<int, 2>(), integral_constant<int, 0>(), rows());
-#endif
-    return fail(TG_ERR_UNSUPPORTED, "no kernel shape for this horizon");
+    if constexpr (W <= 2 && (NC == 0 || HS)) {
+        k.step_p1 = tw_mpc_step_kernel<W, S, NC, true, HS>;
+        k.loop_p1 = tw_closed_loop_kernel<W, S, NC, true, HS>;
+    }
+    return k;
 }
-// instances that exist only in their single-problem-per-CTA form: compile-time horizon + state-bound rows on one or two warps
-// (problems with state-bound rows always run one per CTA, choose_tw_ppc)
-#define TW_P1_ONLY(W, NC, HS) ((HS) && (NC) > 0 && (W) <= 2)
+// every compiled instance.  fixed_n selects the compile-time-horizon instances where one exists: mpc_step's default horizon
+// (20), MPC/main.py's (40), BASELINE config 4's (10, 50).  No instance: every pointer null.
+static TwKernels tw_kernels(int W, int S, int N, int ms, bool fixed_n)
+{
+    if (fixed_n && ms == 0) {
+        if (W == 2 && S == 1 && N == 20) return tw_instance<2, 1, 20, false>();
+        if (W == 1 && S == 1 && N == 10) return tw_instance<1, 1, 10, false>();
+        if (W == 8 && S == 1 && N == 40) return tw_instance<8, 1, 40, false>();
+        if (W == 8 && S == 2 && N == 50) return tw_instance<8, 2, 50, false>();
+    }
+    if (fixed_n && ms > 0) {
+        if (W == 2 && S == 1 && N == 20) return tw_instance<2, 1, 20, true>();
+        if (W == 1 && S == 1 && N == 10) return tw_instance<1, 1, 10, true>();
+        if (W == 8 && S == 2 && N == 50) return tw_instance<8, 2, 50, true>();
+    }
+    if (W == 1 && S == 1) return tw_instance<1, 1, 0, true>();
+    if (W == 2 && S == 1) return tw_instance<2, 1, 0, true>();
+    if (W == 4 && S == 1) return tw_instance<4, 1, 0, true>();
+    if (W == 8 && S == 1) return tw_instance<8, 1, 0, true>();
+    if (W == 8 && S == 2) return tw_instance<8, 2, 0, true>();
+    return TwKernels{};
+}
 static size_t tw_stride(const tg_handle *h) { return (((size_t)h->WL.total + 1) & ~(size_t)1) * sizeof(double); }
+
+// warp-per-problem kernels: problems per CTA.  Resident problems per SM are bounded by registers (512 threads x 128) and
+// shared memory either way; larger CTAs share more instruction fetches, smaller ones spread a small batch over more SMs.
+static int choose_tw_ppc(const tg_handle *h, int B)
+{
+    if (h->ppc_env) return h->ppc_env;
+    // problems with state-bound rows have long, unequal solves (tens to hundreds of ADMM iterations): free-running
+    // single-problem CTAs beat problems that wait for one another at every step boundary
+    if (h->dc.ms > 0) return 1;
+    // measured at N = 20 (two warps per problem): 4 problems per CTA 2.65e7 steps/s (B = 2368), 8 per CTA 2.37e7 (B = 4736),
+    // 2 per CTA 2.24e7 and 1 per CTA 1.43e7 (B = 1024): sharing instruction fetches matters, waiting for 7 neighbours costs more
+    int p = h->ppc_max < 4 ? h->ppc_max : 4;
+    while (p > 1 && (B + p - 1) / p < h->num_sms) p >>= 1;   // every SM gets a CTA before CTAs get wider
+    return p < 1 ? 1 : p;
+}
+
+// the single-problem instance where there is no other or where one problem per CTA is chosen, else `multi` with
+// choose_tw_ppc problems per CTA
+template <typename Args>
+static int launch_tw(tg_handle *h, void (*multi)(DevCfg, WLayout, Args), void (*p1)(DevCfg, WLayout, Args), Args &a)
+{
+    int ppc = choose_tw_ppc(h, a.B);
+    void (*kern)(DevCfg, WLayout, Args) = multi;
+    if (p1 && (!multi || ppc == 1)) { kern = p1; ppc = 1; }
+    a.ppc = ppc;
+    const int threads = 32 * h->W * ppc;
+    const size_t smem = (size_t)ppc * tw_stride(h);
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+    if (per_sm < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
+    const int cap = per_sm * h->num_sms, ctas = (a.B + ppc - 1) / ppc;
+    kern<<<ctas < cap ? ctas : cap, threads, smem, h->stream>>>(h->dc, h->WL, a);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    return TG_OK;
+}
 
 extern "C" {
 
@@ -596,30 +637,18 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
         if (h->W > 1 && h->ppc_max > 14) h->ppc_max = 14;                  // named barriers 1..14 + the step barrier 15
         while (h->ppc_max > 1 && (size_t)h->ppc_max * stride > h->smem_optin) h->ppc_max -= 1;
         if (const char *e = getenv("TRAJGEN_PPC")) { const int v = atoi(e); if (v >= 1 && v <= h->ppc_max) h->ppc_env = v; }
+        h->kern = tw_kernels(h->W, h->S, d.N, d.ms, tw_standard_controller(d) && !getenv("TRAJGEN_DYNAMIC_N"));
+        const TwKernels &k = h->kern;
+        if (!k.loop && !k.loop_p1) return fail(TG_ERR_UNSUPPORTED, "no kernel shape for this horizon");
+        // the attributes are per kernel function and process-wide: always raise them to the device limit so that handles with
+        // different layouts can be used side by side
+        for (const void *f : {(const void *)k.step, (const void *)k.step_p1, (const void *)k.loop, (const void *)k.loop_p1}) {
+            if (!f) continue;
+            CK(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+            CK(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        }
         int occ = 0;
-        int rc = dispatch_tw(h->W, h->S, d, [&](auto W_, auto S_, auto NC_, auto HS_) -> int {
-            constexpr int W = decltype(W_)::value, S = decltype(S_)::value, NC = decltype(NC_)::value;
-            constexpr bool HS = decltype(HS_)::value;
-            // the attribute is per kernel function and process-wide: always raise it to the device limit so that handles with
-            // different layouts can be used side by side
-            if constexpr (!TW_P1_ONLY(W, NC, HS)) {
-                CK(cudaFuncSetAttribute(tw_mpc_step_kernel<W, S, NC, false, HS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
-                CK(cudaFuncSetAttribute(tw_closed_loop_kernel<W, S, NC, false, HS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
-                CK(cudaFuncSetAttribute(tw_mpc_step_kernel<W, S, NC, false, HS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                CK(cudaFuncSetAttribute(tw_closed_loop_kernel<W, S, NC, false, HS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            }
-            if constexpr (TW_HAS_P1(W, NC, HS)) {
-                CK(cudaFuncSetAttribute(tw_mpc_step_kernel<W, S, NC, true, HS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
-                CK(cudaFuncSetAttribute(tw_closed_loop_kernel<W, S, NC, true, HS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
-                CK(cudaFuncSetAttribute(tw_mpc_step_kernel<W, S, NC, true, HS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                CK(cudaFuncSetAttribute(tw_closed_loop_kernel<W, S, NC, true, HS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, tw_closed_loop_kernel<W, S, NC, true, HS>, 32 * W, stride));
-            } else {
-                CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, tw_closed_loop_kernel<W, S, NC, false, HS>, 32 * W, stride));
-            }
-            return TG_OK;
-        });
-        if (rc != TG_OK) return rc;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k.loop_p1 ? k.loop_p1 : k.loop, 32 * h->W, stride));
         if (occ < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
         h->grid_cap = occ * h->num_sms;     // resident problems with one problem per CTA
     }
@@ -668,56 +697,11 @@ int tg_tyre_table_info(tg_handle *h, int32_t *in_use, double *max_value_err, dou
 }
 int tg_kernel_launches(tg_handle *h, int64_t *count) { if (!h || !count) return fail(TG_ERR_INVALID, "null argument"); *count = h->launches; return TG_OK; }
 
-// warp-per-problem kernels: problems per CTA.  Resident problems per SM are bounded by registers (512 threads x 128) and
-// shared memory either way; larger CTAs share more instruction fetches, smaller ones spread a small batch over more SMs.
-static int choose_tw_ppc(const tg_handle *h, int B)
-{
-    if (h->ppc_env) return h->ppc_env;
-    // problems with state-bound rows have long, unequal solves (tens to hundreds of ADMM iterations): free-running
-    // single-problem CTAs beat problems that wait for one another at every step boundary
-    if (h->dc.ms > 0) return 1;
-    // measured at N = 20 (two warps per problem): 4 problems per CTA 2.65e7 steps/s (B = 2368), 8 per CTA 2.37e7 (B = 4736),
-    // 2 per CTA 2.24e7 and 1 per CTA 1.43e7 (B = 1024): sharing instruction fetches matters, waiting for 7 neighbours costs more
-    int p = h->ppc_max < 4 ? h->ppc_max : 4;
-    while (p > 1 && (B + p - 1) / p < h->num_sms) p >>= 1;   // every SM gets a CTA before CTAs get wider
-    return p < 1 ? 1 : p;
-}
-
-extern "C++" {
-template <typename Kern, typename Args>
-static int launch_tw(tg_handle *h, Kern kern, Args &a, int B, int W, int ppc_fixed = 0)
-{
-    const int ppc = ppc_fixed > 0 ? ppc_fixed : choose_tw_ppc(h, B);   // ppc_fixed = 1: a single-problem-per-CTA instance
-    a.ppc = ppc;
-    const size_t smem = (size_t)ppc * tw_stride(h);
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 32 * W * ppc, smem));
-    if (per_sm < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
-    const int cap = per_sm * h->num_sms, ctas = (B + ppc - 1) / ppc;
-    int grid = ctas < cap ? ctas : cap;
-    if (const char *e = getenv("TRAJGEN_GRID")) { const int v = atoi(e); if (v >= 1 && v <= cap) grid = v; }   // measurement knob
-    kern<<<grid, 32 * W * ppc, smem, h->stream>>>(h->dc, h->WL, a);
-    h->launches += 1;
-    CK(cudaGetLastError());
-    return TG_OK;
-}
-}  // extern "C++"
-
 static int launch_step(tg_handle *h, StepArgs &a)
 {
     if (a.B <= 0) return TG_OK;   // empty batch: nothing to do
     CK(cudaSetDevice(h->device));
-    return dispatch_tw(h->W, h->S, h->dc, [&](auto W_, auto S_, auto NC_, auto HS_) -> int {
-        constexpr int W = decltype(W_)::value, S = decltype(S_)::value, NC = decltype(NC_)::value;
-        constexpr bool HS = decltype(HS_)::value;
-        if constexpr (TW_P1_ONLY(W, NC, HS)) {
-            return launch_tw(h, tw_mpc_step_kernel<W, S, NC, true, HS>, a, a.B, W, 1);
-        } else {
-            if constexpr (TW_HAS_P1(W, NC, HS))
-                if (choose_tw_ppc(h, a.B) == 1) return launch_tw(h, tw_mpc_step_kernel<W, S, NC, true, HS>, a, a.B, W, 1);
-            return launch_tw(h, tw_mpc_step_kernel<W, S, NC, false, HS>, a, a.B, W);
-        }
-    });
+    return launch_tw(h, h->kern.step, h->kern.step_p1, a);
 }
 
 int tg_linearize(tg_handle *h, int B, const double *x0, const double *u_prev, double *A, double *Bm, double *g, double *xbar)
@@ -727,8 +711,6 @@ int tg_linearize(tg_handle *h, int B, const double *x0, const double *u_prev, do
     memset(&a, 0, sizeof(a));
     a.B = B; a.x0 = x0; a.u_prev = u_prev; a.path_ref = nullptr; a.vref = nullptr;
     a.A = A; a.Bm = Bm; a.g = g; a.xbar = xbar; a.stop = 1;
-    // the tap does not read the reference window; point it at x0 so loads stay in bounds
-    a.path_ref = nullptr;
     return launch_step(h, a);
 }
 
@@ -796,17 +778,7 @@ int tg_closed_loop(tg_handle *h, int B, int T, const double *x0, const double *u
     memset(&a, 0, sizeof(a));
     a.B = B; a.T = T; a.x0 = x0; a.u0 = u0; a.spec = spec; a.brk = brk; a.coef = coef; a.traj_id0 = traj_id0;
     a.clean = clean; a.noisy = noisy; a.U = U; a.status_counts = status_counts; a.iters_total = (long long *)iters_total;
-    return dispatch_tw(h->W, h->S, h->dc, [&](auto W_, auto S_, auto NC_, auto HS_) -> int {
-        constexpr int W = decltype(W_)::value, S = decltype(S_)::value, NC = decltype(NC_)::value;
-        constexpr bool HS = decltype(HS_)::value;
-        if constexpr (TW_P1_ONLY(W, NC, HS)) {
-            return launch_tw(h, tw_closed_loop_kernel<W, S, NC, true, HS>, a, B, W, 1);
-        } else {
-            if constexpr (TW_HAS_P1(W, NC, HS))
-                if (choose_tw_ppc(h, B) == 1) return launch_tw(h, tw_closed_loop_kernel<W, S, NC, true, HS>, a, B, W, 1);
-            return launch_tw(h, tw_closed_loop_kernel<W, S, NC, false, HS>, a, B, W);
-        }
-    });
+    return launch_tw(h, h->kern.loop, h->kern.loop_p1, a);
 }
 
 int tg_plant_rollout(tg_handle *h, int B, int T, const double *x0, const double *U, double *X)
@@ -1198,12 +1170,7 @@ int tg_closed_loop_host(tg_handle *h, int B, int T, const double *x0, const doub
     // Rows leave the SM at ~1 GB/s (112 B per MPC step), far below what PCIe carries, so when the caller's result buffers
     // are pinned the kernel stores straight into them (posted writes overlap the computation) and the device-to-host copy
     // of the rows after the kernel disappears.  Pageable buffers are staged through the device arena.
-    // TRAJGEN_HOST_OUTPUT=staged forces the staged path (measurement knob).
-    const char *mode = getenv("TRAJGEN_HOST_OUTPUT");
-    const bool allow_direct = !(mode && strcmp(mode, "staged") == 0);
-    double *a_cl = allow_direct ? (double *)pinned_device_alias(clean) : nullptr;
-    double *a_no = allow_direct ? (double *)pinned_device_alias(noisy) : nullptr;
-    double *a_U = allow_direct ? (double *)pinned_device_alias(U) : nullptr;
+    double *a_cl = (double *)pinned_device_alias(clean), *a_no = (double *)pinned_device_alias(noisy), *a_U = (double *)pinned_device_alias(U);
     const bool direct = a_cl && a_no && (a_U || !s_U);
     const size_t total = PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + (direct ? 0 : 2 * PAD(s_cl) + PAD(s_U)) + PAD(s_sc) + PAD(s_it) + 4096;
     int rc = ensure_dstage(h, total);

@@ -56,9 +56,8 @@ __device__ __forceinline__ void tg_sync(int bar, int nthreads)
     asm volatile("bar.sync %0, %1;" ::"r"(bar), "r"(nthreads) : "memory");
 }
 
-#ifndef TW_KB
 #define TW_KB 4                  // horizon stages condensed per synchronisation in K2 (twice as many on the eight-warp, one-tile shape,
-#endif                           // N = 31 .. 44, whose synchronisations are the costliest: config 1 53.4 -> 51.8 us per step)
+                                 // N = 31 .. 44, whose synchronisations are the costliest: config 1 53.4 -> 51.8 us per step)
 #define TW_WARM_RESTART_ITER 300
 #define TW_FREE_RHO 1e-6         // rho scale of a solve that starts with no active row (see tw_step_body)
 #define TW_POLISH_MARGIN 1e-3    // a converged standard solve is polished if every row is this far inside its bounds
@@ -365,11 +364,8 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
     // the loads of a stage are issued under the arithmetic of the previous one
     constexpr bool FULLKB = NC > 0 && NC % KB == 0;
     constexpr int UNR = FULLKB ? KB : 1;
-#ifndef TW_UNROLL_ROUNDS
-#define TW_UNROLL_ROUNDS 0   // unrolling the rounds as well measured 1 % slower (more code, no extra overlap)
-#endif
-    constexpr int UNR0 = (FULLKB && TW_UNROLL_ROUNDS) ? (NC > 0 ? NC / KB : 1) : 1;
-#pragma unroll UNR0
+    // unrolling the rounds as well measured 1 % slower (more code, no extra overlap)
+#pragma unroll 1
     for (int k0 = 0; k0 < N; k0 += KB) {
         const int kb = FULLKB ? KB : ((N - k0 < KB) ? N - k0 : KB);
         double *wblk = wbuf + ((LF(nbuf) == 2) ? ((k0 / KB) & 1) * KB * 3 * NVP : 0);
@@ -603,25 +599,10 @@ __device__ __forceinline__ double tw_gs_row_dot(const WLayout &L, const double *
     return acc;
 }
 
-// In-register inversion of the SPD tile by n symmetric sweeps (SWP_k: a_kk <- -1/a_kk, a_ik <- a_ik/a_kk,
-// a_ij <- a_ij - a_ik a_kj / a_kk); on return a = -K^-1 (lower-triangle blocks).
-// Step k = 4 K + kr: the threads holding block row K (their row kr) and block column K (their column kr) publish row k of
-// the matrix (= column k by symmetry) with v[k] = a_kk - 1, the reciprocal pivot beside it; everybody then does one rank-1
-// update of each slot with w_i = v_i / a_kk (w = 1 - 1/a_kk on the pivot row) and the pivot is repaired in place.
-// K is Jacobi-scaled first (K^ = D K D, D = diag(K)^-1/2: the unpivoted sweep is only as accurate as cond(K), and K inherits
-// the variable scaling of H) and un-scaled afterwards.
-template <int W, int S, int NC>
-__device__ __forceinline__ void tw_sweep_invert_scalar(const DevCfg &c, const WLayout &L, double *sm, const TwMap<S> &mp,
-                                                       double (&a)[S][4][4], int bar)
+// a <- D a D with the diagonal D in dsc: the Jacobi scaling of the tile before the sweeps and the un-scaling after them
+template <int S>
+__device__ __forceinline__ void tw_scale_tile(const double *dsc, const TwMap<S> &mp, double (&a)[S][4][4])
 {
-    const int n = NC > 0 ? 2 * NC : c.n, NV = LF(NV), nb = LF(nb);
-    double *vb = sm + LF(piv), *dsc = sm + LF(dsc);
-#pragma unroll
-    for (int s = 0; s < S; ++s)
-        if (mp.act[s] && mp.ro[s] == mp.co[s])
-            tw_st4(dsc + mp.ro[s], (mp.ro[s] + 0 < n) ? rsqrt(a[s][0][0]) : 0.0, (mp.ro[s] + 1 < n) ? rsqrt(a[s][1][1]) : 0.0,
-                   (mp.ro[s] + 2 < n) ? rsqrt(a[s][2][2]) : 0.0, (mp.ro[s] + 3 < n) ? rsqrt(a[s][3][3]) : 0.0);
-    tw_sync<W>(bar);
 #pragma unroll
     for (int s = 0; s < S; ++s) {
         double dr[4], dc[4];
@@ -632,6 +613,34 @@ __device__ __forceinline__ void tw_sweep_invert_scalar(const DevCfg &c, const WL
 #pragma unroll
             for (int cc = 0; cc < 4; ++cc) a[s][r][cc] *= dr[r] * dc[cc];
     }
+}
+// K^ = D K D with D = diag(K)^-1/2 (zero in the pad rows), published in dsc for the un-scaling K^-1 = D K^^-1 D: the unpivoted
+// sweep is only as accurate as cond(K), and K inherits the variable scaling of H
+template <int W, int S>
+__device__ __forceinline__ void tw_jacobi_scale(double *dsc, const TwMap<S> &mp, double (&a)[S][4][4], int n, int bar)
+{
+#pragma unroll
+    for (int s = 0; s < S; ++s)
+        if (mp.act[s] && mp.ro[s] == mp.co[s])
+            tw_st4(dsc + mp.ro[s], (mp.ro[s] + 0 < n) ? rsqrt(a[s][0][0]) : 0.0, (mp.ro[s] + 1 < n) ? rsqrt(a[s][1][1]) : 0.0,
+                   (mp.ro[s] + 2 < n) ? rsqrt(a[s][2][2]) : 0.0, (mp.ro[s] + 3 < n) ? rsqrt(a[s][3][3]) : 0.0);
+    tw_sync<W>(bar);
+    tw_scale_tile<S>(dsc, mp, a);
+}
+
+// In-register inversion of the SPD tile by n symmetric sweeps (SWP_k: a_kk <- -1/a_kk, a_ik <- a_ik/a_kk,
+// a_ij <- a_ij - a_ik a_kj / a_kk); on return a = -K^-1 (lower-triangle blocks).
+// Step k = 4 K + kr: the threads holding block row K (their row kr) and block column K (their column kr) publish row k of
+// the matrix (= column k by symmetry) with v[k] = a_kk - 1, the reciprocal pivot beside it; everybody then does one rank-1
+// update of each slot with w_i = v_i / a_kk (w = 1 - 1/a_kk on the pivot row) and the pivot is repaired in place.
+// K is Jacobi-scaled first and un-scaled afterwards.
+template <int W, int S, int NC>
+__device__ __forceinline__ void tw_sweep_invert_scalar(const DevCfg &c, const WLayout &L, double *sm, const TwMap<S> &mp,
+                                                       double (&a)[S][4][4], int bar)
+{
+    const int n = NC > 0 ? 2 * NC : c.n, NV = LF(NV), nb = LF(nb);
+    double *vb = sm + LF(piv), *dsc = sm + LF(dsc);
+    tw_jacobi_scale<W, S>(dsc, mp, a, n, bar);
     // the reciprocal of pivot k+1 is started as soon as that entry has been updated in step k, so that its latency overlaps
     // the rest of the rank-1 update
     double rp_next = 0.0;
@@ -688,69 +697,25 @@ __device__ __forceinline__ void tw_sweep_invert_scalar(const DevCfg &c, const WL
             }
         }
     }
-#pragma unroll
-    for (int s = 0; s < S; ++s) {   // K^-1 = D K^^-1 D
-        double dr[4], dc[4];
-        tw_ld4(dsc + mp.ro[s], dr);
-        tw_ld4(dsc + mp.co[s], dc);
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-            for (int cc = 0; cc < 4; ++cc) a[s][r][cc] *= dr[r] * dc[cc];
-    }
+    tw_scale_tile<S>(dsc, mp, a);   // K^-1 = D K^^-1 D
     tw_sync<W>(bar);
 }
 
-// BLOCKED sweep: the four pivots of a 4 x 4 diagonal block at once (one synchronisation per block instead of four, and every
-// thread's work is 128 independent FMAs instead of four dependent rank-1 rounds).  Sweeping the index set P of block K:
+// BLOCKED sweep: the pivots of a 4 x 4 diagonal block in two groups of two (two synchronisations per block instead of four).
+// Sweeping the index set P of a group:
 //     A_PP <- -D^-1 (D = A_PP),   A_iP <- A_iP D^-1,   A_ij <- A_ij - A_iP D^-1 A_Pj.
-// The panel V = A_.P (n x 4) is published column-wise (VT[m][i] = A_{i, P_m}; block column K below the diagonal, block row K
+// The panel V = A_.P (n x 2) is published column-wise (VT[m][i] = A_{i, P_m}; block column K below the diagonal, block row K
 // left of it by symmetry), with D - I in the rows of P itself, and the owner of the diagonal block publishes D^-1 (inverted in
 // its registers).  With that patch every block (I, J) -- panel blocks included -- does the same update
 //     A_IJ <- A_IJ - (V_I D^-1) V_J',
-// and only the diagonal block is repaired afterwards (<- -D^-1).  The panel and the inverse of block K + 1 are published
-// right after a thread's update of step K, into the buffer of the other parity.
-#ifndef TW_SWEEP_PB
-#define TW_SWEEP_PB 1    // pivots per synchronisation of the sweep (1 = scalar sweep, 2 or 4 = blocked; measured: DESIGN.md section 8)
-#endif
-// inverse of the PB x PB SPD block d[o .. o+PB-1][o .. o+PB-1] (PB = 2: closed form; PB = 4: four scalar sweeps in registers)
-template <int PB>
-__device__ __forceinline__ void tw_inv_spd(const double (&a)[4][4], int o_static, double (&di)[PB][PB]);
-template <>
-__device__ __forceinline__ void tw_inv_spd<2>(const double (&a)[4][4], int o, double (&di)[2][2])
+// and only the diagonal block is repaired afterwards (<- -D^-1).  The panel and the inverse of the next group are published
+// right after a thread's update of the current one, into the other buffer.
+// inverse of the 2 x 2 SPD block a[o .. o+1][o .. o+1] (closed form)
+__device__ __forceinline__ void tw_inv_spd(const double (&a)[4][4], int o, double (&di)[2][2])
 {
     const double a00 = o ? a[2][2] : a[0][0], a01 = o ? a[3][2] : a[1][0], a11 = o ? a[3][3] : a[1][1];
     const double r = tw_rcp3(fma(a00, a11, -a01 * a01));   // SPD: det > 0
     di[0][0] = a11 * r; di[1][1] = a00 * r; di[0][1] = -a01 * r; di[1][0] = di[0][1];
-}
-template <>
-__device__ __forceinline__ void tw_inv_spd<4>(const double (&a)[4][4], int, double (&di)[4][4])
-{
-    double d[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) d[i][j] = a[i][j];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const double p = tw_rcp3(d[k][k]);   // Schur complements of an SPD matrix: pivots > 0
-        double w[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) w[i] = d[i][k] * p;
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-                if (i != k && j != k) d[i][j] = fma(-w[i], d[k][j], d[i][j]);
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-            if (i != k) { d[i][k] = w[i]; d[k][i] = w[i]; }
-        d[k][k] = -p;
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) di[i][j] = -d[i][j];
 }
 
 template <int W, int S, int NC>
@@ -761,34 +726,20 @@ __device__ __forceinline__ void tw_sweep_invert(const DevCfg &c, const WLayout &
     // (the blocked forms add fp64 work that the 7-8 problems of an SM have to share the fp64 pipe for); with four or eight warps
     // per problem the synchronisation is costlier and the 2-pivot form wins (config 1: 52.0 -> 49.6 us per step; N = 30: +2 %);
     // the 4-pivot form loses everywhere.  Two tiles per thread (N > 44) keep the scalar form.
-    constexpr int PB = (W >= 4 && S == 1) ? 2 : TW_SWEEP_PB;
-    if constexpr (PB == 1 || (S > 1 && PB == 4)) {   // (two tiles per thread leave no registers for the 4-pivot block operands)
+    if constexpr (!(W >= 4 && S == 1)) {
         tw_sweep_invert_scalar<W, S, NC>(c, L, sm, mp, a, bar);
         return;
     } else {
-    constexpr int NH = 4 / PB;   // pivot groups per 4 x 4 block
+    constexpr int PB = 2;   // pivots per group
     const int n = NC > 0 ? 2 * NC : c.n, NV = LF(NV), nb = LF(nb);
     double *vb = sm + LF(piv), *dsc = sm + LF(dsc);
+    tw_jacobi_scale<W, S>(dsc, mp, a, n, bar);
 #pragma unroll
     for (int s = 0; s < S; ++s)
-        if (mp.act[s] && mp.ro[s] == mp.co[s])
-            tw_st4(dsc + mp.ro[s], (mp.ro[s] + 0 < n) ? rsqrt(a[s][0][0]) : 0.0, (mp.ro[s] + 1 < n) ? rsqrt(a[s][1][1]) : 0.0,
-                   (mp.ro[s] + 2 < n) ? rsqrt(a[s][2][2]) : 0.0, (mp.ro[s] + 3 < n) ? rsqrt(a[s][3][3]) : 0.0);
-    tw_sync<W>(bar);
-#pragma unroll
-    for (int s = 0; s < S; ++s) {
-        double dr[4], dc[4];
-        tw_ld4(dsc + mp.ro[s], dr);
-        tw_ld4(dsc + mp.co[s], dc);
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-            for (int cc = 0; cc < 4; ++cc) a[s][r][cc] *= dr[r] * dc[cc];
         if (mp.ro[s] == mp.co[s])   // pad rows (odd horizons) become identity rows: they pass through the block inverse unchanged
 #pragma unroll
             for (int r = 0; r < 4; ++r)
                 if (mp.ro[s] + r >= n) a[s][r][r] = 1.0;
-    }
     // panel buffer of one pivot group: PB columns of NV (VT[m][i] = A_{i, P_m}) + the PB x PB inverse; two buffers, alternating
     constexpr unsigned PS = TW_PS(W, S);
     const unsigned NVP = PS * (unsigned)nb;   // padded panel columns (TW_PAD)
@@ -805,7 +756,7 @@ __device__ __forceinline__ void tw_sweep_invert(const DevCfg &c, const WLayout &
                 if (mp.ro[s] == K4) {
                     if (mp.co[s] == K4) {   // diagonal block: D - I in the pivot rows, D^-1 beside the panel
                         double di[PB][PB];
-                        tw_inv_spd<PB>(a[s], o, di);
+                        tw_inv_spd(a[s], o, di);
 #pragma unroll
                         for (int m = 0; m < PB; ++m) {
                             tw_sts4(ro_a[s] + boff + (unsigned)m * nv8, a[s][0][o + m] - (o + m == 0 ? 1.0 : 0.0), a[s][1][o + m] - (o + m == 1 ? 1.0 : 0.0),
@@ -866,32 +817,15 @@ __device__ __forceinline__ void tw_sweep_invert(const DevCfg &c, const WLayout &
 #pragma unroll 1
     for (int K = 0; K < nb; ++K) {
         const int K4 = 4 * K;
-        // NH pivot groups per block; the buffer alternates with every group (NH is 1 or 2, so group h of block K uses buffer
-        // (K NH + h) & 1)
-        if constexpr (NH == 2) {
-            tw_sync<W>(bar);
-            update(K4, integral_constant<int, 0>(), 0u);
-            publish(K4, integral_constant<int, 1>(), stride_a);
-            tw_sync<W>(bar);
-            update(K4, integral_constant<int, 1>(), stride_a);
-            if (K + 1 < nb) publish(K4 + 4, integral_constant<int, 0>(), 0u);
-        } else {
-            const unsigned boff = (K & 1) ? stride_a : 0u;
-            tw_sync<W>(bar);
-            update(K4, integral_constant<int, 0>(), boff);
-            if (K + 1 < nb) publish(K4 + 4, integral_constant<int, 0>(), (K & 1) ? 0u : stride_a);
-        }
+        // the buffer alternates with every group: group h of a block uses buffer h
+        tw_sync<W>(bar);
+        update(K4, integral_constant<int, 0>(), 0u);
+        publish(K4, integral_constant<int, 1>(), stride_a);
+        tw_sync<W>(bar);
+        update(K4, integral_constant<int, 1>(), stride_a);
+        if (K + 1 < nb) publish(K4 + 4, integral_constant<int, 0>(), 0u);
     }
-#pragma unroll
-    for (int s = 0; s < S; ++s) {   // K^-1 = D K^^-1 D
-        double dr[4], dc[4];
-        tw_ld4(dsc + mp.ro[s], dr);
-        tw_ld4(dsc + mp.co[s], dc);
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-            for (int cc = 0; cc < 4; ++cc) a[s][r][cc] *= dr[r] * dc[cc];
-    }
+    tw_scale_tile<S>(dsc, mp, a);   // K^-1 = D K^^-1 D
     tw_sync<W>(bar);
     }
 }
