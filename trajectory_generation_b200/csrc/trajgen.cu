@@ -57,10 +57,11 @@ struct LoopArgs {
 };
 
 // ------------------------------------------------------------------------------------------------ warp-per-problem kernels
-// tw_solver.cuh: W warps per problem (W = 1 for N <= 20), P problems per CTA side by side, each with its own shared-memory
-// block (and, for W > 1, its own named barrier).  Problems of a CTA are re-aligned at every step boundary (barrier 15) so that
-// they fetch the same instruction lines at the same time (the step body is ~100 KB of mostly straight-line code).
+// tw_solver.cuh: W warps per problem (W = 1 for N <= 14), P problems per CTA side by side, each with its own shared-memory
+// block (and, for W > 1, its own named barrier TW_BAR_PROB + p).  Problems of a CTA are re-aligned at every step boundary
+// (TW_BAR_STEP) so that they fetch the same instruction lines at the same time (the step body is ~100 KB of straight code).
 #define TW_CTA_THREADS 512
+enum { TW_BAR_PROB = 1, TW_BAR_STEP = 15 };
 // register budget: 128 per thread on every shape (the tile takes 32 of them with S = 1, 64 with S = 2).  The kernels state it
 // next to __launch_bounds__, so that ptxas gets both .maxntid and .maxnreg (without .maxntid the single-problem instances
 // compile to different code, without .maxnreg all of them do); nvcc accepts the two qualifiers together only with a value
@@ -78,9 +79,9 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
     constexpr int NT = 32 * W;
     const int P = P1 ? 1 : a.ppc;
     int prob = P1 ? 0 : threadIdx.x / NT, tid = P1 ? threadIdx.x : threadIdx.x % NT;
-    unsigned sm_off = (unsigned)prob * (unsigned)((L.total + 1) & ~1) * 8u;
+    unsigned sm_off = (unsigned)prob * (unsigned)tw_stride(L) * 8u;
     if constexpr (!P1) asm volatile("" : "+r"(tid), "+r"(prob), "+r"(sm_off));   // kept in registers instead of being re-derived at every use
-    const int bar = P1 ? 1 : 1 + prob;
+    const int bar = P1 ? TW_BAR_PROB : TW_BAR_PROB + prob;
     double *sm = reinterpret_cast<double *>(reinterpret_cast<char *>(sm_all) + sm_off);
     const int N = NC > 0 ? NC : c.N, n = 2 * N, ms = HS ? c.ms : 0;
     if (prob >= P) return;
@@ -175,9 +176,9 @@ tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ 
     constexpr int NT = 32 * W;
     const int P = P1 ? 1 : a.ppc;
     int prob = P1 ? 0 : threadIdx.x / NT, tid = P1 ? threadIdx.x : threadIdx.x % NT;
-    unsigned sm_off = (unsigned)prob * (unsigned)((L.total + 1) & ~1) * 8u;
+    unsigned sm_off = (unsigned)prob * (unsigned)tw_stride(L) * 8u;
     if constexpr (!P1) asm volatile("" : "+r"(tid), "+r"(prob), "+r"(sm_off));
-    const int bar = P1 ? 1 : 1 + prob;
+    const int bar = P1 ? TW_BAR_PROB : TW_BAR_PROB + prob;
     double *sm = reinterpret_cast<double *>(reinterpret_cast<char *>(sm_all) + sm_off);
     const int N = NC > 0 ? NC : c.N, n = 2 * N, ms = HS ? c.ms : 0, ns = HS ? c.ns : 0, T = a.T;
     if (prob >= P) return;
@@ -263,7 +264,7 @@ tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ 
             warm = ok && c.warm_start;
             warm_free = warm && r.free_end;
             if constexpr (P1) tw_sync<W>(bar);
-            else if (lockstep) tg_sync(15, NT * active); else tw_sync<W>(bar);
+            else if (lockstep) tg_sync(TW_BAR_STEP, NT * active); else tw_sync<W>(bar);
         }
         tw_sync<W>(bar);
         if (tid < TG_NUM_STATUS && a.status_counts) a.status_counts[(size_t)b * TG_NUM_STATUS + tid] = cnt[tid];
@@ -435,16 +436,6 @@ struct tg_handle {
     void *hstage; size_t hstage_bytes;
 };
 
-static bool pick_tw_shape(int N, int &W, int &S)
-{
-    if (N <= 14) { W = 1; S = 1; }          // 28 blocks on one warp
-    else if (N <= 20) { W = 2; S = 1; }     // 55 blocks on two warps
-    else if (N <= 30) { W = 4; S = 1; }     // 120 blocks
-    else if (N <= 44) { W = 8; S = 1; }     // 253 blocks
-    else if (N <= 56) { W = 8; S = 2; }     // 406 blocks on 512 slots
-    else return false;
-    return true;
-}
 // kernel instances: (W, S) for a run-time horizon, plus the horizons of the reference / the BASELINE configurations compiled in
 // (NC = N: shared-memory offsets become immediates, horizon loops get constant trip counts: 25-50 % faster).  The compile-time
 // instances serve the standard controller only -- MPC tyre model from the tables, analytic Jacobians (tw_standard_controller) --
@@ -460,6 +451,7 @@ static bool tw_standard_controller(const DevCfg &d)
 template <int W, int S, int NC, bool HS>
 static TwKernels tw_instance()
 {
+    static_assert(NC == 0 || (tw_shape(NC).W == W && tw_shape(NC).S == S), "a compile-time horizon runs on its tw_shape");
     TwKernels k = {};
     if constexpr (!(HS && NC > 0 && W <= 2)) {
         k.step = tw_mpc_step_kernel<W, S, NC, false, HS>;
@@ -493,7 +485,6 @@ static TwKernels tw_kernels(int W, int S, int N, int ms, bool fixed_n)
     if (W == 8 && S == 2) return tw_instance<8, 2, 0, true>();
     return TwKernels{};
 }
-static size_t tw_stride(const tg_handle *h) { return (((size_t)h->WL.total + 1) & ~(size_t)1) * sizeof(double); }
 
 // warp-per-problem kernels: problems per CTA.  Resident problems per SM are bounded by registers (512 threads x 128) and
 // shared memory either way; larger CTAs share more instruction fetches, smaller ones spread a small batch over more SMs.
@@ -520,7 +511,7 @@ static int launch_tw(tg_handle *h, void (*multi)(DevCfg, WLayout, Args), void (*
     if (p1 && (!multi || ppc == 1)) { kern = p1; ppc = 1; }
     a.ppc = ppc;
     const int threads = 32 * h->W * ppc;
-    const size_t smem = (size_t)ppc * tw_stride(h);
+    const size_t smem = (size_t)ppc * h->smem_bytes;
     int per_sm = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
     if (per_sm < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
@@ -566,8 +557,8 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
     if (!(cfg->Ts > 0)) return fail(TG_ERR_INVALID, "Ts must be > 0");
     if (cfg->max_iter < 1 || cfg->check_every < 1) return fail(TG_ERR_INVALID, "max_iter and check_every must be >= 1");
     if (!(cfg->rho > 0) || !(cfg->sigma > 0) || !(cfg->alpha > 0 && cfg->alpha < 2)) return fail(TG_ERR_INVALID, "rho, sigma > 0 and 0 < alpha < 2 required");
-    int W_ = 0, S_ = 0;
-    if (!pick_tw_shape(cfg->N, W_, S_)) return fail(TG_ERR_UNSUPPORTED, "horizon N > 56 is not supported");
+    const TwShape shape = tw_shape(cfg->N);
+    if (shape.W == 0) return fail(TG_ERR_UNSUPPORTED, "horizon N > 56 is not supported");
     int ndev = 0;
     CK(cudaGetDeviceCount(&ndev));
     if (ndev == 0) return fail(TG_ERR_CUDA, "no CUDA device: libtrajgen has no CPU fallback");
@@ -581,7 +572,7 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
     if (!h) return fail(TG_ERR_NOMEM, "out of host memory");
     memset(h, 0, sizeof(*h));
     struct Guard { tg_handle *p; ~Guard() { if (p) { cudaFree(p->tyre_tab); delete p; } } } guard{h};   // released on success
-    h->cfg = *cfg; h->W = W_; h->S = S_; h->device = device; h->num_sms = prop.multiProcessorCount;
+    h->cfg = *cfg; h->W = shape.W; h->S = shape.S; h->device = device; h->num_sms = prop.multiProcessorCount;
     DevCfg &d = h->dc;
     d.N = cfg->N; d.n = 2 * cfg->N; d.model = cfg->model; d.plant = cfg->plant; d.jacobian = cfg->jacobian;
     d.ns = 0;
@@ -625,16 +616,16 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
 
     d.free_mode = (cfg->solver_flags & 1) ? 0 : 1;
     h->smem_optin = (size_t)prop.sharedMemPerBlockOptin;
-    h->Lref = tw_make_layout(d.N, 0, 1);
+    h->Lref = tw_make_layout(d.N, 0, TwShape{1, 1});
     CK(cudaFuncSetAttribute(tg_ref_window_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
     h->ppc_env = 0;   // TRAJGEN_PPC pins the number of problems per CTA (measurement knob)
     {
-        h->WL = tw_make_layout(d.N, d.ms, h->W);
-        const size_t stride = tw_stride(h);
+        h->WL = tw_make_layout(d.N, d.ms, shape);
+        const size_t stride = (size_t)tw_stride(h->WL) * sizeof(double);
         h->smem_bytes = stride;
         if (stride > h->smem_optin) return fail(TG_ERR_UNSUPPORTED, "state-bound rows x horizon exceed the 227 KB shared memory of one CTA");
         h->ppc_max = TW_CTA_THREADS / (32 * h->W);
-        if (h->W > 1 && h->ppc_max > 14) h->ppc_max = 14;                  // named barriers 1..14 + the step barrier 15
+        if (h->W > 1) h->ppc_max = std::min(h->ppc_max, TW_BAR_STEP - TW_BAR_PROB);   // a barrier id per problem
         while (h->ppc_max > 1 && (size_t)h->ppc_max * stride > h->smem_optin) h->ppc_max -= 1;
         if (const char *e = getenv("TRAJGEN_PPC")) { const int v = atoi(e); if (v >= 1 && v <= h->ppc_max) h->ppc_env = v; }
         h->kern = tw_kernels(h->W, h->S, d.N, d.ms, tw_standard_controller(d) && !getenv("TRAJGEN_DYNAMIC_N"));

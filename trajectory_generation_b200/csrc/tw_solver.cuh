@@ -1,4 +1,4 @@
-// tw_solver.cuh -- one MPC step for one problem by W warps; W = 1 (horizons N <= 20) is a warp per problem with no CTA
+// tw_solver.cuh -- one MPC step for one problem by W warps; W = 1 (horizons N <= 14) is a warp per problem with no CTA
 // barrier anywhere on the path (sm_100a, fp64).
 //
 // Replaces MPC/mpc_6stati.py:165-275 (nominal rollout, N x linearize_discretize, CVXPY problem construction, OSQP solve,
@@ -9,8 +9,8 @@
 //       three scaled rows W (lateral error, heading, speed); H = sum_k W_k' W_k + band terms accumulates in the tile
 //   K3  ADMM (the OSQP iteration) on K = H + sigma I + A' diag(rho) A.
 // The n x n symmetric matrix (n = 2N) lives in registers as its LOWER TRIANGLE only: 4 x 4 blocks (I, J), J <= I, dealt
-// row-major over the 32 W threads, S blocks ("slots") per thread -- n = 40 is 55 blocks on 64 slots of one warp, 32
-// doubles per lane.  K^-1 comes from n symmetric sweep steps on that tile (one shared-memory round trip per pivot, the
+// row-major over the 32 W threads, S blocks ("slots") per thread (tw_shape) -- n = 40 is 55 blocks on the 64 threads of two
+// warps, 16 doubles per thread.  K^-1 comes from n symmetric sweep steps on that tile (one shared-memory round trip per pivot, the
 // pivot-row index inside a block is a compile-time constant); x~ = K^-1 rhs is 2 x 16 FMAs per off-diagonal block, with
 // the block partials exchanged through shared memory.  The ADMM vectors live in shared memory, lane t owns stage t (the
 // entries 2t, 2t+1 of dU and its two box and two rate rows).
@@ -56,15 +56,13 @@ __device__ __forceinline__ void tg_sync(int bar, int nthreads)
     asm volatile("bar.sync %0, %1;" ::"r"(bar), "r"(nthreads) : "memory");
 }
 
-#define TW_KB 4                  // horizon stages condensed per synchronisation in K2 (twice as many on the eight-warp, one-tile shape,
-                                 // N = 31 .. 44, whose synchronisations are the costliest: config 1 53.4 -> 51.8 us per step)
 #define TW_WARM_RESTART_ITER 300
 #define TW_FREE_RHO 1e-6         // rho scale of a solve that starts with no active row (see tw_step_body)
 #define TW_POLISH_MARGIN 1e-3    // a converged standard solve is polished if every row is this far inside its bounds
 
-// shared-memory layout of one problem (offsets in doubles), identical on host and device.  Everything that does not depend on
-// the number of state-bound rows ms comes first, so that for a compile-time horizon (template parameter NC of the kernels)
-// every offset of the fixed part is an immediate in the load / store instructions; the state-row arrays form the tail.
+// shared-memory layout of one problem (offsets in doubles) on a shape, identical on host and device.  Everything that does not
+// depend on the number of state-bound rows ms comes first, so that for a compile-time horizon (template parameter NC of the
+// kernels) every offset of the fixed part is an immediate in the load / store instructions; the state-row arrays form the tail.
 struct WLayout {
     int x0, uprev, misc, spec, xbar, lin, rr, sn, cs, q, x, xt, v, z, y, rho, rinv, dyr, piv, wb, red;
     int aux, Xr, Yr, Pr, vref, P;   // inside the wb region (dead before / after K2)
@@ -83,21 +81,29 @@ __host__ __device__ constexpr int tw_even(int v) { return (v + 1) & ~1; }   // k
 __host__ __device__ constexpr int tw_gs_len(int k) { return 4 * ((k >> 1) + 1); }
 __host__ __device__ constexpr int tw_gs_off(int k) { return 4 * (k >> 1) * ((k >> 1) + 1) + ((k & 1) ? 4 * ((k >> 1) + 1) : 0); }
 
+// shape of the solver for horizon N: W warps per problem, S tile blocks per thread (28, 55, 120 and 253 blocks on 32 W
+// threads, 406 on 512 slots); W = 0: N is not supported
+struct TwShape { int W, S; };
+__host__ __device__ constexpr TwShape tw_shape(int N)
+{ return N <= 14 ? TwShape{1, 1} : N <= 20 ? TwShape{2, 1} : N <= 30 ? TwShape{4, 1} : N <= 44 ? TwShape{8, 1} : N <= 56 ? TwShape{8, 2} : TwShape{0, 0}; }
+
 // Block vectors that every thread reads at its block row AND its block column (the pivot rows of the sweep, the staging rows of
 // the condensing) are stored PADDED: the four entries of block I at 6 I .. 6 I + 3.  The 16-byte pieces that the lanes of a warp
 // read then fall into distinct banks (stride 48 bytes: 8 block rows cover the 32 banks once) instead of colliding pairwise
 // (stride 32 bytes: block rows I and I + 4 share their banks): one wavefront per 128-bit load instead of two.
 // (Not on the two-tiles-per-thread shape, N > 44, whose constrained problems need the shared memory for their second resident
 // CTA, and not on the one-warp shape, N <= 14, where it gains nothing and costs the sixteenth resident CTA.)
-#define TW_PS(W_, S_) (((S_) >= 2 || (W_) == 1) ? 4 : 6)    // doubles per block in a padded vector
+__host__ __device__ constexpr int tw_ps(int W, int S) { return (S >= 2 || W == 1) ? 4 : 6; }   // doubles per block in a padded vector
 #define TW_PAD(i, PS_) ((PS_) * ((i) >> 2) + ((i) & 3))
-__host__ __device__ constexpr int tw_ps_layout(int N, int W) { return ((W >= 8 && N > 44) || W == 1) ? 4 : 6; }   // = TW_PS(W, S) of the shape
+// horizon stages condensed per synchronisation in K2: twice as many on the eight-warp, one-tile shape, N = 31 .. 44, whose
+// synchronisations are the costliest (config 1 53.4 -> 51.8 us per step)
+__host__ __device__ constexpr int tw_kb(int W, int S) { return (W >= 8 && S == 1) ? 8 : 4; }
 
-__host__ __device__ constexpr WLayout tw_make_layout(int N, int ms, int W)
+__host__ __device__ constexpr WLayout tw_make_layout(int N, int ms, TwShape sh)
 {
     WLayout L = {};
     int o = 0;
-    const int n = 2 * N;
+    const int n = 2 * N, W = sh.W, ps = tw_ps(sh.W, sh.S);
     const int nb = (n + 3) / 4, NV = 4 * nb;
     L.nb = nb; L.NV = NV; L.nbuf = (W == 1) ? 1 : 2;
     L.x0 = o; o += 6; L.uprev = o; o += 2; L.misc = o; o += 24; L.spec = o; o += 12;
@@ -106,8 +112,8 @@ __host__ __device__ constexpr WLayout tw_make_layout(int N, int ms, int W)
     L.q = o; o += NV; L.x = o; o += NV; L.xt = o; o += NV; L.v = o; o += NV;
     L.z = o; o += 2 * NV; L.y = o; o += 2 * NV; L.rho = o; o += 2 * NV + 2; L.rinv = o; o += 2 * NV + 2;   // box rows, then rate rows at + n
     L.dyr = o; o += NV + 2;
-    L.piv = o; o += 2 * (4 * tw_ps_layout(N, W) * nb + 16);   // two panel buffers of the sweep (up to 4 padded columns + the 4 x 4 inverse)
-    int wbn = L.nbuf * ((W >= 8 && N <= 44) ? 2 * TW_KB : TW_KB) * 3 * tw_ps_layout(N, W) * nb;   // padded staging rows (TW_PAD)
+    L.piv = o; o += 2 * (4 * ps * nb + 16);   // two panel buffers of the sweep (up to 4 padded columns + the 4 x 4 inverse)
+    int wbn = L.nbuf * tw_kb(sh.W, sh.S) * 3 * ps * nb;   // padded staging rows (TW_PAD)
     if (wbn < nb * nb * 4) wbn = nb * nb * 4;
     const int k1n = tw_even(6 * N) + 4 * tw_even(N + 2);
     if (wbn < k1n) wbn = k1n;
@@ -125,9 +131,12 @@ __host__ __device__ constexpr WLayout tw_make_layout(int N, int ms, int W)
     return L;
 }
 
-// compile-time geometry of horizon NC (NC = 0: run-time horizon, everything comes from the WLayout kernel argument)
+// compile-time geometry of horizon NC on its shape (NC = 0: run-time horizon, everything comes from the WLayout kernel argument)
 template <int NC, int W>
-struct TwFix { static constexpr WLayout L = tw_make_layout(NC, 0, W); };
+struct TwFix { static_assert(NC == 0 || tw_shape(NC).W == W, "a compile-time horizon runs on its tw_shape");
+               static constexpr WLayout L = tw_make_layout(NC, 0, tw_shape(NC)); };
+// doubles of shared memory per problem: the problems of a CTA lie side by side, each block 16-byte aligned
+__host__ __device__ constexpr int tw_stride(const WLayout &L) { return tw_even(L.total); }
 // offset of a FIXED-part array / a geometry constant
 #define LF(f) (NC > 0 ? TwFix<NC, W>::L.f : L.f)
 
@@ -322,27 +331,23 @@ __device__ __forceinline__ void tw_ref_window_warp(const DevCfg &c, const WLayou
 }
 
 // ---------------------------------------------------------------------------------------------------------------- K2
-// H = sum_k W_k' W_k on the tile (W rows carry sqrt(2 q)); optionally q and the state-bound rows.  Lane j owns column j of G;
-// with one warp and n > 32 a lane owns the columns j and j + 32, the second of which is born at stage 16.
-template <int W, int S, int NPASS, int NC, bool HS>
+// H = sum_k W_k' W_k on the tile (W rows carry sqrt(2 q)); optionally q and the state-bound rows.  Thread j owns column j of G
+// (n <= 32 W on every shape).
+template <int W, int S, int NC, bool HS>
 __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, double *sm, const TwMap<S> &mp, double (&a)[S][4][4],
                                             bool first, int tid, int bar)
 {
-    constexpr int KB = (W >= 8 && S == 1) ? 2 * TW_KB : TW_KB;   // stages per synchronisation (the layout reserves the staging rows: tw_make_layout)
-    constexpr int PS = TW_PS(W, S);
+    constexpr int KB = tw_kb(W, S);   // stages per synchronisation (the layout reserves the staging rows: tw_make_layout)
+    constexpr int PS = tw_ps(W, S);
     const int NVP = PS * LF(nb);                                  // padded length of a staging row
     constexpr int NT = 32 * W;
     const int N = NC > 0 ? NC : c.N, n = 2 * N, NV = LF(NV), ns = HS ? c.ns : 0, ms_ = HS ? c.ms : 0;   // HS: the instance carries the code of the state-bound rows
     const double *lin = sm + LF(lin), *sn = sm + LF(sn), *cs = sm + LF(cs), *rr = sm + LF(rr);
     double *wbuf = sm + LF(wb), *Gs = sm + L.Gs;
     const double sqp = sqrt(2.0 * c.q_phi), sqv = sqrt(2.0 * c.q_vx);
-    double G[NPASS][6], qacc[NPASS];
+    double G[6], qacc = 0.0;
 #pragma unroll
-    for (int p = 0; p < NPASS; ++p) {
-        qacc[p] = 0.0;
-#pragma unroll
-        for (int i = 0; i < 6; ++i) G[p][i] = 0.0;
-    }
+    for (int i = 0; i < 6; ++i) G[i] = 0.0;
 #pragma unroll
     for (int s = 0; s < S; ++s)
 #pragma unroll
@@ -369,47 +374,44 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
     for (int k0 = 0; k0 < N; k0 += KB) {
         const int kb = FULLKB ? KB : ((N - k0 < KB) ? N - k0 : KB);
         double *wblk = wbuf + ((LF(nbuf) == 2) ? ((k0 / KB) & 1) * KB * 3 * NVP : 0);
-#pragma unroll
-        for (int p = 0; p < NPASS; ++p) {
-            const int j = p * NT + tid;
-            if (j < n && k0 + kb > (p * NT + (tid & ~31)) / 2) {   // nothing to do before the first column of this warp is born
-                const int c1 = j & 1, jb = j >> 1, pj = TW_PAD(j, PS);
+        const int j = tid;
+        if (j < n && k0 + kb > (tid & ~31) / 2) {   // nothing to do before the first column of this warp is born
+            const int c1 = j & 1, jb = j >> 1, pj = TW_PAD(j, PS);
 #pragma unroll UNR
-                for (int s_i = 0; s_i < kb; ++s_i) {
-                    const int k = k0 + s_i;
-                    const double *r = lin + TG_LIN * k;
-                    double A_[16];
+            for (int s_i = 0; s_i < kb; ++s_i) {
+                const int k = k0 + s_i;
+                const double *r = lin + TG_LIN * k;
+                double A_[16];
 #pragma unroll
-                    for (int i = 0; i < 8; ++i) { const double2 t = tw_ld2(r + 2 * i); A_[2 * i] = t.x; A_[2 * i + 1] = t.y; }
-                    // G_{k+1} = A_k G_k; the column is born at stage jb as a column of B_k (it holds zeros before, A 0 = 0)
-                    const double bm = (jb == k) ? 1.0 : 0.0;
-                    const double b3 = r[16 + c1], b4 = c1 ? r[18] : 0.0, b5 = c1 ? r[19] : 0.0;
-                    const double n0 = G[p][0] + A_[0] * G[p][2] + A_[1] * G[p][3] + A_[2] * G[p][4];
-                    const double n1 = G[p][1] + A_[3] * G[p][2] + A_[4] * G[p][3] + A_[5] * G[p][4];
-                    const double n2 = G[p][2] + A_[6] * G[p][5];
-                    const double n3 = fma(bm, b3, A_[7] * G[p][3] + A_[8] * G[p][4] + A_[9] * G[p][5]);
-                    const double n4 = fma(bm, b4, A_[10] * G[p][3] + A_[11] * G[p][4] + A_[12] * G[p][5]);
-                    const double n5 = fma(bm, b5, A_[13] * G[p][3] + A_[14] * G[p][4] + A_[15] * G[p][5]);
-                    G[p][0] = n0; G[p][1] = n1; G[p][2] = n2; G[p][3] = n3; G[p][4] = n4; G[p][5] = n5;
-                    const int kk = k + 1;
-                    const double wc = sn[kk] * n0 - cs[kk] * n1, wp = sqp * n2, wv = sqv * n3;   // sn, cs carry sqrt(2 q_c)
-                    double *wrow = wblk + s_i * 3 * NVP;
-                    wrow[pj] = wc; wrow[NVP + pj] = wp; wrow[2 * NVP + pj] = wv;
-                    if (first) {
-                        qacc[p] = fma(rr[3 * kk], wc, fma(rr[3 * kk + 1], wp, fma(rr[3 * kk + 2], wv, qacc[p])));
-                        if (jb <= k)
-                            for (int si = 0; si < ns; ++si) {
-                                const int sx = c.sidx[si];
-                                const double gv = (sx == 0) ? n0 : (sx == 1) ? n1 : (sx == 2) ? n2 : (sx == 3) ? n3 : (sx == 4) ? n4 : n5;
-                                Gs[ns * tw_gs_off(k) + si * tw_gs_len(k) + j] = gv;
-                            }
-                    }
+                for (int i = 0; i < 8; ++i) { const double2 t = tw_ld2(r + 2 * i); A_[2 * i] = t.x; A_[2 * i + 1] = t.y; }
+                // G_{k+1} = A_k G_k; the column is born at stage jb as a column of B_k (it holds zeros before, A 0 = 0)
+                const double bm = (jb == k) ? 1.0 : 0.0;
+                const double b3 = r[16 + c1], b4 = c1 ? r[18] : 0.0, b5 = c1 ? r[19] : 0.0;
+                const double n0 = G[0] + A_[0] * G[2] + A_[1] * G[3] + A_[2] * G[4];
+                const double n1 = G[1] + A_[3] * G[2] + A_[4] * G[3] + A_[5] * G[4];
+                const double n2 = G[2] + A_[6] * G[5];
+                const double n3 = fma(bm, b3, A_[7] * G[3] + A_[8] * G[4] + A_[9] * G[5]);
+                const double n4 = fma(bm, b4, A_[10] * G[3] + A_[11] * G[4] + A_[12] * G[5]);
+                const double n5 = fma(bm, b5, A_[13] * G[3] + A_[14] * G[4] + A_[15] * G[5]);
+                G[0] = n0; G[1] = n1; G[2] = n2; G[3] = n3; G[4] = n4; G[5] = n5;
+                const int kk = k + 1;
+                const double wc = sn[kk] * n0 - cs[kk] * n1, wp = sqp * n2, wv = sqv * n3;   // sn, cs carry sqrt(2 q_c)
+                double *wrow = wblk + s_i * 3 * NVP;
+                wrow[pj] = wc; wrow[NVP + pj] = wp; wrow[2 * NVP + pj] = wv;
+                if (first) {
+                    qacc = fma(rr[3 * kk], wc, fma(rr[3 * kk + 1], wp, fma(rr[3 * kk + 2], wv, qacc)));
+                    if (jb <= k)
+                        for (int si = 0; si < ns; ++si) {
+                            const int sx = c.sidx[si];
+                            const double gv = (sx == 0) ? n0 : (sx == 1) ? n1 : (sx == 2) ? n2 : (sx == 3) ? n3 : (sx == 4) ? n4 : n5;
+                            Gs[ns * tw_gs_off(k) + si * tw_gs_len(k) + j] = gv;
+                        }
                 }
-            } else if (j < n) {   // not born in this block of stages: its W entries are zero
-                for (int s_i = 0; s_i < kb; ++s_i) {
-                    double *wrow = wblk + s_i * 3 * NVP;
-                    wrow[TW_PAD(j, PS)] = 0.0; wrow[NVP + TW_PAD(j, PS)] = 0.0; wrow[2 * NVP + TW_PAD(j, PS)] = 0.0;
-                }
+            }
+        } else if (j < n) {   // not born in this block of stages: its W entries are zero
+            for (int s_i = 0; s_i < kb; ++s_i) {
+                double *wrow = wblk + s_i * 3 * NVP;
+                wrow[TW_PAD(j, PS)] = 0.0; wrow[NVP + TW_PAD(j, PS)] = 0.0; wrow[2 * NVP + TW_PAD(j, PS)] = 0.0;
             }
         }
         tw_sync<W>(bar);
@@ -437,11 +439,11 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
     }
     if (first) {
 #pragma unroll
-        for (int p = 0; p < NPASS; ++p) {
-            const int j = p * NT + tid;
+        for (int p = 0; p < 1; ++p) {   // a one-trip loop only because it keeps the generated code unchanged
+            const int j = tid;
             if (j < n) {
                 const int cc = j & 1;
-                sm[LF(q) + j] = qacc[p] + 2.0 * (c.Rs[cc * 2] * sm[LF(uprev)] + c.Rs[cc * 2 + 1] * sm[LF(uprev) + 1]);
+                sm[LF(q) + j] = qacc + 2.0 * (c.Rs[cc * 2] * sm[LF(uprev)] + c.Rs[cc * 2 + 1] * sm[LF(uprev) + 1]);
             }
         }
     }
@@ -648,7 +650,7 @@ __device__ __forceinline__ void tw_sweep_invert_scalar(const DevCfg &c, const WL
     for (int s = 0; s < S; ++s)
         if (mp.act[s] && mp.ro[s] == 0 && mp.co[s] == 0) rp_next = tw_rcp3(a[s][0][0]);
     // shared-space addresses of this thread's operands in the two pivot-row buffers (buffer = pivot parity)
-    constexpr unsigned PS = TW_PS(W, S);
+    constexpr unsigned PS = tw_ps(W, S);
     const unsigned NVP = PS * (unsigned)nb;   // padded pivot rows (TW_PAD)
     const unsigned vb_a = tw_saddr(vb), stride_a = (NVP + 2u) * 8u;
     unsigned ro_a[S], co_a[S];
@@ -741,7 +743,7 @@ __device__ __forceinline__ void tw_sweep_invert(const DevCfg &c, const WLayout &
             for (int r = 0; r < 4; ++r)
                 if (mp.ro[s] + r >= n) a[s][r][r] = 1.0;
     // panel buffer of one pivot group: PB columns of NV (VT[m][i] = A_{i, P_m}) + the PB x PB inverse; two buffers, alternating
-    constexpr unsigned PS = TW_PS(W, S);
+    constexpr unsigned PS = tw_ps(W, S);
     const unsigned NVP = PS * (unsigned)nb;   // padded panel columns (TW_PAD)
     const unsigned vb_a = tw_saddr(vb), stride_a = ((unsigned)PB * NVP + (unsigned)(PB * PB)) * 8u, nv8 = NVP * 8u, dinv_o = (unsigned)PB * nv8;
     unsigned ro_a[S], co_a[S];
@@ -881,7 +883,6 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
                                    const StepTaps &tap, const FusedCtx *fx, int tid, int bar)
 {
     constexpr int NT = 32 * W;
-    constexpr int NPASS = (W == 1 && S >= 2) ? 2 : 1;
     const int N = NC > 0 ? NC : c.N, n = 2 * N, NV = LF(NV), ms = HS ? c.ms : 0, ns = HS ? c.ns : 0;   // HS: the instance carries the code of the state-bound rows
     StepResult res;
     res.status = TG_STATUS_NAN; res.iters = 0; res.objective = 0.0; res.free_end = false;
@@ -1049,7 +1050,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
 
 #pragma unroll 1
     while (!done) {
-        tw_condense<W, S, NPASS, NC, HS>(c, L, sm, mp, a, first, tid, bar);
+        tw_condense<W, S, NC, HS>(c, L, sm, mp, a, first, tid, bar);
         if (first) {
 #pragma unroll
             for (int s = 0; s < S; ++s)
