@@ -123,6 +123,22 @@ typedef struct tg_ref_spec {
     double vref[6];
 } tg_ref_spec;
 
+/* per-problem (step API) / per-trajectory (closed loop) controller settings for the *_ctrl entry points.  The fields mean
+ * what the same fields of tg_config mean, and the symmetric parts of R and Rd are used.  +-TG_INF = absent.  Everything else
+ * stays per handle: N, Ts, model, plant, Jacobian mode, vehicle parameters, noise, the solver settings, and WHICH state
+ * components carry bounds (tg_config's x_lo / x_hi fix that set, and with it the shared-memory layout).  A row may give any
+ * finite or infinite bound on a component the handle bounds.  Rules (checked by the *_host entry points, which return
+ * TG_ERR_INVALID naming the first bad row and field before anything is launched; preconditions of the device-pointer ones):
+ * weights finite and >= 0; R, Rd finite, the symmetric part of R positive definite, that of Rd positive semidefinite;
+ * lo <= hi for every bound; no finite x_lo / x_hi on a state component the handle does not bound. */
+typedef struct tg_ctrl_spec {
+    double q_c, q_phi, q_vx;
+    double R[4], Rd[4];        /* row-major 2x2 */
+    double u_lo[2], u_hi[2];
+    double du_lo[2], du_hi[2];
+    double x_lo[6], x_hi[6];
+} tg_ctrl_spec;
+
 typedef struct tg_handle tg_handle;
 
 const char *tg_last_error(void);
@@ -162,6 +178,13 @@ int tg_mpc_step(tg_handle *h, int B, const double *x0, const double *u_prev, con
 int tg_mpc_step_host(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref,
                      const double *vref, double *u_cmd, int32_t *status, int32_t *iters, double *objective,
                      double *U_opt, double *X_opt, double *y_opt);
+/* the same with problem b solved under its own settings ctrl[b] (tg_ctrl_spec); ctrl == NULL is tg_mpc_step[_host] */
+int tg_mpc_step_ctrl(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref,
+                     const double *vref, const tg_ctrl_spec *ctrl, double *u_cmd, int32_t *status, int32_t *iters,
+                     double *objective, double *U_opt, double *X_opt, double *y_opt);
+int tg_mpc_step_ctrl_host(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref,
+                          const double *vref, const tg_ctrl_spec *ctrl, double *u_cmd, int32_t *status, int32_t *iters,
+                          double *objective, double *U_opt, double *X_opt, double *y_opt);
 
 /* a10 tap -- MPC/main.py:28-47,51-68: reference window for the current state.
  * x0[B][6], spec[B], step index t -> path_ref[B][N+1][3], vref[B][N+1] */
@@ -179,6 +202,15 @@ int tg_closed_loop_host(tg_handle *h, int B, int T, const double *x0, const doub
                         const double *spl_breaks, int64_t n_breaks, const double *spl_coef, int64_t n_coef,
                         int64_t traj_id0, double *clean, double *noisy, double *U, int32_t *status_counts,
                         int64_t *iters_total);
+/* the same with trajectory b controlled under its own settings ctrl[b] (tg_ctrl_spec) for all its T steps;
+ * ctrl == NULL is tg_closed_loop[_host] */
+int tg_closed_loop_ctrl(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                        const tg_ctrl_spec *ctrl, const double *spl_breaks, const double *spl_coef, int64_t traj_id0,
+                        double *clean, double *noisy, double *U, int32_t *status_counts, int64_t *iters_total);
+int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                             const tg_ctrl_spec *ctrl, const double *spl_breaks, int64_t n_breaks, const double *spl_coef,
+                             int64_t n_coef, int64_t traj_id0, double *clean, double *noisy, double *U,
+                             int32_t *status_counts, int64_t *iters_total);
 
 /* ---- scenario + initial-state generation on the device (SURVEY.md 8(d) configs 2, 3, 5): x0 from the ranges of
  * generation_type1.py:260-265 / generation_type2.py:171-174 (Y and phi relative to the reference path), one reference path

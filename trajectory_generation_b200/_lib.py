@@ -83,11 +83,18 @@ REF_SPEC_DTYPE = np.dtype([("path_kind", np.int32), ("vref_kind", np.int32), ("s
                            ("spline_count", np.int32), ("path", np.float64, 4), ("vref", np.float64, 6)], align=True)
 assert REF_SPEC_DTYPE.itemsize == 96
 
+# include/trajgen.h::tg_ctrl_spec: one row of per-problem / per-trajectory controller settings
+CTRL_SPEC_DTYPE = np.dtype([("q_c", np.float64), ("q_phi", np.float64), ("q_vx", np.float64), ("R", np.float64, 4),
+                            ("Rd", np.float64, 4), ("u_lo", np.float64, 2), ("u_hi", np.float64, 2), ("du_lo", np.float64, 2),
+                            ("du_hi", np.float64, 2), ("x_lo", np.float64, 6), ("x_hi", np.float64, 6)], align=True)
+assert CTRL_SPEC_DTYPE.itemsize == 248
+
 # every symbol include/trajgen.h declares
 EXPORTS = (
     "tg_last_error", "tg_version", "tg_default_config", "tg_create", "tg_destroy", "tg_set_stream", "tg_synchronize",
-    "tg_kernel_launches", "tg_info", "tg_tyre_table_info", "tg_linearize", "tg_assemble", "tg_mpc_step", "tg_mpc_step_host", "tg_ref_window",
-    "tg_closed_loop", "tg_closed_loop_host", "tg_default_scenario_rules", "tg_make_scenarios", "tg_make_scenarios_host", "tg_default_type1_rules", "tg_default_type2_rules", "tg_openloop_type1",
+    "tg_kernel_launches", "tg_info", "tg_tyre_table_info", "tg_linearize", "tg_assemble", "tg_mpc_step", "tg_mpc_step_host",
+    "tg_mpc_step_ctrl", "tg_mpc_step_ctrl_host", "tg_ref_window",
+    "tg_closed_loop", "tg_closed_loop_host", "tg_closed_loop_ctrl", "tg_closed_loop_ctrl_host", "tg_default_scenario_rules", "tg_make_scenarios", "tg_make_scenarios_host", "tg_default_type1_rules", "tg_default_type2_rules", "tg_openloop_type1",
     "tg_openloop_type2", "tg_openloop_type1_host", "tg_openloop_type2_host", "tg_write_csv", "tg_merge_csv", "tg_estimator_step", "tg_estimator_step_vjp",
     "tg_estimator_rollout", "tg_plant_rollout", "tg_sensor_noise", "tg_philox_u32", "tg_fma_peak",
     "tg_device_count", "tg_malloc", "tg_malloc_on", "tg_free", "tg_memcpy_h2d", "tg_memcpy_d2h", "tg_malloc_host", "tg_free_host",
@@ -137,9 +144,13 @@ def load():
     L.tg_assemble.argtypes = [vp, ctypes.c_int] + [vp] * 10
     L.tg_mpc_step.argtypes = [vp, ctypes.c_int] + [vp] * 11
     L.tg_mpc_step_host.argtypes = [vp, ctypes.c_int] + [vp] * 11
+    L.tg_mpc_step_ctrl.argtypes = [vp, ctypes.c_int] + [vp] * 12
+    L.tg_mpc_step_ctrl_host.argtypes = [vp, ctypes.c_int] + [vp] * 12
     L.tg_ref_window.argtypes = [vp, ctypes.c_int, vp, vp, vp, vp, ctypes.c_int, vp, vp]
     L.tg_closed_loop.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp]
     L.tg_closed_loop_host.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, i64, vp, i64, i64, vp, vp, vp, vp, vp]
+    L.tg_closed_loop_ctrl.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp]
+    L.tg_closed_loop_ctrl_host.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, i64, vp, i64, i64, vp, vp, vp, vp, vp]
     L.tg_default_scenario_rules.argtypes = [ctypes.POINTER(TgScenarioRules)]
     L.tg_default_scenario_rules.restype = None
     L.tg_make_scenarios.argtypes = [vp, ctypes.c_int, i64, ctypes.POINTER(TgScenarioRules), vp, vp, vp, vp, vp]

@@ -42,6 +42,8 @@ struct StepArgs {
     int stop;
     double *ws_x, *ws_y; int *ws_valid;   // per-problem warm-start state (step API), may be null
     int ppc;                              // problems per CTA
+    const tg_ctrl_spec *ctrl;             // [B] per-problem settings: read by the ctrl instances only (appended last, so that the
+                                          // parameter offsets of every other instance stay as they were)
 };
 
 struct LoopArgs {
@@ -54,6 +56,7 @@ struct LoopArgs {
     int *status_counts;
     long long *iters_total;
     int ppc;   // problems per CTA
+    const tg_ctrl_spec *ctrl;   // [B] per-trajectory settings: read by the ctrl instances only (appended last, like StepArgs::ctrl)
 };
 
 // ------------------------------------------------------------------------------------------------ warp-per-problem kernels
@@ -71,7 +74,9 @@ template <int S> constexpr int tw_regs() { return 128; }
 // P1 = true: the single-problem-per-CTA instance.  Its only barrier id is the constant 1, so the kernel is built with 2
 // hardware barriers instead of 16 (a barrier id held in a register makes ptxas reserve all 16, and an SM has 64: four
 // resident CTAs at most, whatever the registers and the shared memory would allow).
-template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0)>
+// CT = true: the ctrl instance.  Each problem stages its own tg_ctrl_spec (a.ctrl[b]) behind its shared-memory block
+// (tw_stage_ctrl, stride tw_stride(L) + TW_CTRL_DBL) and the solver takes its weights and bounds from there.
+template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0), bool CT = false>
 __global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(tw_regs<S>())
 tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLayout L, const __grid_constant__ StepArgs a)
 {
@@ -79,7 +84,7 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
     constexpr int NT = 32 * W;
     const int P = P1 ? 1 : a.ppc;
     int prob = P1 ? 0 : threadIdx.x / NT, tid = P1 ? threadIdx.x : threadIdx.x % NT;
-    unsigned sm_off = (unsigned)prob * (unsigned)tw_stride(L) * 8u;
+    unsigned sm_off = (unsigned)prob * (unsigned)(tw_stride(L) + (CT ? TW_CTRL_DBL : 0)) * 8u;
     if constexpr (!P1) asm volatile("" : "+r"(tid), "+r"(prob), "+r"(sm_off));   // kept in registers instead of being re-derived at every use
     const int bar = P1 ? TW_BAR_PROB : TW_BAR_PROB + prob;
     double *sm = reinterpret_cast<double *>(reinterpret_cast<char *>(sm_all) + sm_off);
@@ -92,6 +97,7 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
         tw_sync<W>(bar);
         if (tid < 6) sm[LF(x0) + tid] = a.x0[6 * (size_t)b + tid];
         if (tid < 2) sm[LF(uprev) + tid] = a.u_prev[2 * (size_t)b + tid];
+        if constexpr (CT) tw_stage_ctrl(sm + tw_stride(L), a.ctrl + b, tid);
         const double vx0 = a.x0[6 * (size_t)b + 3];
         for (int k = tid; k <= N; k += NT) {
             if (a.path_ref) {
@@ -121,7 +127,8 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
         tap.u = a.u ? a.u + (size_t)b * (2 * n + ms) : nullptr;
         tap.Gs = a.Gs ? a.Gs + (size_t)b * c.ms * n : nullptr;
         tap.stop = a.stop;
-        const StepResult r = tw_step_body<W, S, NC, HS>(c, L, sm, mp, warm, warm_free, tap, nullptr, tid, bar);
+        const StepResult r = tw_step_body<W, S, NC, HS, CT>(c, L, sm, mp, warm, warm_free, tap, nullptr, tid, bar,
+                                                             CT ? reinterpret_cast<const TwCtrl *>(sm + tw_stride(L)) : nullptr);
         if (a.stop) continue;
         const bool ok = (r.status == TG_STATUS_OPTIMAL || r.status == TG_STATUS_OPTIMAL_INACCURATE);  // :261
         const double ud = sm[LF(uprev)], udel = sm[LF(uprev) + 1];
@@ -168,7 +175,7 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
     }
 }
 
-template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0)>
+template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0), bool CT = false>
 __global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(tw_regs<S>())
 tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLayout L, const __grid_constant__ LoopArgs a)
 {
@@ -176,7 +183,7 @@ tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ 
     constexpr int NT = 32 * W;
     const int P = P1 ? 1 : a.ppc;
     int prob = P1 ? 0 : threadIdx.x / NT, tid = P1 ? threadIdx.x : threadIdx.x % NT;
-    unsigned sm_off = (unsigned)prob * (unsigned)tw_stride(L) * 8u;
+    unsigned sm_off = (unsigned)prob * (unsigned)(tw_stride(L) + (CT ? TW_CTRL_DBL : 0)) * 8u;
     if constexpr (!P1) asm volatile("" : "+r"(tid), "+r"(prob), "+r"(sm_off));
     const int bar = P1 ? TW_BAR_PROB : TW_BAR_PROB + prob;
     double *sm = reinterpret_cast<double *>(reinterpret_cast<char *>(sm_all) + sm_off);
@@ -202,6 +209,7 @@ tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ 
         if (tid < 12) sm[LF(spec) + tid] = reinterpret_cast<const double *>(a.spec + b)[tid];   // scenario -> shared memory
         if (tid < 6) { const double v_ = a.x0[6 * (size_t)b + tid]; sm[LF(x0) + tid] = v_; a.clean[(size_t)b * (T + 1) * 6 + tid] = v_; }
         if (tid < 2) sm[LF(uprev) + tid] = a.u0[2 * (size_t)b + tid];
+        if constexpr (CT) tw_stage_ctrl(sm + tw_stride(L), a.ctrl + b, tid);   // the trajectory's settings, once
         if (tid < TG_NUM_STATUS) cnt[tid] = 0;
         if (tid == 0) *itsum = 0;
         bool warm = false, warm_free = false;
@@ -224,7 +232,8 @@ tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ 
                 }
                 break;
             }
-            const StepResult r = tw_step_body<W, S, NC, HS>(c, L, sm, mp, warm, warm_free, tap, &fx, tid, bar);
+            const StepResult r = tw_step_body<W, S, NC, HS, CT>(c, L, sm, mp, warm, warm_free, tap, &fx, tid, bar,
+                                                                 CT ? reinterpret_cast<const TwCtrl *>(sm + tw_stride(L)) : nullptr);
             const bool ok = (r.status == TG_STATUS_OPTIMAL || r.status == TG_STATUS_OPTIMAL_INACCURATE);
             if (tid == 0) { cnt[r.status] += 1; *itsum += r.iters; }
             // shifted warm start for the next step, in the next step's dU coordinates
@@ -421,6 +430,9 @@ struct tg_handle {
     // warp-per-problem kernels (tw_solver.cuh): W warps per problem, S tile blocks per thread
     int W, S;
     TwKernels kern;
+    TwKernels kern_ctrl;      // the ctrl instances of the shape (per-problem settings, tg_mpc_step_ctrl / tg_closed_loop_ctrl)
+    int ppc_max_ctrl;         // most problems per CTA of a ctrl launch (stride smem_ctrl_bytes); 0: the record does not fit
+    size_t smem_ctrl_bytes;   // per-problem shared memory of a ctrl launch: the block plus the staged tg_ctrl_spec
     WLayout WL;
     WLayout Lref;             // layout of the reference-window tap kernel (no state rows, one warp)
     size_t smem_optin;
@@ -485,33 +497,59 @@ static TwKernels tw_kernels(int W, int S, int N, int ms, bool fixed_n)
     if (W == 8 && S == 2) return tw_instance<8, 2, 0, true>();
     return TwKernels{};
 }
+// the ctrl instances (per-problem settings staged in shared memory, template flag CT): run-time horizon with the code of the
+// state-bound rows, on every shape, with the same P1 rule as tw_instance<W, S, 0, true>
+template <int W, int S>
+static TwKernels tw_ctrl_instance()
+{
+    TwKernels k = {};
+    k.step = tw_mpc_step_kernel<W, S, 0, false, true, true>;
+    k.loop = tw_closed_loop_kernel<W, S, 0, false, true, true>;
+    if constexpr (W <= 2) {
+        k.step_p1 = tw_mpc_step_kernel<W, S, 0, true, true, true>;
+        k.loop_p1 = tw_closed_loop_kernel<W, S, 0, true, true, true>;
+    }
+    return k;
+}
+static TwKernels tw_ctrl_kernels(int W, int S)
+{
+    if (W == 1 && S == 1) return tw_ctrl_instance<1, 1>();
+    if (W == 2 && S == 1) return tw_ctrl_instance<2, 1>();
+    if (W == 4 && S == 1) return tw_ctrl_instance<4, 1>();
+    if (W == 8 && S == 1) return tw_ctrl_instance<8, 1>();
+    if (W == 8 && S == 2) return tw_ctrl_instance<8, 2>();
+    return TwKernels{};
+}
 
 // warp-per-problem kernels: problems per CTA.  Resident problems per SM are bounded by registers (512 threads x 128) and
 // shared memory either way; larger CTAs share more instruction fetches, smaller ones spread a small batch over more SMs.
-static int choose_tw_ppc(const tg_handle *h, int B)
+static int choose_tw_ppc(const tg_handle *h, int B, int ppc_max)
 {
-    if (h->ppc_env) return h->ppc_env;
+    if (h->ppc_env) return h->ppc_env < ppc_max ? h->ppc_env : ppc_max;
     // problems with state-bound rows have long, unequal solves (tens to hundreds of ADMM iterations): free-running
     // single-problem CTAs beat problems that wait for one another at every step boundary
     if (h->dc.ms > 0) return 1;
     // measured at N = 20 (two warps per problem): 4 problems per CTA 2.65e7 steps/s (B = 2368), 8 per CTA 2.37e7 (B = 4736),
     // 2 per CTA 2.24e7 and 1 per CTA 1.43e7 (B = 1024): sharing instruction fetches matters, waiting for 7 neighbours costs more
-    int p = h->ppc_max < 4 ? h->ppc_max : 4;
+    int p = ppc_max < 4 ? ppc_max : 4;
     while (p > 1 && (B + p - 1) / p < h->num_sms) p >>= 1;   // every SM gets a CTA before CTAs get wider
     return p < 1 ? 1 : p;
 }
 
 // the single-problem instance where there is no other or where one problem per CTA is chosen, else `multi` with
-// choose_tw_ppc problems per CTA
+// choose_tw_ppc problems per CTA.  A launch with per-problem settings (a.ctrl) runs the ctrl instances, whose problems take
+// smem_ctrl_bytes each.
 template <typename Args>
 static int launch_tw(tg_handle *h, void (*multi)(DevCfg, WLayout, Args), void (*p1)(DevCfg, WLayout, Args), Args &a)
 {
-    int ppc = choose_tw_ppc(h, a.B);
+    const bool ct = a.ctrl != nullptr;
+    if (ct && h->ppc_max_ctrl < 1) return fail(TG_ERR_UNSUPPORTED, "per-problem settings: the record does not fit beside the problem's shared memory");
+    int ppc = choose_tw_ppc(h, a.B, ct ? h->ppc_max_ctrl : h->ppc_max);
     void (*kern)(DevCfg, WLayout, Args) = multi;
     if (p1 && (!multi || ppc == 1)) { kern = p1; ppc = 1; }
     a.ppc = ppc;
     const int threads = 32 * h->W * ppc;
-    const size_t smem = (size_t)ppc * h->smem_bytes;
+    const size_t smem = (size_t)ppc * (ct ? h->smem_ctrl_bytes : h->smem_bytes);
     int per_sm = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
     if (per_sm < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
@@ -642,6 +680,22 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k.loop_p1 ? k.loop_p1 : k.loop, 32 * h->W, stride));
         if (occ < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
         h->grid_cap = occ * h->num_sms;     // resident problems with one problem per CTA
+        // the ctrl instances: the same rules for the stride with the staged record (launch_tw takes the occupancy per launch)
+        h->kern_ctrl = tw_ctrl_kernels(h->W, h->S);
+        const TwKernels &kc = h->kern_ctrl;
+        const size_t stride_c = stride + TW_CTRL_DBL * sizeof(double);
+        h->smem_ctrl_bytes = stride_c;
+        h->ppc_max_ctrl = 0;
+        if (stride_c <= h->smem_optin) {
+            h->ppc_max_ctrl = TW_CTA_THREADS / (32 * h->W);
+            if (h->W > 1) h->ppc_max_ctrl = std::min(h->ppc_max_ctrl, TW_BAR_STEP - TW_BAR_PROB);
+            while (h->ppc_max_ctrl > 1 && (size_t)h->ppc_max_ctrl * stride_c > h->smem_optin) h->ppc_max_ctrl -= 1;
+        }
+        for (const void *f : {(const void *)kc.step, (const void *)kc.step_p1, (const void *)kc.loop, (const void *)kc.loop_p1}) {
+            if (!f) continue;
+            CK(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+            CK(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        }
     }
     h->stream = 0;
     guard.p = nullptr;
@@ -692,7 +746,44 @@ static int launch_step(tg_handle *h, StepArgs &a)
 {
     if (a.B <= 0) return TG_OK;   // empty batch: nothing to do
     CK(cudaSetDevice(h->device));
-    return launch_tw(h, h->kern.step, h->kern.step_p1, a);
+    const TwKernels &k = a.ctrl ? h->kern_ctrl : h->kern;
+    return launch_tw(h, k.step, k.step_p1, a);
+}
+
+// the rules of tg_ctrl_spec (include/trajgen.h), row by row: TG_ERR_INVALID naming the first bad row and field
+static int ctrl_check(const tg_handle *h, int B, const tg_ctrl_spec *ctrl)
+{
+    if (B > 0 && !ctrl) return fail(TG_ERR_INVALID, "bad argument: ctrl is null");
+    bool bounded[6] = {false, false, false, false, false, false};
+    for (int si = 0; si < h->dc.ns; ++si) bounded[h->dc.sidx[si]] = true;
+    for (int b = 0; b < B; ++b) {
+        const tg_ctrl_spec &r = ctrl[b];
+        auto bad = [&](const std::string &field, const char *why) { return fail(TG_ERR_INVALID, "ctrl row " + std::to_string(b) + ": " + field + " " + why); };
+        const double *q[3] = {&r.q_c, &r.q_phi, &r.q_vx};
+        const char *qn[3] = {"q_c", "q_phi", "q_vx"};
+        for (int i = 0; i < 3; ++i)
+            if (!(std::isfinite(*q[i]) && *q[i] >= 0.0)) return bad(qn[i], "must be finite and >= 0");
+        for (int i = 0; i < 4; ++i) {
+            if (!std::isfinite(r.R[i])) return bad("R[" + std::to_string(i) + "]", "must be finite");
+            if (!std::isfinite(r.Rd[i])) return bad("Rd[" + std::to_string(i) + "]", "must be finite");
+        }
+        {   // symmetric parts, as the kernels use them
+            const double a = r.R[0], c = 0.5 * (r.R[1] + r.R[2]), d = r.R[3];
+            if (!(a > 0.0 && a * d - c * c > 0.0)) return bad("R", "symmetric part is not positive definite");
+            const double ad = r.Rd[0], cd = 0.5 * (r.Rd[1] + r.Rd[2]), dd = r.Rd[3];
+            if (!(ad >= 0.0 && dd >= 0.0 && ad * dd - cd * cd >= 0.0)) return bad("Rd", "symmetric part is not positive semidefinite");
+        }
+        for (int i = 0; i < 2; ++i) {
+            if (!(r.u_lo[i] <= r.u_hi[i])) return bad("u_lo[" + std::to_string(i) + "] / u_hi[" + std::to_string(i) + "]", "lo > hi");
+            if (!(r.du_lo[i] <= r.du_hi[i])) return bad("du_lo[" + std::to_string(i) + "] / du_hi[" + std::to_string(i) + "]", "lo > hi");
+        }
+        for (int i = 0; i < 6; ++i) {
+            const std::string f = "x_lo[" + std::to_string(i) + "] / x_hi[" + std::to_string(i) + "]";
+            if (!(r.x_lo[i] <= r.x_hi[i])) return bad(f, "lo > hi");
+            if (!bounded[i] && (r.x_lo[i] > -TG_INF || r.x_hi[i] < TG_INF)) return bad(f, "finite bound on a state component the handle does not bound");
+        }
+    }
+    return TG_OK;
 }
 
 int tg_linearize(tg_handle *h, int B, const double *x0, const double *u_prev, double *A, double *Bm, double *g, double *xbar)
@@ -733,6 +824,13 @@ static int ensure_ws(tg_handle *h, int B)
 int tg_mpc_step(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref, const double *vref,
                 double *u_cmd, int32_t *status, int32_t *iters, double *objective, double *U_opt, double *X_opt, double *y_opt)
 {
+    return tg_mpc_step_ctrl(h, B, x0, u_prev, path_ref, vref, nullptr, u_cmd, status, iters, objective, U_opt, X_opt, y_opt);
+}
+
+int tg_mpc_step_ctrl(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref, const double *vref,
+                     const tg_ctrl_spec *ctrl, double *u_cmd, int32_t *status, int32_t *iters, double *objective, double *U_opt,
+                     double *X_opt, double *y_opt)
+{
     if (!h || B < 0 || (B > 0 && (!x0 || !u_prev || !path_ref || !u_cmd))) return fail(TG_ERR_INVALID, "bad argument");
     CK(cudaSetDevice(h->device));
     int rc = ensure_ws(h, B);
@@ -742,6 +840,7 @@ int tg_mpc_step(tg_handle *h, int B, const double *x0, const double *u_prev, con
     a.B = B; a.x0 = x0; a.u_prev = u_prev; a.path_ref = path_ref; a.vref = vref;
     a.u_cmd = u_cmd; a.status = status; a.iters = iters; a.objective = objective; a.U_opt = U_opt; a.X_opt = X_opt; a.y_opt = y_opt;
     a.ws_x = h->ws_x; a.ws_y = h->ws_y; a.ws_valid = h->ws_valid;
+    a.ctrl = ctrl;
     return launch_step(h, a);
 }
 
@@ -762,6 +861,13 @@ int tg_closed_loop(tg_handle *h, int B, int T, const double *x0, const double *u
                    const double *brk, const double *coef, int64_t traj_id0, double *clean, double *noisy, double *U,
                    int32_t *status_counts, int64_t *iters_total)
 {
+    return tg_closed_loop_ctrl(h, B, T, x0, u0, spec, nullptr, brk, coef, traj_id0, clean, noisy, U, status_counts, iters_total);
+}
+
+int tg_closed_loop_ctrl(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                        const tg_ctrl_spec *ctrl, const double *brk, const double *coef, int64_t traj_id0, double *clean,
+                        double *noisy, double *U, int32_t *status_counts, int64_t *iters_total)
+{
     if (!h || B < 0 || T < 0 || (B > 0 && (!x0 || !u0 || !spec || !clean || !noisy || (T > 0 && !U)))) return fail(TG_ERR_INVALID, "bad argument");
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
@@ -769,7 +875,9 @@ int tg_closed_loop(tg_handle *h, int B, int T, const double *x0, const double *u
     memset(&a, 0, sizeof(a));
     a.B = B; a.T = T; a.x0 = x0; a.u0 = u0; a.spec = spec; a.brk = brk; a.coef = coef; a.traj_id0 = traj_id0;
     a.clean = clean; a.noisy = noisy; a.U = U; a.status_counts = status_counts; a.iters_total = (long long *)iters_total;
-    return launch_tw(h, h->kern.loop, h->kern.loop_p1, a);
+    a.ctrl = ctrl;
+    const TwKernels &k = ctrl ? h->kern_ctrl : h->kern;
+    return launch_tw(h, k.loop, k.loop_p1, a);
 }
 
 int tg_plant_rollout(tg_handle *h, int B, int T, const double *x0, const double *U, double *X)
@@ -1094,14 +1202,23 @@ static int ensure_dstage(tg_handle *h, size_t bytes)
 int tg_mpc_step_host(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref, const double *vref,
                      double *u_cmd, int32_t *status, int32_t *iters, double *objective, double *U_opt, double *X_opt, double *y_opt)
 {
+    return tg_mpc_step_ctrl_host(h, B, x0, u_prev, path_ref, vref, nullptr, u_cmd, status, iters, objective, U_opt, X_opt, y_opt);
+}
+
+int tg_mpc_step_ctrl_host(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref, const double *vref,
+                          const tg_ctrl_spec *ctrl, double *u_cmd, int32_t *status, int32_t *iters, double *objective,
+                          double *U_opt, double *X_opt, double *y_opt)
+{
     if (!h || B < 0 || (B > 0 && (!x0 || !u_prev || !path_ref || !u_cmd))) return fail(TG_ERR_INVALID, "bad argument");
+    if (ctrl) { const int rc = ctrl_check(h, B, ctrl); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
     const int N = h->dc.N, n = h->dc.n, m = h->dc.m;
     const size_t b8 = sizeof(double);
     const size_t s_x0 = (size_t)B * 6 * b8, s_up = (size_t)B * 2 * b8, s_pr = (size_t)B * (N + 1) * 3 * b8, s_vr = (size_t)B * (N + 1) * b8;
     const size_t s_uc = (size_t)B * 2 * b8, s_i = (size_t)B * 4, s_ob = (size_t)B * b8, s_U = (size_t)B * n * b8, s_X = (size_t)B * (N + 1) * 6 * b8, s_y = (size_t)B * m * b8;
-    const size_t total = PAD(s_x0) + PAD(s_up) + PAD(s_pr) + PAD(s_vr) + PAD(s_uc) + 2 * PAD(s_i) + PAD(s_ob) + PAD(s_U) + PAD(s_X) + PAD(s_y) + 4096;
+    const size_t s_ct = ctrl ? (size_t)B * sizeof(tg_ctrl_spec) : 0;
+    const size_t total = PAD(s_x0) + PAD(s_up) + PAD(s_pr) + PAD(s_vr) + PAD(s_uc) + 2 * PAD(s_i) + PAD(s_ob) + PAD(s_U) + PAD(s_X) + PAD(s_y) + PAD(s_ct) + 4096;
     int rc = ensure_dstage(h, total);
     if (rc != TG_OK) return rc;
     Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
@@ -1111,9 +1228,11 @@ int tg_mpc_step_host(tg_handle *h, int B, const double *x0, const double *u_prev
     int32_t *d_st = (int32_t *)ar.take(s_i), *d_it = (int32_t *)ar.take(s_i);
     double *d_ob = (double *)ar.take(s_ob);
     double *d_U = U_opt ? (double *)ar.take(s_U) : nullptr, *d_X = X_opt ? (double *)ar.take(s_X) : nullptr, *d_y = y_opt ? (double *)ar.take(s_y) : nullptr;
+    tg_ctrl_spec *d_ct = ctrl ? (tg_ctrl_spec *)ar.take(s_ct) : nullptr;
     H2D(d_x0, x0, s_x0); H2D(d_up, u_prev, s_up); H2D(d_pr, path_ref, s_pr);
     if (vref) H2D(d_vr, vref, s_vr);
-    rc = tg_mpc_step(h, B, d_x0, d_up, d_pr, d_vr, d_uc, d_st, d_it, d_ob, d_U, d_X, d_y);
+    if (ctrl) H2D(d_ct, ctrl, s_ct);
+    rc = tg_mpc_step_ctrl(h, B, d_x0, d_up, d_pr, d_vr, d_ct, d_uc, d_st, d_it, d_ob, d_U, d_X, d_y);
     if (rc != TG_OK) return rc;
     D2H(u_cmd, d_uc, s_uc);
     if (status) D2H(status, d_st, s_i);
@@ -1138,7 +1257,17 @@ int tg_closed_loop_host(tg_handle *h, int B, int T, const double *x0, const doub
                         const double *brk, int64_t n_breaks, const double *coef, int64_t n_coef, int64_t traj_id0,
                         double *clean, double *noisy, double *U, int32_t *status_counts, int64_t *iters_total)
 {
+    return tg_closed_loop_ctrl_host(h, B, T, x0, u0, spec, nullptr, brk, n_breaks, coef, n_coef, traj_id0, clean, noisy, U,
+                                    status_counts, iters_total);
+}
+
+int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                             const tg_ctrl_spec *ctrl, const double *brk, int64_t n_breaks, const double *coef, int64_t n_coef,
+                             int64_t traj_id0, double *clean, double *noisy, double *U, int32_t *status_counts,
+                             int64_t *iters_total)
+{
     if (!h || B < 0 || T < 0 || (B > 0 && (!x0 || !u0 || !spec || !clean || !noisy || (T > 0 && !U)))) return fail(TG_ERR_INVALID, "bad argument");
+    if (ctrl) { const int rc = ctrl_check(h, B, ctrl); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     {   // the scenario table is host memory here: reject what would send the device out of bounds
         const int64_t n_tab = (brk && coef) ? (n_breaks < n_coef ? n_breaks : n_coef) : 0;
@@ -1163,7 +1292,8 @@ int tg_closed_loop_host(tg_handle *h, int B, int T, const double *x0, const doub
     // of the rows after the kernel disappears.  Pageable buffers are staged through the device arena.
     double *a_cl = (double *)pinned_device_alias(clean), *a_no = (double *)pinned_device_alias(noisy), *a_U = (double *)pinned_device_alias(U);
     const bool direct = a_cl && a_no && (a_U || !s_U);
-    const size_t total = PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + (direct ? 0 : 2 * PAD(s_cl) + PAD(s_U)) + PAD(s_sc) + PAD(s_it) + 4096;
+    const size_t s_ct = ctrl ? (size_t)B * sizeof(tg_ctrl_spec) : 0;
+    const size_t total = PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + (direct ? 0 : 2 * PAD(s_cl) + PAD(s_U)) + PAD(s_sc) + PAD(s_it) + PAD(s_ct) + 4096;
     int rc = ensure_dstage(h, total);
     if (rc != TG_OK) return rc;
     Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
@@ -1174,10 +1304,12 @@ int tg_closed_loop_host(tg_handle *h, int B, int T, const double *x0, const doub
     double *d_U = direct ? a_U : (double *)ar.take(s_U ? s_U : 8);
     int32_t *d_sc = (int32_t *)ar.take(s_sc);
     long long *d_it = (long long *)ar.take(s_it);
+    tg_ctrl_spec *d_ct = ctrl ? (tg_ctrl_spec *)ar.take(s_ct) : nullptr;
     H2D(d_x0, x0, s_x0); H2D(d_u0, u0, s_u0); H2D(d_sp, spec, s_sp);
     if (s_bk) H2D(d_bk, brk, s_bk);
     if (s_cf) H2D(d_cf, coef, s_cf);
-    rc = tg_closed_loop(h, B, T, d_x0, d_u0, d_sp, d_bk, d_cf, traj_id0, d_cl, d_no, d_U, d_sc, (int64_t *)d_it);
+    if (ctrl) H2D(d_ct, ctrl, s_ct);
+    rc = tg_closed_loop_ctrl(h, B, T, d_x0, d_u0, d_sp, d_ct, d_bk, d_cf, traj_id0, d_cl, d_no, d_U, d_sc, (int64_t *)d_it);
     if (rc != TG_OK) return rc;
     if (!direct) {
         D2H(clean, d_cl, s_cl); D2H(noisy, d_no, s_cl);

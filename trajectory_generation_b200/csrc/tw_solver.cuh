@@ -140,6 +140,28 @@ __host__ __device__ constexpr int tw_stride(const WLayout &L) { return tw_even(L
 // offset of a FIXED-part array / a geometry constant
 #define LF(f) (NC > 0 ? TwFix<NC, W>::L.f : L.f)
 
+// Per-problem controller settings (tg_ctrl_spec, with R and Rd replaced by their symmetric parts as tg_create does for DevCfg).
+// The ctrl instances (template flag CT) stage a problem's record in shared memory right after its block, at sm + tw_stride(L),
+// so that their stride is tw_stride(L) + TW_CTRL_DBL; every other instance reads the same fields from DevCfg.  TWC(f) is the
+// field f of whichever applies.
+struct TwCtrl { double q_c, q_phi, q_vx, Rs[4], Rds[4], u_lo[2], u_hi[2], du_lo[2], du_hi[2], x_lo[6], x_hi[6]; };
+static_assert(sizeof(TwCtrl) == sizeof(tg_ctrl_spec), "TwCtrl mirrors tg_ctrl_spec field by field");
+constexpr int TW_CTRL_DBL = tw_even((int)(sizeof(TwCtrl) / sizeof(double)));
+#define TWC(f) (CT ? cr->f : c.f)
+// thread i < 31 stages field i of the record; the caller synchronises before the record is read
+__device__ __forceinline__ void tw_stage_ctrl(double *rec, const tg_ctrl_spec *src, int tid)
+{
+    const double *s = reinterpret_cast<const double *>(src);
+    if (tid < 31) {
+        double v = s[tid];
+        if (tid >= 3 && tid < 11) {   // R, Rd: 0.5 (M_ij + M_ji)
+            const int k = (tid - 3) & 3;
+            v = 0.5 * (v + s[tid - k + (((k & 1) << 1) | (k >> 1))]);
+        }
+        rec[tid] = v;
+    }
+}
+
 // synchronise the threads of ONE problem: a warp for W = 1, a named barrier otherwise
 template <int W>
 __device__ __forceinline__ void tw_sync(int bar)
@@ -333,9 +355,9 @@ __device__ __forceinline__ void tw_ref_window_warp(const DevCfg &c, const WLayou
 // ---------------------------------------------------------------------------------------------------------------- K2
 // H = sum_k W_k' W_k on the tile (W rows carry sqrt(2 q)); optionally q and the state-bound rows.  Thread j owns column j of G
 // (n <= 32 W on every shape).
-template <int W, int S, int NC, bool HS>
+template <int W, int S, int NC, bool HS, bool CT = false>
 __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, double *sm, const TwMap<S> &mp, double (&a)[S][4][4],
-                                            bool first, int tid, int bar)
+                                            bool first, int tid, int bar, const TwCtrl *cr = nullptr)
 {
     constexpr int KB = tw_kb(W, S);   // stages per synchronisation (the layout reserves the staging rows: tw_make_layout)
     constexpr int PS = tw_ps(W, S);
@@ -344,7 +366,7 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
     const int N = NC > 0 ? NC : c.N, n = 2 * N, NV = LF(NV), ns = HS ? c.ns : 0, ms_ = HS ? c.ms : 0;   // HS: the instance carries the code of the state-bound rows
     const double *lin = sm + LF(lin), *sn = sm + LF(sn), *cs = sm + LF(cs), *rr = sm + LF(rr);
     double *wbuf = sm + LF(wb), *Gs = sm + L.Gs;
-    const double sqp = sqrt(2.0 * c.q_phi), sqv = sqrt(2.0 * c.q_vx);
+    const double sqp = sqrt(2.0 * TWC(q_phi)), sqv = sqrt(2.0 * TWC(q_vx));
     double G[6], qacc = 0.0;
 #pragma unroll
     for (int i = 0; i < 6; ++i) G[i] = 0.0;
@@ -443,7 +465,7 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
             const int j = tid;
             if (j < n) {
                 const int cc = j & 1;
-                sm[LF(q) + j] = qacc + 2.0 * (c.Rs[cc * 2] * sm[LF(uprev)] + c.Rs[cc * 2 + 1] * sm[LF(uprev) + 1]);
+                sm[LF(q) + j] = qacc + 2.0 * (TWC(Rs[cc * 2]) * sm[LF(uprev)] + TWC(Rs[cc * 2 + 1]) * sm[LF(uprev) + 1]);
             }
         }
     }
@@ -461,8 +483,8 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
                     const int str = st0 + sr, stc = st0 + sc;
                     if (str < N && stc < N) {
                         double add;
-                        if (sr == sc) add = 2.0 * c.Rs[ar * 2 + ac] + ((str < N - 1) ? 4.0 : 2.0) * c.Rds[ar * 2 + ac];
-                        else add = -2.0 * c.Rds[ar * 2 + ac];
+                        if (sr == sc) add = 2.0 * TWC(Rs[ar * 2 + ac]) + ((str < N - 1) ? 4.0 : 2.0) * TWC(Rds[ar * 2 + ac]);
+                        else add = -2.0 * TWC(Rds[ar * 2 + ac]);
                         a[s][r][cc] += add;
                     }
                 }
@@ -471,7 +493,7 @@ __device__ __forceinline__ void tw_condense(const DevCfg &c, const WLayout &L, d
 #pragma unroll
                 for (int r = 0; r < 2; ++r)
 #pragma unroll
-                    for (int cc = 2; cc < 4; ++cc) a[s][r][cc] += -2.0 * c.Rds[(r & 1) * 2 + (cc & 1)];
+                    for (int cc = 2; cc < 4; ++cc) a[s][r][cc] += -2.0 * TWC(Rds[(r & 1) * 2 + (cc & 1)]);
             }
         }
     }
@@ -870,7 +892,8 @@ __device__ __forceinline__ double2 tw_matvec_sum(const WLayout &L, const double 
 // ------------------------------------------------------------------------------------------------------------ the step
 // On entry shared memory holds x0, uprev and -- unless `fx` is given, in which case the body builds it from the scenario in
 // sm[LF(spec)] -- the reference window (Xr, Yr, Pr, vref); if `warm`, the warm-start dU in sm[LF(x)] and duals in sm[LF(y)].
-// On exit sm[LF(xt)] holds dU*, sm[LF(y)] the duals, and the result is returned to every thread.
+// On exit sm[LF(xt)] holds dU*, sm[LF(y)] the duals, and the result is returned to every thread.  CT: the weights and bounds
+// come from the problem's record `cr` (TwCtrl, in shared memory) instead of DevCfg; nothing else changes.
 //
 // Solver: the OSQP iteration on the condensed problem with per-row rho_i = rho / max_j(a_ij^2 / H_jj).  A solve that starts
 // with every dual at zero (cold start, or a warm start from a solution with no active row: 99.9 % of the steps of the
@@ -878,9 +901,9 @@ __device__ __forceinline__ double2 tw_matvec_sum(const WLayout &L, const double 
 // x <- x - K^-1 (H x + q) with K = H + O(1e-6), so two iterations land on the unconstrained optimum to ~1e-12 -- the EXACT
 // optimum of the QP whenever it satisfies every row, which the standard residual test then certifies (r_prim = 0).  As soon
 // as a row clamps, the solve falls back to the standard settings (rho, alpha) and refactors.
-template <int W, int S, int NC, bool HS>
+template <int W, int S, int NC, bool HS, bool CT = false>
 __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm, const TwMap<S> &mp, bool warm, bool warm_free,
-                                   const StepTaps &tap, const FusedCtx *fx, int tid, int bar)
+                                   const StepTaps &tap, const FusedCtx *fx, int tid, int bar, const TwCtrl *cr = nullptr)
 {
     constexpr int NT = 32 * W;
     const int N = NC > 0 ? NC : c.N, n = 2 * N, NV = LF(NV), ms = HS ? c.ms : 0, ns = HS ? c.ns : 0;   // HS: the instance carries the code of the state-bound rows
@@ -974,7 +997,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
     TG_TICK(0);
 
     // ---------------- K1b: linearise every stage (mpc_6stati.py:175-178) + tracking residuals at xbar (rows carry sqrt(2 q))
-    const double sqc = sqrt(2.0 * c.q_c), sqp = sqrt(2.0 * c.q_phi), sqv = sqrt(2.0 * c.q_vx);
+    const double sqc = sqrt(2.0 * TWC(q_c)), sqp = sqrt(2.0 * TWC(q_phi)), sqv = sqrt(2.0 * TWC(q_vx));
     {
         const double ud = sm[LF(uprev)], udel = sm[LF(uprev) + 1];
         for (int k = tid; k < N; k += NT) {
@@ -1006,7 +1029,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
         for (int k = NT - 1 - tid; k <= N; k += NT) { sn[k] *= sqc; cs[k] *= sqc; }
         if (!fx) {   // constant term: stage costs at xbar + N u_prev' R u_prev (only the step API reports the objective)
             double c0 = tw_reduce_sum<W>(c0_part, red, tid, bar);
-            c0 += (double)N * (ud * (c.Rs[0] * ud + c.Rs[1] * udel) + udel * (c.Rs[2] * ud + c.Rs[3] * udel));
+            c0 += (double)N * (ud * (TWC(Rs[0]) * ud + TWC(Rs[1]) * udel) + udel * (TWC(Rs[2]) * ud + TWC(Rs[3]) * udel));
             if (tid == 0) misc[M_C0] = c0;
         }
     }
@@ -1022,8 +1045,8 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
 
     // ---------------- K2 + bounds + rho, K3: factor; ADMM.  The factor pass is re-entered when rho changes.
     double a[S][4][4];
-    const double lb0 = c.u_lo[0] - sm[LF(uprev)], ub0 = c.u_hi[0] - sm[LF(uprev)];
-    const double lb1 = c.u_lo[1] - sm[LF(uprev) + 1], ub1 = c.u_hi[1] - sm[LF(uprev) + 1];
+    const double lb0 = TWC(u_lo[0]) - sm[LF(uprev)], ub0 = TWC(u_hi[0]) - sm[LF(uprev)];
+    const double lb1 = TWC(u_lo[1]) - sm[LF(uprev) + 1], ub1 = TWC(u_hi[1]) - sm[LF(uprev) + 1];
     const double sigma = c.sigma;
     bool x0_infeasible = false;
     for (int si = 0; si < ns; ++si) {
@@ -1034,7 +1057,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
         // outside a bound that the previous step's plan touched -- so the same tolerance applies here, whatever tighter
         // tolerance this library's own iteration runs at.
         const double ea = fmax(c.eps_abs, 1e-5), er = fmax(c.eps_rel, 1e-5);
-        if (xv < c.x_lo[sx] - (ea + er * fmax(fabs(xv), fabs(c.x_lo[sx]))) || xv > c.x_hi[sx] + (ea + er * fmax(fabs(xv), fabs(c.x_hi[sx]))))
+        if (xv < TWC(x_lo[sx]) - (ea + er * fmax(fabs(xv), fabs(TWC(x_lo[sx])))) || xv > TWC(x_hi[sx]) + (ea + er * fmax(fabs(xv), fabs(TWC(x_hi[sx])))))
             x0_infeasible = true;
     }
     bool free_mode = (!warm || warm_free) && c.free_mode;
@@ -1050,7 +1073,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
 
 #pragma unroll 1
     while (!done) {
-        tw_condense<W, S, NC, HS>(c, L, sm, mp, a, first, tid, bar);
+        tw_condense<W, S, NC, HS, CT>(c, L, sm, mp, a, first, tid, bar, cr);
         if (first) {
 #pragma unroll
             for (int s = 0; s < S; ++s)
@@ -1069,8 +1092,8 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
             for (int i = tid; i < ms; i += NT) {
                 const int nsd = ns > 0 ? ns : 1, kk = i / nsd + 1, sx = c.sidx[i % nsd];
                 const double xb = xbar[6 * kk + sx];
-                ls[i] = (c.x_lo[sx] <= -TG_INF) ? -TG_INF : c.x_lo[sx] - xb;
-                us[i] = (c.x_hi[sx] >= TG_INF) ? TG_INF : c.x_hi[sx] - xb;
+                ls[i] = (TWC(x_lo[sx]) <= -TG_INF) ? -TG_INF : TWC(x_lo[sx]) - xb;
+                us[i] = (TWC(x_hi[sx]) >= TG_INF) ? TG_INF : TWC(x_hi[sx]) - xb;
                 double mx = 0.0;
                 const double *grow = Gs + ns * tw_gs_off(kk - 1) + (i % nsd) * tw_gs_len(kk - 1);
                 for (int j = 0; j < 2 * kk; ++j) { const double gij = grow[j]; mx = fmax(mx, gij * gij / dH[j]); }
@@ -1102,7 +1125,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
             if (tap.l) {
                 for (int i = tid; i < n; i += NT) {
                     tap.l[i] = (i & 1) ? lb1 : lb0; tap.u[i] = (i & 1) ? ub1 : ub0;
-                    tap.l[n + i] = c.du_lo[i & 1]; tap.u[n + i] = c.du_hi[i & 1];
+                    tap.l[n + i] = TWC(du_lo[i & 1]); tap.u[n + i] = TWC(du_hi[i & 1]);
                 }
                 for (int i = tid; i < ms; i += NT) { tap.l[2 * n + i] = ls[i]; tap.u[2 * n + i] = us[i]; }
             }
@@ -1128,7 +1151,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
                     const double2 xj = tw_ld2(x + j0);
                     const double2 xp = (tid > 0) ? tw_ld2(x + j0 - 2) : make_double2(0.0, 0.0);
                     tw_st2(z + j0, tg_clamp(xj.x, lb0, ub0), tg_clamp(xj.y, lb1, ub1));
-                    tw_st2(z + n + j0, tg_clamp(xj.x - xp.x, c.du_lo[0], c.du_hi[0]), tg_clamp(xj.y - xp.y, c.du_lo[1], c.du_hi[1]));
+                    tw_st2(z + n + j0, tg_clamp(xj.x - xp.x, TWC(du_lo[0]), TWC(du_hi[0])), tg_clamp(xj.y - xp.y, TWC(du_lo[1]), TWC(du_hi[1])));
                 }
                 for (int r0 = 0; r0 < ms; r0 += NT >> geo.lg_tpr) {
                     const int r_ = r0 + (tid >> geo.lg_tpr);
@@ -1216,7 +1239,7 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
                     const double2 zo = tw_ld2(z + n + j0), yo = tw_ld2(y + n + j0), ri = tw_ld2(rinv + n + j0), r_ = tw_ld2(rho + n + j0);
                     const double zr0 = alpha * zt0 + (1.0 - alpha) * zo.x, zr1 = alpha * zt1 + (1.0 - alpha) * zo.y;
                     const double t0 = zr0 + yo.x * ri.x, t1 = zr1 + yo.y * ri.y;
-                    const double zn0 = tg_clamp(t0, c.du_lo[0], c.du_hi[0]), zn1 = tg_clamp(t1, c.du_lo[1], c.du_hi[1]);
+                    const double zn0 = tg_clamp(t0, TWC(du_lo[0]), TWC(du_hi[0])), zn1 = tg_clamp(t1, TWC(du_lo[1]), TWC(du_hi[1]));
                     const double yn0 = yo.x + r_.x * (zr0 - zn0), yn1 = yo.y + r_.y * (zr1 - zn1);
                     clamped = clamped || zn0 != t0 || zn1 != t1;
                     dyr2 = make_double2(yn0 - yo.x, yn1 - yo.y);
@@ -1226,8 +1249,8 @@ __device__ StepResult tw_step_body(const DevCfg &c, const WLayout &L, double *sm
                     if (check) {
                         tw_st2(dyr + j0, dyr2.x, dyr2.y);
                         ndy = fmax(ndy, fmax(fabs(dyr2.x), fabs(dyr2.y)));
-                        cert += (dyr2.x > 0.0 ? c.du_hi[0] : c.du_lo[0]) * dyr2.x + (dyr2.y > 0.0 ? c.du_hi[1] : c.du_lo[1]) * dyr2.y;
-                        near = near || fmin(fmin(zt0 - c.du_lo[0], c.du_hi[0] - zt0), fmin(zt1 - c.du_lo[1], c.du_hi[1] - zt1)) < TW_POLISH_MARGIN;
+                        cert += (dyr2.x > 0.0 ? TWC(du_hi[0]) : TWC(du_lo[0])) * dyr2.x + (dyr2.y > 0.0 ? TWC(du_hi[1]) : TWC(du_lo[1])) * dyr2.y;
+                        near = near || fmin(fmin(zt0 - TWC(du_lo[0]), TWC(du_hi[0]) - zt0), fmin(zt1 - TWC(du_lo[1]), TWC(du_hi[1]) - zt1)) < TW_POLISH_MARGIN;
                     }
                 }
             }

@@ -200,7 +200,7 @@ class ClosedLoopGenerator(BatchedMPC):
     #: generate() streams batches whose result rows exceed this many bytes through two page-locked chunk buffers
     STREAM_BYTES = 1 << 30
 
-    def generate(self, x0, u0, scenarios, T, traj_id0=0, out=None, pinned=True, chunk=None):
+    def generate(self, x0, u0, scenarios, T, traj_id0=0, out=None, pinned=True, chunk=None, ctrl=None):
         """x0[B,6], u0[B,2], scenarios (len B), T steps -> dict(clean[B,T+1,6], noisy[B,T+1,6], U[B,T,2],
         status_counts[B,6], iters_total[B]).  Row 0 of clean is x0; noise seed = base + traj_id0 + i.
         The result arrays are page-locked by default (``pinned``), so the kernel writes its rows straight into them
@@ -208,23 +208,29 @@ class ClosedLoopGenerator(BatchedMPC):
         the buffers of an earlier call (see ``alloc_result``).  Page-locking gigabytes takes longer than generating them, so
         a batch whose rows exceed STREAM_BYTES (or any batch when ``chunk`` is given) is generated in chunks through two
         cached page-locked chunk buffers (generate_chunks) and gathered into ordinary arrays by host threads while the next
-        chunk computes."""
+        chunk computes.  ``ctrl``: a [B] table of per-trajectory weights and bounds (``ctrl_table``), held for all T steps;
+        None = the handle's settings for every trajectory."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B, T = x0.shape[0], int(T)
         u0 = self._arr(np.asarray(u0, float).reshape(-1, 2), (B, 2))
         if len(scenarios) != B:
             raise ValueError("one scenario per trajectory required")
+        ctrl = None if ctrl is None else self._ctrl_arg(ctrl, B)
         row_bytes = (2 * (T + 1) * 6 + T * 2) * 8
         if out is None and (chunk is not None or (pinned and B * row_bytes > self.STREAM_BYTES)):
-            return self._generate_streamed(x0, u0, scenarios, T, traj_id0, chunk)
+            return self._generate_streamed(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl)
         spec = np.ascontiguousarray(scenarios.spec)
         brk, coef = scenarios.tables()
         if out is None:
             out = self.alloc_result(B, T, pinned)
         elif out["clean"].shape != (B, T + 1, 6) or out["U"].shape != (B, T, 2):
             raise ValueError("`out` was allocated for another batch size / horizon")
-        _lib.check(_lib.load().tg_closed_loop_host(
-            self._h, B, T, _lib.ptr(x0), _lib.ptr(u0), spec.ctypes.data, _lib.ptr(brk) if len(brk) else None,
+        L = _lib.load()
+        head = (self._h, B, T, _lib.ptr(x0), _lib.ptr(u0), spec.ctypes.data)
+        if ctrl is not None:
+            head += (ctrl.ctypes.data,)
+        _lib.check((L.tg_closed_loop_host if ctrl is None else L.tg_closed_loop_ctrl_host)(
+            *head, _lib.ptr(brk) if len(brk) else None,
             len(brk), _lib.ptr(coef) if len(coef) else None, len(coef), int(traj_id0),
             _lib.ptr(out["clean"]), _lib.ptr(out["noisy"]), _lib.ptr(out["U"]), _lib.ptr(out["status_counts"]),
             _lib.ptr(out["iters_total"])))
@@ -245,15 +251,17 @@ class ClosedLoopGenerator(BatchedMPC):
             self._chunk_key = key
         return self._chunk_bufs
 
-    def generate_chunks(self, x0, u0, scenarios, T, traj_id0=0, chunk=None):
+    def generate_chunks(self, x0, u0, scenarios, T, traj_id0=0, chunk=None, ctrl=None):
         """Iterator over a large batch: yields (lo, hi, res) with res = the result dict of trajectories lo .. hi - 1 as views of
         one of two page-locked chunk buffers.  The GPU computes chunk k + 1 (a host thread sits in tg_closed_loop_host, which
         releases the GIL) while the caller consumes chunk k; a yielded view stays valid until the caller asks for the
-        next-but-one chunk.  ``chunk`` defaults to 8192 trajectories (1.1 GB of rows at T = 1200)."""
+        next-but-one chunk.  ``chunk`` defaults to 8192 trajectories (1.1 GB of rows at T = 1200).  ``ctrl`` ([B] table, see
+        ``generate``) is sliced with the scenarios."""
         from concurrent.futures import ThreadPoolExecutor
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         u0 = np.ascontiguousarray(np.asarray(u0, float).reshape(-1, 2))
         B, T = x0.shape[0], int(T)
+        ctrl = None if ctrl is None else self._ctrl_arg(ctrl, B)   # checked before the first chunk is launched
         chunk = int(chunk) if chunk else 8192
         nb = min(chunk, B)
         bufs = self._chunk_buffers(nb, T)
@@ -262,7 +270,8 @@ class ClosedLoopGenerator(BatchedMPC):
         def run(k):
             lo = los[k]; hi = min(lo + chunk, B)
             res = {k_: v[:hi - lo] for k_, v in bufs[k % 2].items()}
-            ClosedLoopGenerator.generate(self, x0[lo:hi], u0[lo:hi], scenarios.slice(lo, hi), T, traj_id0 + lo, out=res)
+            ClosedLoopGenerator.generate(self, x0[lo:hi], u0[lo:hi], scenarios.slice(lo, hi), T, traj_id0 + lo, out=res,
+                                         ctrl=None if ctrl is None else ctrl[lo:hi])
             return lo, hi, res
 
         with ThreadPoolExecutor(1) as ex:
@@ -273,12 +282,12 @@ class ClosedLoopGenerator(BatchedMPC):
                     fut = ex.submit(run, k + 1)          # into the buffer the caller released when it asked for this chunk
                 yield item
 
-    def _generate_streamed(self, x0, u0, scenarios, T, traj_id0, chunk, n_copy_threads=4):
+    def _generate_streamed(self, x0, u0, scenarios, T, traj_id0, chunk, n_copy_threads=4, ctrl=None):
         from concurrent.futures import ThreadPoolExecutor
         B = x0.shape[0]
         out = self.alloc_result(B, T, pinned=False)
         with ThreadPoolExecutor(n_copy_threads) as pool:
-            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk):
+            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl):
                 jobs = []
                 step = max(1, (hi - lo + n_copy_threads - 1) // n_copy_threads)
                 for a in range(0, hi - lo, step):        # ndarray copies release the GIL: first touch + copy on several cores
@@ -291,12 +300,13 @@ class ClosedLoopGenerator(BatchedMPC):
         return out
 
     def generate_to_csv(self, x0, u0, scenarios, T, clean_path, noisy_path, traj_id0=0, chunk=8192, keep=False, n_threads=0,
-                        csv_ids=None):
+                        csv_ids=None, ctrl=None):
         """generate() in chunks of ``chunk`` trajectories with the dataset files written as it goes (the reference holds
         every DataFrame in RAM and writes once at the end, generation_type2.py:166,216-218,319-322): while the GPU computes
         chunk k + 1 into one set of pinned buffers, the host formats chunk k from the other (tg_write_csv, all cores,
         appending).  ``csv_ids``: write only the first csv_ids trajectories to the files (BASELINE config 5: CSV for the
-        first 5 000 ids, the rest stays binary).  Returns dict(status_counts[B,6], iters_total[B]) (+ the rows if ``keep``)."""
+        first 5 000 ids, the rest stays binary).  ``ctrl``: per-trajectory settings as in ``generate``.  Returns
+        dict(status_counts[B,6], iters_total[B]) (+ the rows if ``keep``)."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B, T = x0.shape[0], int(T)
         n_csv = B if csv_ids is None else min(int(csv_ids), B)
@@ -306,7 +316,7 @@ class ClosedLoopGenerator(BatchedMPC):
         from concurrent.futures import ThreadPoolExecutor
         with ThreadPoolExecutor(1) as writer:                # one writer: chunks are appended in order
             pending = []
-            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk):
+            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl):
                 out["status_counts"][lo:hi] = res["status_counts"]; out["iters_total"][lo:hi] = res["iters_total"]
                 if keep:
                     for k_ in ("clean", "noisy", "U"):

@@ -61,6 +61,40 @@ def make_config(Ts=0.02, N=20, params=None, q_c=6.0, q_phi=0.5, q_vx=0.5, R=None
     return cfg
 
 
+
+
+def check_ctrl_table(table, bounded):
+    """The rules of include/trajgen.h::tg_ctrl_spec for every row of ``table`` (CTRL_SPEC_DTYPE); ``bounded[6]`` says which
+    state components the handle bounds.  Raises ValueError naming the first bad row and field, as the C entry points do."""
+    t = table
+    checks = []                                             # (field, reason, bad[B]) in the order the library checks them
+    for f in ("q_c", "q_phi", "q_vx"):
+        checks.append((f, "must be finite and >= 0", ~(np.isfinite(t[f]) & (t[f] >= 0.0))))
+    for i in range(4):
+        checks.append((f"R[{i}]", "must be finite", ~np.isfinite(t["R"][:, i])))
+        checks.append((f"Rd[{i}]", "must be finite", ~np.isfinite(t["Rd"][:, i])))
+    with np.errstate(invalid="ignore", over="ignore"):
+        R, Rd = t["R"], t["Rd"]
+        a, c, d_ = R[:, 0], 0.5 * (R[:, 1] + R[:, 2]), R[:, 3]
+        checks.append(("R", "symmetric part is not positive definite", ~((a > 0.0) & (a * d_ - c * c > 0.0))))
+        a, c, d_ = Rd[:, 0], 0.5 * (Rd[:, 1] + Rd[:, 2]), Rd[:, 3]
+        checks.append(("Rd", "symmetric part is not positive semidefinite", ~((a >= 0.0) & (d_ >= 0.0) & (a * d_ - c * c >= 0.0))))
+    for i in range(2):
+        for lo, hi in (("u_lo", "u_hi"), ("du_lo", "du_hi")):
+            checks.append((f"{lo}[{i}] / {hi}[{i}]", "lo > hi", ~(t[lo][:, i] <= t[hi][:, i])))
+    for i in range(6):
+        f = f"x_lo[{i}] / x_hi[{i}]"
+        checks.append((f, "lo > hi", ~(t["x_lo"][:, i] <= t["x_hi"][:, i])))
+        if not bounded[i]:
+            checks.append((f, "finite bound on a state component the handle does not bound",
+                           (t["x_lo"][:, i] > -_lib.TG_INF) | (t["x_hi"][:, i] < _lib.TG_INF)))
+    first = min((int(np.argmax(bad)) for _, _, bad in checks if bad.any()), default=None)
+    if first is not None:
+        field, why = next((f, w) for f, w, bad in checks if bad[first])
+        raise ValueError(f"ctrl row {first}: {field} {why}")
+    return table
+
+
 class BatchedMPC:
     """B independent MPC problems per call on one B200.  Construction takes mpc_step's keyword
     arguments; ``step`` takes the per-problem arrays."""
@@ -113,6 +147,49 @@ class BatchedMPC:
         u, a, b = ctypes.c_int32(), ctypes.c_double(), ctypes.c_double()
         _lib.check(_lib.load().tg_tyre_table_info(self._h, ctypes.byref(u), ctypes.byref(a), ctypes.byref(b)))
         return {"in_use": bool(u.value & 1), "atan_in_use": bool(u.value & 2), "max_value_err": a.value, "max_slope_err": b.value}
+
+    # -- per-problem settings
+    @property
+    def bounded_states(self):
+        """which of the six state components this handle bounds (tg_config's finite x_lo / x_hi): the components on which a
+        ctrl table may set bounds"""
+        return tuple(self.cfg.x_lo[i] > -_lib.TG_INF or self.cfg.x_hi[i] < _lib.TG_INF for i in range(6))
+
+    def ctrl_table(self, B, **fields):
+        """A [B] table of per-problem controller settings (CTRL_SPEC_DTYPE, include/trajgen.h::tg_ctrl_spec) for ``step`` and
+        ``ClosedLoopGenerator.generate``.  Every row starts as this handle's own settings; a keyword overrides a field with an
+        array that broadcasts to [B] (q_c, q_phi, q_vx) or [B, k] (R and Rd: k = 4 row-major, or [..., 2, 2]; u_lo, u_hi,
+        du_lo, du_hi: 2; x_lo, x_hi: 6).  A bound of +-TG_INF (or +-inf) is absent.  Raises ValueError naming the first row
+        that breaks a rule of tg_ctrl_spec."""
+        B = int(B)
+        t = np.zeros(B, _lib.CTRL_SPEC_DTYPE)
+        cfg = self.cfg
+        for f in _lib.CTRL_SPEC_DTYPE.names:
+            v = getattr(cfg, f)
+            t[f] = v if isinstance(v, float) else np.asarray(v[:], float)
+        for f, v in fields.items():
+            if f not in _lib.CTRL_SPEC_DTYPE.names:
+                raise TypeError(f"unknown ctrl field {f!r}")
+            v = np.asarray(v, float)
+            shape = _lib.CTRL_SPEC_DTYPE[f].shape
+            if f in ("R", "Rd") and v.shape[-2:] == (2, 2):
+                v = v.reshape(v.shape[:-2] + (4,))
+            if f in ("x_lo", "x_hi"):
+                v = np.clip(v, -_lib.TG_INF, _lib.TG_INF)
+            try:
+                t[f] = np.broadcast_to(v, (B,) + shape)
+            except ValueError:
+                raise ValueError(f"ctrl field {f}: shape {v.shape} does not broadcast to {(B,) + shape}") from None
+        return check_ctrl_table(t, self.bounded_states)
+
+    def _ctrl_arg(self, ctrl, B):
+        """a caller's ctrl table, checked: a C-contiguous [B] array of CTRL_SPEC_DTYPE that satisfies tg_ctrl_spec's rules"""
+        t = np.ascontiguousarray(ctrl)
+        if t.dtype != _lib.CTRL_SPEC_DTYPE:
+            raise ValueError("ctrl must be a table of CTRL_SPEC_DTYPE (see ctrl_table)")
+        if t.shape != (B,):
+            raise ValueError(f"ctrl: expected {B} rows, got shape {t.shape}")
+        return check_ctrl_table(t, self.bounded_states)
 
     # -- host-array API
     @staticmethod
@@ -171,22 +248,27 @@ class BatchedMPC:
                 "c0": self._from_device(oc, (B,)), "l": self._from_device(ol, (B, m)), "u": self._from_device(ou, (B, m)),
                 "Gs": self._from_device(oG, (B, ms, n)) if ms else np.zeros((B, 0, n))}
 
-    def step(self, x0, u_prev, path_ref, vref=None, want_trajectory=True):
+    def step(self, x0, u_prev, path_ref, vref=None, want_trajectory=True, ctrl=None):
         """Batched mpc_step.  x0[B,6], u_prev[B,2], path_ref[B,N+1,3], vref[B,N+1] | None
         -> dict(u_cmd[B,2], status[B] int32, iters[B], objective[B], U_opt[B,N,2], X_opt[B,N+1,6], y_opt[B,m]).
-        Rows whose status is not accepted carry u_cmd = u_prev and NaN in the optional outputs."""
+        Rows whose status is not accepted carry u_cmd = u_prev and NaN in the optional outputs.  ``ctrl``: a [B] table of
+        per-problem weights and bounds (``ctrl_table``); None = the handle's settings for every problem."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B, N = x0.shape[0], self.N
         u_prev = self._arr(np.asarray(u_prev, float).reshape(-1, 2), (B, 2))
         path_ref = self._arr(path_ref, (B, N + 1, 3))                 # :151
         vref = None if vref is None else self._arr(vref, (B, N + 1))
+        ctrl = None if ctrl is None else self._ctrl_arg(ctrl, B)
         out = {"u_cmd": np.empty((B, 2)), "status": np.empty(B, np.int32), "iters": np.empty(B, np.int32),
                "objective": np.empty(B)}
         if want_trajectory:
             out.update(U_opt=np.empty((B, N, 2)), X_opt=np.empty((B, N + 1, 6)), y_opt=np.empty((B, self.m)))
-        _lib.check(_lib.load().tg_mpc_step_host(
-            self._h, B, _lib.ptr(x0), _lib.ptr(u_prev), _lib.ptr(path_ref), _lib.ptr(vref),
-            _lib.ptr(out["u_cmd"]), _lib.ptr(out["status"]), _lib.ptr(out["iters"]), _lib.ptr(out["objective"]),
+        L = _lib.load()
+        args = (self._h, B, _lib.ptr(x0), _lib.ptr(u_prev), _lib.ptr(path_ref), _lib.ptr(vref))
+        if ctrl is not None:
+            args += (ctrl.ctypes.data,)
+        _lib.check((L.tg_mpc_step_host if ctrl is None else L.tg_mpc_step_ctrl_host)(
+            *args, _lib.ptr(out["u_cmd"]), _lib.ptr(out["status"]), _lib.ptr(out["iters"]), _lib.ptr(out["objective"]),
             _lib.ptr(out.get("U_opt")), _lib.ptr(out.get("X_opt")), _lib.ptr(out.get("y_opt"))))
         return out
 
