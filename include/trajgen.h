@@ -127,10 +127,10 @@ typedef struct tg_ref_spec {
  * what the same fields of tg_config mean, and the symmetric parts of R and Rd are used.  +-TG_INF = absent.  Everything else
  * stays per handle: N, Ts, model, plant, Jacobian mode, vehicle parameters, noise, the solver settings, and WHICH state
  * components carry bounds (tg_config's x_lo / x_hi fix that set, and with it the shared-memory layout).  A row may give any
- * finite or infinite bound on a component the handle bounds.  Rules (checked by the *_host entry points, which return
- * TG_ERR_INVALID naming the first bad row and field before anything is launched; preconditions of the device-pointer ones):
- * weights finite and >= 0; R, Rd finite, the symmetric part of R positive definite, that of Rd positive semidefinite;
- * lo <= hi for every bound; no finite x_lo / x_hi on a state component the handle does not bound. */
+ * finite or infinite bound on a component the handle bounds.  Rules (checked by tg_check_ctrl and by the *_host entry points,
+ * which return TG_ERR_INVALID naming the first bad row and field before anything is launched; preconditions of the
+ * device-pointer ones): weights finite and >= 0; R, Rd finite, the symmetric part of R positive definite, that of Rd positive
+ * semidefinite; lo <= hi for every bound; no finite x_lo / x_hi on a state component the handle does not bound. */
 typedef struct tg_ctrl_spec {
     double q_c, q_phi, q_vx;
     double R[4], Rd[4];        /* row-major 2x2 */
@@ -138,6 +138,11 @@ typedef struct tg_ctrl_spec {
     double du_lo[2], du_hi[2];
     double x_lo[6], x_hi[6];
 } tg_ctrl_spec;
+
+/* the rules of tg_ctrl_spec for the host table ctrl[B], for a handle that bounds state component i when bit i of
+ * bounded_states is set.  TG_OK, or TG_ERR_INVALID with tg_last_error() = "ctrl row b: <field> <why>" for the first bad row.
+ * Needs no handle and no GPU. */
+int tg_check_ctrl(int B, const tg_ctrl_spec *ctrl, uint32_t bounded_states);
 
 typedef struct tg_handle tg_handle;
 

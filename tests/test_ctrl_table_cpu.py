@@ -1,5 +1,6 @@
-"""CPU: the NumPy mirror of tg_ctrl_spec has the header's layout, and the Python checks of a ctrl table follow the rules the
-header states (the C entry points apply the same rules; tests/test_gpu_ctrl_table.py checks both on the GPU)."""
+"""CPU: the NumPy mirror of tg_ctrl_spec has the header's layout, and the library's checks of a ctrl table (tg_check_ctrl,
+which check_ctrl_table and the *_host entry points call; it needs no GPU) follow the rules the header states
+(tests/test_gpu_ctrl_table.py checks the entry points on the GPU)."""
 import os
 import re
 

@@ -93,7 +93,7 @@ assert CTRL_SPEC_DTYPE.itemsize == 248
 EXPORTS = (
     "tg_last_error", "tg_version", "tg_default_config", "tg_create", "tg_destroy", "tg_set_stream", "tg_synchronize",
     "tg_kernel_launches", "tg_info", "tg_tyre_table_info", "tg_linearize", "tg_assemble", "tg_mpc_step", "tg_mpc_step_host",
-    "tg_mpc_step_ctrl", "tg_mpc_step_ctrl_host", "tg_ref_window",
+    "tg_mpc_step_ctrl", "tg_mpc_step_ctrl_host", "tg_check_ctrl", "tg_ref_window",
     "tg_closed_loop", "tg_closed_loop_host", "tg_closed_loop_ctrl", "tg_closed_loop_ctrl_host", "tg_default_scenario_rules", "tg_make_scenarios", "tg_make_scenarios_host", "tg_default_type1_rules", "tg_default_type2_rules", "tg_openloop_type1",
     "tg_openloop_type2", "tg_openloop_type1_host", "tg_openloop_type2_host", "tg_write_csv", "tg_merge_csv", "tg_estimator_step", "tg_estimator_step_vjp",
     "tg_estimator_rollout", "tg_plant_rollout", "tg_sensor_noise", "tg_philox_u32", "tg_fma_peak",
@@ -146,6 +146,7 @@ def load():
     L.tg_mpc_step_host.argtypes = [vp, ctypes.c_int] + [vp] * 11
     L.tg_mpc_step_ctrl.argtypes = [vp, ctypes.c_int] + [vp] * 12
     L.tg_mpc_step_ctrl_host.argtypes = [vp, ctypes.c_int] + [vp] * 12
+    L.tg_check_ctrl.argtypes = [ctypes.c_int, vp, ctypes.c_uint32]
     L.tg_ref_window.argtypes = [vp, ctypes.c_int, vp, vp, vp, vp, ctypes.c_int, vp, vp]
     L.tg_closed_loop.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp]
     L.tg_closed_loop_host.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, i64, vp, i64, i64, vp, vp, vp, vp, vp]

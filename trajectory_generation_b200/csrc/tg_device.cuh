@@ -21,6 +21,11 @@
 #define TG_TAB_ROWS (TG_TAB_NI + 1)
 #define TG_ATAN_ROWS (TG_ATAN_NI + 1)
 
+// controller settings: tg_ctrl_spec with R and Rd replaced by their symmetric parts.  The handle's own are DevCfg::ctl; the
+// ctrl instances of tw_solver.cuh read a problem's own record of the same type
+struct TwCtrl { double q_c, q_phi, q_vx, Rs[4], Rds[4], u_lo[2], u_hi[2], du_lo[2], du_hi[2], x_lo[6], x_hi[6]; };
+static_assert(sizeof(TwCtrl) == sizeof(tg_ctrl_spec), "TwCtrl mirrors tg_ctrl_spec field by field");
+
 struct DevCfg {
     int N, n;         // horizon, 2N
     int model, plant, jacobian;
@@ -35,9 +40,7 @@ struct DevCfg {
     const double *tyre_tab; // [2][TG_TAB_NI][TG_TAB_NC] piecewise polynomials of sin(C atan(B alpha)) on [-maxAlpha, maxAlpha], or null
     double tab_scale;       // TG_TAB_NI / (2 maxAlpha)
     const double *atan_tab; // [TG_ATAN_NI][TG_TAB_NC] piecewise polynomials of atan on [-TG_ATAN_T0, TG_ATAN_T0], or null
-    double q_c, q_phi, q_vx;
-    double Rs[4], Rds[4];  // symmetric parts
-    double u_lo[2], u_hi[2], du_lo[2], du_hi[2], x_lo[6], x_hi[6];
+    TwCtrl ctl;             // weights and bounds
     double rho, sigma, alpha, alpha_warm, eps_abs, eps_rel, eps_pinf, adapt_tol;
     double noise_std[6];
     unsigned long long seed_base;

@@ -421,22 +421,26 @@ struct TwKernels {
     TwStepKernel step, step_p1;
     TwLoopKernel loop, loop_p1;
 };
+// what a launch of one set of instances needs: the kernels, the shared memory per problem, and the most problems per CTA
+// (0: one problem does not fit)
+struct TwLaunch {
+    TwKernels k;
+    size_t smem;
+    int ppc_max;
+};
 
 struct tg_handle {
     tg_config cfg;
     DevCfg dc;
     int device, num_sms, grid_cap;
-    int ppc_max, ppc_env;     // closed-loop kernel: most problems per CTA that fit / TRAJGEN_PPC override (0 = automatic)
+    int ppc_env;              // TRAJGEN_PPC override of the problems per CTA (0 = automatic)
     // warp-per-problem kernels (tw_solver.cuh): W warps per problem, S tile blocks per thread
     int W, S;
-    TwKernels kern;
-    TwKernels kern_ctrl;      // the ctrl instances of the shape (per-problem settings, tg_mpc_step_ctrl / tg_closed_loop_ctrl)
-    int ppc_max_ctrl;         // most problems per CTA of a ctrl launch (stride smem_ctrl_bytes); 0: the record does not fit
-    size_t smem_ctrl_bytes;   // per-problem shared memory of a ctrl launch: the block plus the staged tg_ctrl_spec
+    TwLaunch tw;              // the instances of the handle's own settings
+    TwLaunch tw_ctrl;         // the ctrl instances of the shape (per-problem settings, tg_mpc_step_ctrl / tg_closed_loop_ctrl)
     WLayout WL;
     WLayout Lref;             // layout of the reference-window tap kernel (no state rows, one warp)
     size_t smem_optin;
-    size_t smem_bytes;
     cudaStream_t stream;
     long long launches;
     double *tyre_tab;   // device copy of the tyre-curve table, or null (fit not at rounding level -> atan/sin path)
@@ -456,69 +460,74 @@ static bool tw_standard_controller(const DevCfg &d)
 {
     return d.model == TG_MODEL_MPC && d.jacobian == TG_JAC_ANALYTIC && d.tyre_tab && d.atan_tab;
 }
-// the kernels of one (W, S, NC, HS).  Single-problem-per-CTA instances exist for the one- and two-warp shapes, where four CTAs
-// per SM would leave most of the register file and shared memory unused, except for a compile-time horizon without state-bound
-// rows.  A compile-time horizon with state-bound rows on those shapes has only that instance (problems with state-bound rows
-// always run one per CTA, choose_tw_ppc).
-template <int W, int S, int NC, bool HS>
+// the kernels of one (W, S, NC, HS, CT).  Single-problem-per-CTA instances exist for the one- and two-warp shapes, where four
+// CTAs per SM would leave most of the register file and shared memory unused, except for a compile-time horizon without
+// state-bound rows.  A compile-time horizon with state-bound rows on those shapes has only that instance (problems with
+// state-bound rows always run one per CTA, choose_tw_ppc).  The ctrl instances (CT, per-problem settings staged in shared
+// memory) exist for the run-time horizon with the code of the state-bound rows only.
+template <int W, int S, int NC, bool HS, bool CT = false>
 static TwKernels tw_instance()
 {
     static_assert(NC == 0 || (tw_shape(NC).W == W && tw_shape(NC).S == S), "a compile-time horizon runs on its tw_shape");
+    static_assert(!CT || (NC == 0 && HS), "ctrl instances: run-time horizon with state-bound rows only");
     TwKernels k = {};
     if constexpr (!(HS && NC > 0 && W <= 2)) {
-        k.step = tw_mpc_step_kernel<W, S, NC, false, HS>;
-        k.loop = tw_closed_loop_kernel<W, S, NC, false, HS>;
+        k.step = tw_mpc_step_kernel<W, S, NC, false, HS, CT>;
+        k.loop = tw_closed_loop_kernel<W, S, NC, false, HS, CT>;
     }
     if constexpr (W <= 2 && (NC == 0 || HS)) {
-        k.step_p1 = tw_mpc_step_kernel<W, S, NC, true, HS>;
-        k.loop_p1 = tw_closed_loop_kernel<W, S, NC, true, HS>;
+        k.step_p1 = tw_mpc_step_kernel<W, S, NC, true, HS, CT>;
+        k.loop_p1 = tw_closed_loop_kernel<W, S, NC, true, HS, CT>;
     }
     return k;
 }
-// every compiled instance.  fixed_n selects the compile-time-horizon instances where one exists: mpc_step's default horizon
-// (20), MPC/main.py's (40), BASELINE config 4's (10, 50).  No instance: every pointer null.
-static TwKernels tw_kernels(int W, int S, int N, int ms, bool fixed_n)
+// the run-time-horizon instances of the five shapes
+template <bool CT>
+static TwKernels tw_runtime(int W, int S)
 {
-    if (fixed_n && ms == 0) {
+    if (W == 1 && S == 1) return tw_instance<1, 1, 0, true, CT>();
+    if (W == 2 && S == 1) return tw_instance<2, 1, 0, true, CT>();
+    if (W == 4 && S == 1) return tw_instance<4, 1, 0, true, CT>();
+    if (W == 8 && S == 1) return tw_instance<8, 1, 0, true, CT>();
+    if (W == 8 && S == 2) return tw_instance<8, 2, 0, true, CT>();
+    return TwKernels{};
+}
+// every compiled instance.  ct selects the ctrl instances.  Otherwise fixed_n selects the compile-time-horizon instances where
+// one exists: mpc_step's default horizon (20), MPC/main.py's (40), BASELINE config 4's (10, 50).  No instance: every pointer
+// null.
+static TwKernels tw_kernels(int W, int S, int N, int ms, bool fixed_n, bool ct)
+{
+    if (fixed_n && !ct && ms == 0) {
         if (W == 2 && S == 1 && N == 20) return tw_instance<2, 1, 20, false>();
         if (W == 1 && S == 1 && N == 10) return tw_instance<1, 1, 10, false>();
         if (W == 8 && S == 1 && N == 40) return tw_instance<8, 1, 40, false>();
         if (W == 8 && S == 2 && N == 50) return tw_instance<8, 2, 50, false>();
     }
-    if (fixed_n && ms > 0) {
+    if (fixed_n && !ct && ms > 0) {
         if (W == 2 && S == 1 && N == 20) return tw_instance<2, 1, 20, true>();
         if (W == 1 && S == 1 && N == 10) return tw_instance<1, 1, 10, true>();
         if (W == 8 && S == 2 && N == 50) return tw_instance<8, 2, 50, true>();
     }
-    if (W == 1 && S == 1) return tw_instance<1, 1, 0, true>();
-    if (W == 2 && S == 1) return tw_instance<2, 1, 0, true>();
-    if (W == 4 && S == 1) return tw_instance<4, 1, 0, true>();
-    if (W == 8 && S == 1) return tw_instance<8, 1, 0, true>();
-    if (W == 8 && S == 2) return tw_instance<8, 2, 0, true>();
-    return TwKernels{};
+    if (!ct) return tw_runtime<false>(W, S);
+    return tw_runtime<true>(W, S);
 }
-// the ctrl instances (per-problem settings staged in shared memory, template flag CT): run-time horizon with the code of the
-// state-bound rows, on every shape, with the same P1 rule as tw_instance<W, S, 0, true>
-template <int W, int S>
-static TwKernels tw_ctrl_instance()
+// a TwLaunch of the instances k with `smem` bytes per problem.  Problems per CTA: within the CTA's threads, a barrier id per
+// problem for W > 1, and the opt-in shared memory.  The shared-memory attributes are per kernel function and process-wide:
+// always raise them to the device limit so that handles with different layouts can be used side by side.
+static int make_tw_launch(const tg_handle *h, const TwKernels &k, size_t smem, TwLaunch &out)
 {
-    TwKernels k = {};
-    k.step = tw_mpc_step_kernel<W, S, 0, false, true, true>;
-    k.loop = tw_closed_loop_kernel<W, S, 0, false, true, true>;
-    if constexpr (W <= 2) {
-        k.step_p1 = tw_mpc_step_kernel<W, S, 0, true, true, true>;
-        k.loop_p1 = tw_closed_loop_kernel<W, S, 0, true, true, true>;
+    out.k = k; out.smem = smem; out.ppc_max = 0;
+    if (smem > h->smem_optin) return TG_OK;
+    int p = TW_CTA_THREADS / (32 * h->W);
+    if (h->W > 1) p = std::min(p, TW_BAR_STEP - TW_BAR_PROB);
+    while (p > 1 && (size_t)p * smem > h->smem_optin) p -= 1;
+    out.ppc_max = p;
+    for (const void *f : {(const void *)k.step, (const void *)k.step_p1, (const void *)k.loop, (const void *)k.loop_p1}) {
+        if (!f) continue;
+        CK(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+        CK(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
-    return k;
-}
-static TwKernels tw_ctrl_kernels(int W, int S)
-{
-    if (W == 1 && S == 1) return tw_ctrl_instance<1, 1>();
-    if (W == 2 && S == 1) return tw_ctrl_instance<2, 1>();
-    if (W == 4 && S == 1) return tw_ctrl_instance<4, 1>();
-    if (W == 8 && S == 1) return tw_ctrl_instance<8, 1>();
-    if (W == 8 && S == 2) return tw_ctrl_instance<8, 2>();
-    return TwKernels{};
+    return TG_OK;
 }
 
 // warp-per-problem kernels: problems per CTA.  Resident problems per SM are bounded by registers (512 threads x 128) and
@@ -537,19 +546,19 @@ static int choose_tw_ppc(const tg_handle *h, int B, int ppc_max)
 }
 
 // the single-problem instance where there is no other or where one problem per CTA is chosen, else `multi` with
-// choose_tw_ppc problems per CTA.  A launch with per-problem settings (a.ctrl) runs the ctrl instances, whose problems take
-// smem_ctrl_bytes each.
+// choose_tw_ppc problems per CTA; `multi` and `p1` are kernels of `t`
 template <typename Args>
-static int launch_tw(tg_handle *h, void (*multi)(DevCfg, WLayout, Args), void (*p1)(DevCfg, WLayout, Args), Args &a)
+static int launch_tw(tg_handle *h, const TwLaunch &t, void (*multi)(DevCfg, WLayout, Args), void (*p1)(DevCfg, WLayout, Args),
+                     Args &a)
 {
-    const bool ct = a.ctrl != nullptr;
-    if (ct && h->ppc_max_ctrl < 1) return fail(TG_ERR_UNSUPPORTED, "per-problem settings: the record does not fit beside the problem's shared memory");
-    int ppc = choose_tw_ppc(h, a.B, ct ? h->ppc_max_ctrl : h->ppc_max);
+    // tg_create refuses a handle whose own problems do not fit, so only the ctrl instances can get here without a fit
+    if (t.ppc_max < 1) return fail(TG_ERR_UNSUPPORTED, "per-problem settings: the record does not fit beside the problem's shared memory");
+    int ppc = choose_tw_ppc(h, a.B, t.ppc_max);
     void (*kern)(DevCfg, WLayout, Args) = multi;
     if (p1 && (!multi || ppc == 1)) { kern = p1; ppc = 1; }
     a.ppc = ppc;
     const int threads = 32 * h->W * ppc;
-    const size_t smem = (size_t)ppc * (ct ? h->smem_ctrl_bytes : h->smem_bytes);
+    const size_t smem = (size_t)ppc * t.smem;
     int per_sm = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
     if (per_sm < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
@@ -638,14 +647,14 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
             if (e_at <= 4e-16) d.atan_tab = h->tyre_tab + 2 * TG_TAB_ROWS * TG_TAB_NC;
         }
     }
-    d.q_c = cfg->q_c; d.q_phi = cfg->q_phi; d.q_vx = cfg->q_vx;
+    d.ctl.q_c = cfg->q_c; d.ctl.q_phi = cfg->q_phi; d.ctl.q_vx = cfg->q_vx;
     for (int i = 0; i < 2; ++i)
         for (int j = 0; j < 2; ++j) {
-            d.Rs[i * 2 + j] = 0.5 * (cfg->R[i * 2 + j] + cfg->R[j * 2 + i]);
-            d.Rds[i * 2 + j] = 0.5 * (cfg->Rd[i * 2 + j] + cfg->Rd[j * 2 + i]);
+            d.ctl.Rs[i * 2 + j] = 0.5 * (cfg->R[i * 2 + j] + cfg->R[j * 2 + i]);
+            d.ctl.Rds[i * 2 + j] = 0.5 * (cfg->Rd[i * 2 + j] + cfg->Rd[j * 2 + i]);
         }
-    memcpy(d.u_lo, cfg->u_lo, 16); memcpy(d.u_hi, cfg->u_hi, 16); memcpy(d.du_lo, cfg->du_lo, 16); memcpy(d.du_hi, cfg->du_hi, 16);
-    memcpy(d.x_lo, cfg->x_lo, 48); memcpy(d.x_hi, cfg->x_hi, 48);
+    memcpy(d.ctl.u_lo, cfg->u_lo, 16); memcpy(d.ctl.u_hi, cfg->u_hi, 16); memcpy(d.ctl.du_lo, cfg->du_lo, 16); memcpy(d.ctl.du_hi, cfg->du_hi, 16);
+    memcpy(d.ctl.x_lo, cfg->x_lo, 48); memcpy(d.ctl.x_hi, cfg->x_hi, 48);
     d.rho = cfg->rho; d.sigma = cfg->sigma; d.alpha = cfg->alpha;
     d.alpha_warm = (cfg->alpha_warm > 0.0 && cfg->alpha_warm < 2.0) ? cfg->alpha_warm : cfg->alpha; d.eps_abs = cfg->eps_abs; d.eps_rel = cfg->eps_rel;
     d.eps_pinf = cfg->eps_prim_inf; d.adapt_tol = cfg->adaptive_rho_tol > 1.0 ? cfg->adaptive_rho_tol : 5.0;
@@ -660,42 +669,19 @@ int tg_create(const tg_config *cfg, int device, tg_handle **out)
     {
         h->WL = tw_make_layout(d.N, d.ms, shape);
         const size_t stride = (size_t)tw_stride(h->WL) * sizeof(double);
-        h->smem_bytes = stride;
-        if (stride > h->smem_optin) return fail(TG_ERR_UNSUPPORTED, "state-bound rows x horizon exceed the 227 KB shared memory of one CTA");
-        h->ppc_max = TW_CTA_THREADS / (32 * h->W);
-        if (h->W > 1) h->ppc_max = std::min(h->ppc_max, TW_BAR_STEP - TW_BAR_PROB);   // a barrier id per problem
-        while (h->ppc_max > 1 && (size_t)h->ppc_max * stride > h->smem_optin) h->ppc_max -= 1;
-        if (const char *e = getenv("TRAJGEN_PPC")) { const int v = atoi(e); if (v >= 1 && v <= h->ppc_max) h->ppc_env = v; }
-        h->kern = tw_kernels(h->W, h->S, d.N, d.ms, tw_standard_controller(d) && !getenv("TRAJGEN_DYNAMIC_N"));
-        const TwKernels &k = h->kern;
+        const TwKernels k = tw_kernels(h->W, h->S, d.N, d.ms, tw_standard_controller(d) && !getenv("TRAJGEN_DYNAMIC_N"), false);
+        int rc = make_tw_launch(h, k, stride, h->tw);
+        if (rc != TG_OK) return rc;
+        if (h->tw.ppc_max < 1) return fail(TG_ERR_UNSUPPORTED, "state-bound rows x horizon exceed the 227 KB shared memory of one CTA");
+        if (const char *e = getenv("TRAJGEN_PPC")) { const int v = atoi(e); if (v >= 1 && v <= h->tw.ppc_max) h->ppc_env = v; }
         if (!k.loop && !k.loop_p1) return fail(TG_ERR_UNSUPPORTED, "no kernel shape for this horizon");
-        // the attributes are per kernel function and process-wide: always raise them to the device limit so that handles with
-        // different layouts can be used side by side
-        for (const void *f : {(const void *)k.step, (const void *)k.step_p1, (const void *)k.loop, (const void *)k.loop_p1}) {
-            if (!f) continue;
-            CK(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
-            CK(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        }
         int occ = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k.loop_p1 ? k.loop_p1 : k.loop, 32 * h->W, stride));
         if (occ < 1) return fail(TG_ERR_UNSUPPORTED, "kernel does not fit on an SM with this configuration");
         h->grid_cap = occ * h->num_sms;     // resident problems with one problem per CTA
-        // the ctrl instances: the same rules for the stride with the staged record (launch_tw takes the occupancy per launch)
-        h->kern_ctrl = tw_ctrl_kernels(h->W, h->S);
-        const TwKernels &kc = h->kern_ctrl;
-        const size_t stride_c = stride + TW_CTRL_DBL * sizeof(double);
-        h->smem_ctrl_bytes = stride_c;
-        h->ppc_max_ctrl = 0;
-        if (stride_c <= h->smem_optin) {
-            h->ppc_max_ctrl = TW_CTA_THREADS / (32 * h->W);
-            if (h->W > 1) h->ppc_max_ctrl = std::min(h->ppc_max_ctrl, TW_BAR_STEP - TW_BAR_PROB);
-            while (h->ppc_max_ctrl > 1 && (size_t)h->ppc_max_ctrl * stride_c > h->smem_optin) h->ppc_max_ctrl -= 1;
-        }
-        for (const void *f : {(const void *)kc.step, (const void *)kc.step_p1, (const void *)kc.loop, (const void *)kc.loop_p1}) {
-            if (!f) continue;
-            CK(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
-            CK(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        }
+        // the ctrl instances: the block plus the staged record (launch_tw takes the occupancy per launch)
+        rc = make_tw_launch(h, tw_kernels(h->W, h->S, d.N, d.ms, false, true), stride + TW_CTRL_DBL * sizeof(double), h->tw_ctrl);
+        if (rc != TG_OK) return rc;
     }
     h->stream = 0;
     guard.p = nullptr;
@@ -720,7 +706,7 @@ int tg_info(tg_handle *h, int32_t *ctas_per_sm, int32_t *threads_per_cta, int32_
     if (!h) return fail(TG_ERR_INVALID, "null handle");
     if (ctas_per_sm) *ctas_per_sm = h->grid_cap / h->num_sms;
     if (threads_per_cta) *threads_per_cta = 32 * h->W;
-    if (smem_bytes) *smem_bytes = (int32_t)h->smem_bytes;
+    if (smem_bytes) *smem_bytes = (int32_t)h->tw.smem;
     if (num_sms) *num_sms = h->num_sms;
     return TG_OK;
 }
@@ -746,16 +732,14 @@ static int launch_step(tg_handle *h, StepArgs &a)
 {
     if (a.B <= 0) return TG_OK;   // empty batch: nothing to do
     CK(cudaSetDevice(h->device));
-    const TwKernels &k = a.ctrl ? h->kern_ctrl : h->kern;
-    return launch_tw(h, k.step, k.step_p1, a);
+    const TwLaunch &t = a.ctrl ? h->tw_ctrl : h->tw;
+    return launch_tw(h, t, t.k.step, t.k.step_p1, a);
 }
 
 // the rules of tg_ctrl_spec (include/trajgen.h), row by row: TG_ERR_INVALID naming the first bad row and field
-static int ctrl_check(const tg_handle *h, int B, const tg_ctrl_spec *ctrl)
+int tg_check_ctrl(int B, const tg_ctrl_spec *ctrl, uint32_t bounded_states)
 {
     if (B > 0 && !ctrl) return fail(TG_ERR_INVALID, "bad argument: ctrl is null");
-    bool bounded[6] = {false, false, false, false, false, false};
-    for (int si = 0; si < h->dc.ns; ++si) bounded[h->dc.sidx[si]] = true;
     for (int b = 0; b < B; ++b) {
         const tg_ctrl_spec &r = ctrl[b];
         auto bad = [&](const std::string &field, const char *why) { return fail(TG_ERR_INVALID, "ctrl row " + std::to_string(b) + ": " + field + " " + why); };
@@ -780,10 +764,17 @@ static int ctrl_check(const tg_handle *h, int B, const tg_ctrl_spec *ctrl)
         for (int i = 0; i < 6; ++i) {
             const std::string f = "x_lo[" + std::to_string(i) + "] / x_hi[" + std::to_string(i) + "]";
             if (!(r.x_lo[i] <= r.x_hi[i])) return bad(f, "lo > hi");
-            if (!bounded[i] && (r.x_lo[i] > -TG_INF || r.x_hi[i] < TG_INF)) return bad(f, "finite bound on a state component the handle does not bound");
+            if (!(bounded_states >> i & 1u) && (r.x_lo[i] > -TG_INF || r.x_hi[i] < TG_INF)) return bad(f, "finite bound on a state component the handle does not bound");
         }
     }
     return TG_OK;
+}
+// tg_check_ctrl's bounded_states of a handle: bit i set when it bounds state component i
+static uint32_t bounded_states(const tg_handle *h)
+{
+    uint32_t m = 0;
+    for (int si = 0; si < h->dc.ns; ++si) m |= 1u << h->dc.sidx[si];
+    return m;
 }
 
 int tg_linearize(tg_handle *h, int B, const double *x0, const double *u_prev, double *A, double *Bm, double *g, double *xbar)
@@ -876,8 +867,8 @@ int tg_closed_loop_ctrl(tg_handle *h, int B, int T, const double *x0, const doub
     a.B = B; a.T = T; a.x0 = x0; a.u0 = u0; a.spec = spec; a.brk = brk; a.coef = coef; a.traj_id0 = traj_id0;
     a.clean = clean; a.noisy = noisy; a.U = U; a.status_counts = status_counts; a.iters_total = (long long *)iters_total;
     a.ctrl = ctrl;
-    const TwKernels &k = ctrl ? h->kern_ctrl : h->kern;
-    return launch_tw(h, k.loop, k.loop_p1, a);
+    const TwLaunch &t = ctrl ? h->tw_ctrl : h->tw;
+    return launch_tw(h, t, t.k.loop, t.k.loop_p1, a);
 }
 
 int tg_plant_rollout(tg_handle *h, int B, int T, const double *x0, const double *U, double *X)
@@ -1210,7 +1201,7 @@ int tg_mpc_step_ctrl_host(tg_handle *h, int B, const double *x0, const double *u
                           double *U_opt, double *X_opt, double *y_opt)
 {
     if (!h || B < 0 || (B > 0 && (!x0 || !u_prev || !path_ref || !u_cmd))) return fail(TG_ERR_INVALID, "bad argument");
-    if (ctrl) { const int rc = ctrl_check(h, B, ctrl); if (rc != TG_OK) return rc; }
+    if (ctrl) { const int rc = tg_check_ctrl(B, ctrl, bounded_states(h)); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
     const int N = h->dc.N, n = h->dc.n, m = h->dc.m;
@@ -1267,7 +1258,7 @@ int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const
                              int64_t *iters_total)
 {
     if (!h || B < 0 || T < 0 || (B > 0 && (!x0 || !u0 || !spec || !clean || !noisy || (T > 0 && !U)))) return fail(TG_ERR_INVALID, "bad argument");
-    if (ctrl) { const int rc = ctrl_check(h, B, ctrl); if (rc != TG_OK) return rc; }
+    if (ctrl) { const int rc = tg_check_ctrl(B, ctrl, bounded_states(h)); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     {   // the scenario table is host memory here: reject what would send the device out of bounds
         const int64_t n_tab = (brk && coef) ? (n_breaks < n_coef ? n_breaks : n_coef) : 0;

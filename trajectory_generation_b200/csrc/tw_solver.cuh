@@ -140,14 +140,12 @@ __host__ __device__ constexpr int tw_stride(const WLayout &L) { return tw_even(L
 // offset of a FIXED-part array / a geometry constant
 #define LF(f) (NC > 0 ? TwFix<NC, W>::L.f : L.f)
 
-// Per-problem controller settings (tg_ctrl_spec, with R and Rd replaced by their symmetric parts as tg_create does for DevCfg).
-// The ctrl instances (template flag CT) stage a problem's record in shared memory right after its block, at sm + tw_stride(L),
-// so that their stride is tw_stride(L) + TW_CTRL_DBL; every other instance reads the same fields from DevCfg.  TWC(f) is the
-// field f of whichever applies.
-struct TwCtrl { double q_c, q_phi, q_vx, Rs[4], Rds[4], u_lo[2], u_hi[2], du_lo[2], du_hi[2], x_lo[6], x_hi[6]; };
-static_assert(sizeof(TwCtrl) == sizeof(tg_ctrl_spec), "TwCtrl mirrors tg_ctrl_spec field by field");
+// Per-problem controller settings (TwCtrl, tg_device.cuh).  The ctrl instances (template flag CT) stage a problem's record in
+// shared memory right after its block, at sm + tw_stride(L), so that their stride is tw_stride(L) + TW_CTRL_DBL; every other
+// instance reads the handle's settings, DevCfg::ctl.  TWC(f) is the field f of whichever applies.  It names c.ctl.f directly:
+// a reference to c.ctl would take the address of the __grid_constant__ parameter and can turn its loads into generic ones.
 constexpr int TW_CTRL_DBL = tw_even((int)(sizeof(TwCtrl) / sizeof(double)));
-#define TWC(f) (CT ? cr->f : c.f)
+#define TWC(f) (CT ? cr->f : c.ctl.f)
 // thread i < 31 stages field i of the record; the caller synchronises before the record is read
 __device__ __forceinline__ void tw_stage_ctrl(double *rec, const tg_ctrl_spec *src, int tid)
 {

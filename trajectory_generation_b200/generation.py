@@ -225,12 +225,8 @@ class ClosedLoopGenerator(BatchedMPC):
             out = self.alloc_result(B, T, pinned)
         elif out["clean"].shape != (B, T + 1, 6) or out["U"].shape != (B, T, 2):
             raise ValueError("`out` was allocated for another batch size / horizon")
-        L = _lib.load()
-        head = (self._h, B, T, _lib.ptr(x0), _lib.ptr(u0), spec.ctypes.data)
-        if ctrl is not None:
-            head += (ctrl.ctypes.data,)
-        _lib.check((L.tg_closed_loop_host if ctrl is None else L.tg_closed_loop_ctrl_host)(
-            *head, _lib.ptr(brk) if len(brk) else None,
+        _lib.check(_lib.load().tg_closed_loop_ctrl_host(
+            self._h, B, T, _lib.ptr(x0), _lib.ptr(u0), spec.ctypes.data, _lib.ptr(ctrl), _lib.ptr(brk) if len(brk) else None,
             len(brk), _lib.ptr(coef) if len(coef) else None, len(coef), int(traj_id0),
             _lib.ptr(out["clean"]), _lib.ptr(out["noisy"]), _lib.ptr(out["U"]), _lib.ptr(out["status_counts"]),
             _lib.ptr(out["iters_total"])))

@@ -64,34 +64,15 @@ def make_config(Ts=0.02, N=20, params=None, q_c=6.0, q_phi=0.5, q_vx=0.5, R=None
 
 
 def check_ctrl_table(table, bounded):
-    """The rules of include/trajgen.h::tg_ctrl_spec for every row of ``table`` (CTRL_SPEC_DTYPE); ``bounded[6]`` says which
-    state components the handle bounds.  Raises ValueError naming the first bad row and field, as the C entry points do."""
-    t = table
-    checks = []                                             # (field, reason, bad[B]) in the order the library checks them
-    for f in ("q_c", "q_phi", "q_vx"):
-        checks.append((f, "must be finite and >= 0", ~(np.isfinite(t[f]) & (t[f] >= 0.0))))
-    for i in range(4):
-        checks.append((f"R[{i}]", "must be finite", ~np.isfinite(t["R"][:, i])))
-        checks.append((f"Rd[{i}]", "must be finite", ~np.isfinite(t["Rd"][:, i])))
-    with np.errstate(invalid="ignore", over="ignore"):
-        R, Rd = t["R"], t["Rd"]
-        a, c, d_ = R[:, 0], 0.5 * (R[:, 1] + R[:, 2]), R[:, 3]
-        checks.append(("R", "symmetric part is not positive definite", ~((a > 0.0) & (a * d_ - c * c > 0.0))))
-        a, c, d_ = Rd[:, 0], 0.5 * (Rd[:, 1] + Rd[:, 2]), Rd[:, 3]
-        checks.append(("Rd", "symmetric part is not positive semidefinite", ~((a >= 0.0) & (d_ >= 0.0) & (a * d_ - c * c >= 0.0))))
-    for i in range(2):
-        for lo, hi in (("u_lo", "u_hi"), ("du_lo", "du_hi")):
-            checks.append((f"{lo}[{i}] / {hi}[{i}]", "lo > hi", ~(t[lo][:, i] <= t[hi][:, i])))
-    for i in range(6):
-        f = f"x_lo[{i}] / x_hi[{i}]"
-        checks.append((f, "lo > hi", ~(t["x_lo"][:, i] <= t["x_hi"][:, i])))
-        if not bounded[i]:
-            checks.append((f, "finite bound on a state component the handle does not bound",
-                           (t["x_lo"][:, i] > -_lib.TG_INF) | (t["x_hi"][:, i] < _lib.TG_INF)))
-    first = min((int(np.argmax(bad)) for _, _, bad in checks if bad.any()), default=None)
-    if first is not None:
-        field, why = next((f, w) for f, w, bad in checks if bad[first])
-        raise ValueError(f"ctrl row {first}: {field} {why}")
+    """The rules of include/trajgen.h::tg_ctrl_spec for every row of ``table`` (CTRL_SPEC_DTYPE), checked by the library's
+    tg_check_ctrl; ``bounded[6]`` says which state components the handle bounds.  Raises ValueError naming the first bad row
+    and field, as the C entry points do."""
+    t = np.ascontiguousarray(table)
+    if t.dtype != _lib.CTRL_SPEC_DTYPE or t.ndim != 1:
+        raise ValueError("ctrl must be a table of CTRL_SPEC_DTYPE (see ctrl_table)")
+    L = _lib.load()
+    if L.tg_check_ctrl(len(t), _lib.ptr(t), sum(1 << i for i in range(6) if bounded[i])) != 0:
+        raise ValueError(L.tg_last_error().decode())
     return table
 
 
@@ -105,7 +86,7 @@ class BatchedMPC:
         self._h = ctypes.c_void_p()
         _lib.check(_lib.load().tg_create(ctypes.byref(self.cfg), int(device), ctypes.byref(self._h)))
         self.n = 2 * self.N
-        self.ns = sum(1 for i in range(6) if self.cfg.x_lo[i] > -_lib.TG_INF or self.cfg.x_hi[i] < _lib.TG_INF)
+        self.ns = sum(self.bounded_states)
         self.ms = self.ns * self.N
         self.m = 4 * self.N + self.ms
 
@@ -185,8 +166,6 @@ class BatchedMPC:
     def _ctrl_arg(self, ctrl, B):
         """a caller's ctrl table, checked: a C-contiguous [B] array of CTRL_SPEC_DTYPE that satisfies tg_ctrl_spec's rules"""
         t = np.ascontiguousarray(ctrl)
-        if t.dtype != _lib.CTRL_SPEC_DTYPE:
-            raise ValueError("ctrl must be a table of CTRL_SPEC_DTYPE (see ctrl_table)")
         if t.shape != (B,):
             raise ValueError(f"ctrl: expected {B} rows, got shape {t.shape}")
         return check_ctrl_table(t, self.bounded_states)
@@ -263,12 +242,9 @@ class BatchedMPC:
                "objective": np.empty(B)}
         if want_trajectory:
             out.update(U_opt=np.empty((B, N, 2)), X_opt=np.empty((B, N + 1, 6)), y_opt=np.empty((B, self.m)))
-        L = _lib.load()
-        args = (self._h, B, _lib.ptr(x0), _lib.ptr(u_prev), _lib.ptr(path_ref), _lib.ptr(vref))
-        if ctrl is not None:
-            args += (ctrl.ctypes.data,)
-        _lib.check((L.tg_mpc_step_host if ctrl is None else L.tg_mpc_step_ctrl_host)(
-            *args, _lib.ptr(out["u_cmd"]), _lib.ptr(out["status"]), _lib.ptr(out["iters"]), _lib.ptr(out["objective"]),
+        _lib.check(_lib.load().tg_mpc_step_ctrl_host(
+            self._h, B, _lib.ptr(x0), _lib.ptr(u_prev), _lib.ptr(path_ref), _lib.ptr(vref), _lib.ptr(ctrl),
+            _lib.ptr(out["u_cmd"]), _lib.ptr(out["status"]), _lib.ptr(out["iters"]), _lib.ptr(out["objective"]),
             _lib.ptr(out.get("U_opt")), _lib.ptr(out.get("X_opt")), _lib.ptr(out.get("y_opt"))))
         return out
 
