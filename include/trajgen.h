@@ -130,7 +130,8 @@ typedef struct tg_ref_spec {
  * finite or infinite bound on a component the handle bounds.  Rules (checked by tg_check_ctrl and by the *_host entry points,
  * which return TG_ERR_INVALID naming the first bad row and field before anything is launched; preconditions of the
  * device-pointer ones): weights finite and >= 0; R, Rd finite, the symmetric part of R positive definite, that of Rd positive
- * semidefinite; lo <= hi for every bound; no finite x_lo / x_hi on a state component the handle does not bound. */
+ * semidefinite; lo <= hi for every bound; no finite x_lo / x_hi on a state component the handle does not bound.
+ * (The vehicle that the closed loop integrates -- its plant -- can be set per trajectory as well: see tg_closed_loop_params.) */
 typedef struct tg_ctrl_spec {
     double q_c, q_phi, q_vx;
     double R[4], Rd[4];        /* row-major 2x2 */
@@ -143,6 +144,23 @@ typedef struct tg_ctrl_spec {
  * bounded_states is set.  TG_OK, or TG_ERR_INVALID with tg_last_error() = "ctrl row b: <field> <why>" for the first bad row.
  * Needs no handle and no GPU. */
 int tg_check_ctrl(int B, const tg_ctrl_spec *ctrl, uint32_t bounded_states);
+
+/* ---- per-trajectory plant parameters (the *_params entry points).  plant[B][TG_NPARAMS] (fp64, the order of params[]): row b
+ * is the vehicle that trajectory b's ground truth integrates for all of its steps -- the closed-loop plant step (MPC/main.py:97,
+ * with the clipping of generation_type1.py:81-82 / generation_type2.py:186-187 for the generator plants), tg_plant_rollout's
+ * integration and the open-loop generators' (generation_type1.py:70-84, generation_type2.py:180-187).  NULL = the handle's
+ * params for every trajectory.  The table changes nothing else: the controller's rollout, linearisation and QP keep the
+ * handle's params (a plant that differs from the controller's model), and so do the reference windows, the sensor noise,
+ * tg_make_scenarios' u0 and the plant variant.  g is unused, as everywhere.
+ * Tyre curve: a row whose Bf, Cf, Br, Cr and maxAlpha equal the handle's bit for bit, on a handle whose tables are in use
+ * (tg_tyre_table_info), evaluates the handle's tyre-curve and slip-angle tables; any other row evaluates atan2 / atan / sin with
+ * libdevice (the tables are fitted and verified for the handle's constants only).  So row b gives the bits that a handle created
+ * with params = row b gives -- with TRAJGEN_NO_TYRE_TABLE=1 when its tyre constants differ from the handle's.  Varying masses,
+ * inertias, motor / drag constants or tyre peaks (D) keeps the tables; varying B, C or maxAlpha costs libdevice in the plant.
+ * Rules: every entry finite; m, Iz, vx_zero and maxAlpha > 0.  tg_check_plant_params checks them (no handle, no GPU needed):
+ * TG_OK, or TG_ERR_INVALID with tg_last_error() = "plant row b: <name> <why>" for the first bad row.  The *_host entry points
+ * check them before anything is launched; for the device-pointer ones they are a precondition. */
+int tg_check_plant_params(int B, const double *plant);
 
 typedef struct tg_handle tg_handle;
 
@@ -216,6 +234,17 @@ int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const
                              const tg_ctrl_spec *ctrl, const double *spl_breaks, int64_t n_breaks, const double *spl_coef,
                              int64_t n_coef, int64_t traj_id0, double *clean, double *noisy, double *U,
                              int32_t *status_counts, int64_t *iters_total);
+/* the same with trajectory b's plant integrated with the vehicle plant[b] (see tg_check_plant_params) while its controller keeps
+ * the handle's model.  ctrl and plant may each be NULL; (NULL, NULL) is tg_closed_loop[_host].  ctrl == NULL runs the handle's
+ * own kernel instances (the compile-time horizons included), ctrl != NULL the ctrl instances. */
+int tg_closed_loop_params(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                          const tg_ctrl_spec *ctrl, const double *plant, const double *spl_breaks, const double *spl_coef,
+                          int64_t traj_id0, double *clean, double *noisy, double *U, int32_t *status_counts,
+                          int64_t *iters_total);
+int tg_closed_loop_params_host(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                               const tg_ctrl_spec *ctrl, const double *plant, const double *spl_breaks, int64_t n_breaks,
+                               const double *spl_coef, int64_t n_coef, int64_t traj_id0, double *clean, double *noisy,
+                               double *U, int32_t *status_counts, int64_t *iters_total);
 
 /* ---- scenario + initial-state generation on the device (SURVEY.md 8(d) configs 2, 3, 5): x0 from the ranges of
  * generation_type1.py:260-265 / generation_type2.py:171-174 (Y and phi relative to the reference path), one reference path
@@ -246,6 +275,8 @@ int tg_make_scenarios_host(tg_handle *h, int B, int64_t traj_id0, const tg_scena
  * tg_sensor_noise: standard normals [n_traj][n_rows][6] for seeds seed_base + traj_id0 + i (Philox4x32-10).
  * tg_philox_u32: raw stream, out[n][4] = philox(ctr=(first+i, block, 0, 0), key=seed). */
 int tg_plant_rollout(tg_handle *h, int B, int T, const double *x0, const double *U, double *X);
+/* the same with trajectory b integrated with the vehicle plant[b][TG_NPARAMS] (NULL = tg_plant_rollout; see tg_check_plant_params) */
+int tg_plant_rollout_params(tg_handle *h, int B, int T, const double *x0, const double *U, const double *plant, double *X);
 int tg_sensor_noise(tg_handle *h, int64_t traj_id0, int n_traj, int n_rows, double *out);
 int tg_philox_u32(tg_handle *h, uint64_t seed, uint32_t first, uint32_t block, int n, uint32_t *out);
 
@@ -300,6 +331,19 @@ int tg_openloop_type1_host(tg_handle *h, int B, int T, const double *x0, const t
                            int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes);
 int tg_openloop_type2_host(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
                            int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes);
+/* the same with trajectory b's ground truth integrated with the vehicle plant[b][TG_NPARAMS] (generation_type1.py:70-84,
+ * generation_type2.py:180-187; NULL = the functions above; see tg_check_plant_params).  The control synthesis is unchanged;
+ * type 2's shadow simulation reads the plant's state, so its controls follow the row's vehicle. */
+int tg_openloop_type1_params(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules, uint64_t ctrl_seed_base,
+                             int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes);
+int tg_openloop_type2_params(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
+                             int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes);
+int tg_openloop_type1_params_host(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules,
+                                  uint64_t ctrl_seed_base, int64_t traj_id0, const double *plant, double *clean, double *noisy,
+                                  double *U, int8_t *modes);
+int tg_openloop_type2_params_host(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules,
+                                  uint64_t ctrl_seed_base, int64_t traj_id0, const double *plant, double *clean, double *noisy,
+                                  double *U, int8_t *modes);
 
 /* ---- estimator-side physics (SURVEY.md section 8(f) rank 4): KalmanNet's prior step, fused.  DEVICE pointers (e.g. the
  * data_ptr() of torch CUDA tensors), dtype 0 = fp64, 1 = fp32 (torch's default, what the reference runs in); Ts and the

@@ -7,7 +7,7 @@ marshals arrays; the arithmetic runs in hand-written CUDA kernels behind the C A
 """
 from . import _lib
 from ._lib import TrajgenError, build, CTRL_SPEC_DTYPE
-from .mpc import (BatchedMPC, Params, mpc_step, make_config, check_ctrl_table, MODEL_MPC, MODEL_GEN1, MODEL_GEN2, PLANT_MPC,
+from .mpc import (BatchedMPC, Params, mpc_step, make_config, check_ctrl_table, check_plant_table, MODEL_MPC, MODEL_GEN1, MODEL_GEN2, PLANT_MPC,
                   PLANT_GEN1, PLANT_GEN2, JAC_ANALYTIC, JAC_FD)
 from .generation import (ClosedLoopGenerator, Scenarios, scenario_rules, PATH_ARC, d_steady_state, sample_x0, to_frames, write_csv, merge_datasets,
                          to_loader_tensors, PATH_PARABOLA, PATH_SINE, PATH_SPLINE, VREF_HOLD, VREF_CONST, VREF_RAMP,

@@ -94,7 +94,9 @@ EXPORTS = (
     "tg_last_error", "tg_version", "tg_default_config", "tg_create", "tg_destroy", "tg_set_stream", "tg_synchronize",
     "tg_kernel_launches", "tg_info", "tg_tyre_table_info", "tg_linearize", "tg_assemble", "tg_mpc_step", "tg_mpc_step_host",
     "tg_mpc_step_ctrl", "tg_mpc_step_ctrl_host", "tg_check_ctrl", "tg_ref_window",
-    "tg_closed_loop", "tg_closed_loop_host", "tg_closed_loop_ctrl", "tg_closed_loop_ctrl_host", "tg_default_scenario_rules", "tg_make_scenarios", "tg_make_scenarios_host", "tg_default_type1_rules", "tg_default_type2_rules", "tg_openloop_type1",
+    "tg_closed_loop", "tg_closed_loop_host", "tg_closed_loop_ctrl", "tg_closed_loop_ctrl_host", "tg_check_plant_params",
+    "tg_closed_loop_params", "tg_closed_loop_params_host", "tg_plant_rollout_params", "tg_openloop_type1_params",
+    "tg_openloop_type2_params", "tg_openloop_type1_params_host", "tg_openloop_type2_params_host", "tg_default_scenario_rules", "tg_make_scenarios", "tg_make_scenarios_host", "tg_default_type1_rules", "tg_default_type2_rules", "tg_openloop_type1",
     "tg_openloop_type2", "tg_openloop_type1_host", "tg_openloop_type2_host", "tg_write_csv", "tg_merge_csv", "tg_estimator_step", "tg_estimator_step_vjp",
     "tg_estimator_rollout", "tg_plant_rollout", "tg_sensor_noise", "tg_philox_u32", "tg_fma_peak",
     "tg_device_count", "tg_malloc", "tg_malloc_on", "tg_free", "tg_memcpy_h2d", "tg_memcpy_d2h", "tg_malloc_host", "tg_free_host",
@@ -152,6 +154,10 @@ def load():
     L.tg_closed_loop_host.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, i64, vp, i64, i64, vp, vp, vp, vp, vp]
     L.tg_closed_loop_ctrl.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp]
     L.tg_closed_loop_ctrl_host.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, i64, vp, i64, i64, vp, vp, vp, vp, vp]
+    L.tg_check_plant_params.argtypes = [ctypes.c_int, vp]
+    L.tg_closed_loop_params.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp]
+    L.tg_closed_loop_params_host.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp, i64, vp, i64, i64, vp, vp, vp,
+                                             vp, vp]
     L.tg_default_scenario_rules.argtypes = [ctypes.POINTER(TgScenarioRules)]
     L.tg_default_scenario_rules.restype = None
     L.tg_make_scenarios.argtypes = [vp, ctypes.c_int, i64, ctypes.POINTER(TgScenarioRules), vp, vp, vp, vp, vp]
@@ -163,6 +169,8 @@ def load():
     for name, rules in (("tg_openloop_type1", TgType1Rules), ("tg_openloop_type2", TgType2Rules)):
         for suffix in ("", "_host"):
             getattr(L, name + suffix).argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(rules), u64, i64, vp, vp, vp, vp]
+            getattr(L, name + "_params" + suffix).argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, ctypes.POINTER(rules), u64, i64, vp,
+                                                             vp, vp, vp, vp]
     L.tg_write_csv.argtypes = [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int, ctypes.c_int, d, i64, vp, vp, vp, ctypes.c_int, ctypes.c_int]
     L.tg_merge_csv.argtypes = [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, i64, ctypes.POINTER(i64), ctypes.POINTER(i64)]
     L.tg_estimator_step.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, ctypes.POINTER(TgStateLimits), vp]
@@ -170,6 +178,7 @@ def load():
     L.tg_estimator_rollout.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp,
                                        ctypes.POINTER(TgStateLimits), vp, ctypes.POINTER(i32)]
     L.tg_plant_rollout.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp]
+    L.tg_plant_rollout_params.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp]
     L.tg_sensor_noise.argtypes = [vp, i64, ctypes.c_int, ctypes.c_int, vp]
     L.tg_philox_u32.argtypes = [vp, u64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, vp]
     L.tg_fma_peak.argtypes = [vp, ctypes.c_int, ctypes.POINTER(d)]

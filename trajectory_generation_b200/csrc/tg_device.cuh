@@ -99,12 +99,13 @@ __device__ __noinline__ void tg_f_cont(const double *__restrict__ p, int variant
     }
 }
 
-// plant step: x <- x + Ts f(x,u) (+ clipping for the generator plants)
-__device__ __forceinline__ void tg_plant_step(const DevCfg &c, double x[6], double d, double delta)
+// plant step: x <- x + Ts f(x,u) (+ clipping for the generator plants) for the vehicle p (the handle's c.p or a row of a
+// per-trajectory plant table); c supplies Ts and the plant variant
+__device__ __forceinline__ void tg_plant_step(const DevCfg &c, const double *p, double x[6], double d, double delta)
 {
     double sd, cd, f[6];
     TG_SINCOS(delta, sd, cd);
-    tg_f_cont(c.p, c.plant, x, d, delta, sd, cd, f);
+    tg_f_cont(p, c.plant, x, d, delta, sd, cd, f);
 #pragma unroll
     for (int i = 0; i < 6; ++i) x[i] = x[i] + c.Ts * f[i];
     if (c.plant != TG_PLANT_MPC) {
@@ -270,23 +271,25 @@ __device__ __forceinline__ void tg_rotate_small(double &sp, double &cp, double d
 // the caller.  GEN1 leaves the rear slip angle unclamped (generation_type1.py:46): inside the clamp interval the table still
 // applies, outside it that lane evaluates atan / sin.
 // aux (optional, shared memory) receives {alpha_f raw, alpha_r raw, sin phi, cos phi} for the linearisation.
-__device__ __forceinline__ void tg_f_cont_tab(const DevCfg &c, int variant, const double x[6], double d, double delta,
-                                              double sd, double cd, double sp, double cp, int lane, double f[6],
-                                              double *aux = nullptr)
+// p, inv_m = 1/m, inv_Iz = 1/Iz: the vehicle; tyre_tab / atan_tab: the handle's tables (c.tab_scale is their scale), which
+// only serve a vehicle whose B, C and maxAlpha are the handle's (tg_plant_row_tables).  atan_tab may be null.
+__device__ __forceinline__ void tg_f_cont_tab(const DevCfg &c, const double *__restrict__ p, double inv_m, double inv_Iz,
+                                              const double *__restrict__ tyre_tab, const double *__restrict__ atan_tab, int variant,
+                                              const double x[6], double d, double delta, double sd, double cd, double sp, double cp,
+                                              int lane, double f[6], double *aux = nullptr)
 {
-    const double *__restrict__ p = c.p;
     const int rear = lane & 1, base = lane & ~1;
     const double vx = x[3], vy = x[4], om = x[5];
     const double vmag = fmax(fabs(vx), p[P_vx_zero]);
     const double vx_eff = (variant == TG_MODEL_MPC) ? (double)((vx > 0.0) - (vx < 0.0)) * vmag : vmag;
     const double nl = rear ? (om * p[P_lr] - vy) : (om * p[P_lf] + vy);
-    const double at = tg_slip_atan(c.atan_tab, nl, vx_eff);
+    const double at = tg_slip_atan(atan_tab, nl, vx_eff);
     const double alpha_raw = rear ? at : (-at + delta);
     const bool free_rear = rear && variant == TG_MODEL_GEN1;
     const double alpha = free_rear ? alpha_raw : tg_clamp(alpha_raw, -p[P_maxAlpha], p[P_maxAlpha]);
     double g, dg;
     if (free_rear && fabs(alpha) > p[P_maxAlpha]) g = tg_sin(p[P_Cr] * tg_atan(p[P_Br] * alpha));
-    else tg_tyre_tab(c.tyre_tab + rear * (TG_TAB_ROWS * TG_TAB_NC), alpha, p[P_maxAlpha], c.tab_scale, g, dg);
+    else tg_tyre_tab(tyre_tab + rear * (TG_TAB_ROWS * TG_TAB_NC), alpha, p[P_maxAlpha], c.tab_scale, g, dg);
     const double F = (rear ? p[P_Dr] : p[P_Df]) * g;
     if (aux && lane < 2) { aux[rear] = alpha_raw; aux[2 + rear] = rear ? cp : sp; }
     const double Fyf = __shfl_sync(0xffffffffu, F, base), Fyr = __shfl_sync(0xffffffffu, F, base + 1);
@@ -297,9 +300,9 @@ __device__ __forceinline__ void tg_f_cont_tab(const DevCfg &c, int variant, cons
     f[1] = vx * sp + vy * cp;
     f[2] = om;
     if (variant == TG_MODEL_MPC) {
-        f[3] = c.inv_m * (Frx - Fyf * sd + m * vy * om);       // (1.0/m) * (...), MPC/mpc_6stati.py:67
-        f[4] = c.inv_m * (Fyr + Fyf * cd - m * vx * om);
-        f[5] = c.inv_Iz * (Fyf * p[P_lf] * cd - Fyr * p[P_lr]);
+        f[3] = inv_m * (Frx - Fyf * sd + m * vy * om);       // (1.0/m) * (...), MPC/mpc_6stati.py:67
+        f[4] = inv_m * (Fyr + Fyf * cd - m * vx * om);
+        f[5] = inv_Iz * (Fyf * p[P_lf] * cd - Fyr * p[P_lr]);
     } else {
         f[3] = (Frx - Fyf * sd + m * vy * om) / m;
         f[4] = (Fyr + Fyf * cd - m * vx * om) / m;
@@ -373,17 +376,31 @@ __device__ __forceinline__ void tg_roll_stage(const DevCfg &c, const TgRoll &k, 
     om = fma(k.Ts_iI5f, Fyf, fma(-k.Ts_iI5r, Fyr, om));
 }
 
-// plant step by a whole warp (see tg_f_cont_lanes)
-__device__ __forceinline__ void tg_plant_step_lanes(const DevCfg &c, double x[6], double d, double delta, int lane)
+// Which tables a row of a per-trajectory plant table (p = the row) may use: the handle's, when the row's tyre constants Bf, Cf,
+// Br, Cr and maxAlpha equal the handle's bit for bit (the tables are fitted and verified for those constants only); none
+// otherwise, and none when the handle has none -- the row's plant then evaluates atan2 / atan / sin with libdevice, as a handle
+// without tables does.  Either way row b computes what a handle created with params = row b computes.
+__device__ __forceinline__ bool tg_plant_row_tables(const DevCfg &c, const double *__restrict__ p)
+{
+    if (!c.tyre_tab) return false;
+    auto same = [&](int i) { return __double_as_longlong(p[i]) == __double_as_longlong(c.p[i]); };
+    return same(P_Bf) && same(P_Cf) && same(P_Br) && same(P_Cr) && same(P_maxAlpha);
+}
+
+// plant step by a whole warp (see tg_f_cont_lanes) for the vehicle p with 1/m, 1/Iz and the tables tyre_tab / atan_tab
+// (null: libdevice)
+__device__ __forceinline__ void tg_plant_step_lanes(const DevCfg &c, const double *__restrict__ p, double inv_m, double inv_Iz,
+                                                    const double *tyre_tab, const double *atan_tab, double x[6], double d,
+                                                    double delta, int lane)
 {
     double sd, cd, f[6];
     TG_SINCOS(delta, sd, cd);
-    if (c.tyre_tab) {
+    if (tyre_tab) {
         double sp, cp;
         TG_SINCOS(x[2], sp, cp);
-        tg_f_cont_tab(c, c.plant, x, d, delta, sd, cd, sp, cp, lane, f);
+        tg_f_cont_tab(c, p, inv_m, inv_Iz, tyre_tab, atan_tab, c.plant, x, d, delta, sd, cd, sp, cp, lane, f);
     } else {
-        tg_f_cont_lanes(c.p, c.inv_m, c.inv_Iz, c.plant, x, d, delta, sd, cd, lane, f);
+        tg_f_cont_lanes(p, inv_m, inv_Iz, c.plant, x, d, delta, sd, cd, lane, f);
     }
 #pragma unroll
     for (int i = 0; i < 6; ++i) x[i] = x[i] + c.Ts * f[i];
@@ -395,21 +412,23 @@ __device__ __forceinline__ void tg_plant_step_lanes(const DevCfg &c, double x[6]
 
 // Plant step of the generator plants (TG_PLANT_GEN1 / GEN2) by ONE thread, for the open-loop kernels where a thread owns
 // a trajectory.  vx_eff = max(|vx|, vx_zero) > 0 there (generation_type1.py:41), so atan2(y, vx_eff) = atan(y / vx_eff),
-// and the tyre curve comes from the handle's table wherever the slip angle lies inside the clamp interval (always for
-// the front tyre and for GEN2's rear tyre; GEN1 leaves the rear angle free, :46, and falls back to atan / sin outside).
-__device__ __forceinline__ void tg_plant_step_gen(const DevCfg &c, double x[6], double d, double delta)
+// and the tyre curve comes from the table (tyre_tab: the handle's, or null for libdevice; pv: the vehicle) wherever the slip
+// angle lies inside the clamp interval (always for the front tyre and for GEN2's rear tyre; GEN1 leaves the rear angle free,
+// :46, and falls back to atan / sin outside).
+__device__ __forceinline__ void tg_plant_step_gen(const DevCfg &c, const double *pv, const double *tyre_tab,
+                                                  const double *atan_tab, double x[6], double d, double delta)
 {
-    const double *__restrict__ p = c.p;
+    const double *__restrict__ p = pv;
     const double vx = x[3], vy = x[4], om = x[5];
     const double ma = p[P_maxAlpha];
     const double vmag = fmax(fabs(vx), p[P_vx_zero]);
-    const double af = tg_clamp(delta - tg_slip_atan(c.atan_tab, om * p[P_lf] + vy, vmag), -ma, ma);
-    double ar = tg_slip_atan(c.atan_tab, om * p[P_lr] - vy, vmag);
+    const double af = tg_clamp(delta - tg_slip_atan(atan_tab, om * p[P_lf] + vy, vmag), -ma, ma);
+    double ar = tg_slip_atan(atan_tab, om * p[P_lr] - vy, vmag);
     if (c.plant != TG_PLANT_GEN1) ar = tg_clamp(ar, -ma, ma);
     double gf, gr, dg;
-    if (c.tyre_tab) {
-        tg_tyre_tab(c.tyre_tab, af, ma, c.tab_scale, gf, dg);
-        if (fabs(ar) <= ma) tg_tyre_tab(c.tyre_tab + TG_TAB_ROWS * TG_TAB_NC, ar, ma, c.tab_scale, gr, dg);
+    if (tyre_tab) {
+        tg_tyre_tab(tyre_tab, af, ma, c.tab_scale, gf, dg);
+        if (fabs(ar) <= ma) tg_tyre_tab(tyre_tab + TG_TAB_ROWS * TG_TAB_NC, ar, ma, c.tab_scale, gr, dg);
         else gr = tg_sin(p[P_Cr] * tg_atan(p[P_Br] * ar));
     } else {
         gf = tg_sin(p[P_Cf] * tg_atan(p[P_Bf] * af));

@@ -232,6 +232,7 @@ struct OpenLoopArgs {
     unsigned long long ctrl_seed_base;
     double *clean, *noisy, *U;
     signed char *modes;      // type 1: [B]; type 2: [B][T]; may be null
+    const double *plant;     // [B][TG_NPARAMS] per-trajectory plant parameters, read by the PT instances only; null = c.p
 };
 
 // cooperative write-out of rows [r0, r0 + TG_OL_CHUNK) of the warp's 32 trajectories (b0 = first trajectory)
@@ -266,7 +267,10 @@ __device__ __forceinline__ void tg_ol_flush(const DevCfg &c, const OpenLoopArgs 
     }
 }
 
-template <int KIND, typename Rules>   // KIND 1 = generation_type1, 2 = generation_type2
+// KIND 1 = generation_type1, 2 = generation_type2.  PT = true: trajectory b integrates its plant with the row a.plant[b]
+// (read from global memory at every step; L1 keeps it) and the tables tg_plant_row_tables gives it.  PT = false reads the
+// handle's parameters from the constant bank, as the kernel did before plant tables existed (DESIGN.md section 3).
+template <int KIND, typename Rules, bool PT = false>
 __global__ void __launch_bounds__(32 * TG_OL_WARPS) tg_openloop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Rules rules,
                                                                      const OpenLoopArgs a)
 {
@@ -282,6 +286,8 @@ __global__ void __launch_bounds__(32 * TG_OL_WARPS) tg_openloop_kernel(const __g
     double x[6];
 #pragma unroll
     for (int i = 0; i < 6; ++i) x[i] = a.x0[6 * (size_t)(live ? b : b0) + i];
+    const double *__restrict__ pv = PT ? a.plant + (size_t)(live ? b : b0) * TG_NPARAMS : nullptr;
+    const bool row_tab = PT && tg_plant_row_tables(c, pv);
     Type1Thread s1;
     Type2Thread s2;
     if constexpr (KIND == 1) {
@@ -308,8 +314,13 @@ __global__ void __launch_bounds__(32 * TG_OL_WARPS) tg_openloop_kernel(const __g
                 }
                 col[6 * TG_OL_STRIDE] = d_cmd;
                 col[7 * TG_OL_STRIDE] = delta_cmd;
-                if (c.plant == TG_PLANT_MPC) tg_plant_step(c, x, d_cmd, delta_cmd);
-                else tg_plant_step_gen(c, x, d_cmd, delta_cmd);
+                if constexpr (PT) {
+                    if (c.plant == TG_PLANT_MPC) tg_plant_step(c, pv, x, d_cmd, delta_cmd);
+                    else tg_plant_step_gen(c, pv, row_tab ? c.tyre_tab : nullptr, row_tab ? c.atan_tab : nullptr, x, d_cmd, delta_cmd);
+                } else {
+                    if (c.plant == TG_PLANT_MPC) tg_plant_step(c, c.p, x, d_cmd, delta_cmd);
+                    else tg_plant_step_gen(c, c.p, c.tyre_tab, c.atan_tab, x, d_cmd, delta_cmd);
+                }
             }
         }
         __syncwarp();

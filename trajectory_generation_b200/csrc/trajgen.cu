@@ -5,7 +5,7 @@
 //   tg_closed_loop_kernel  fused K1..K4: replaces the loop MPC/main.py:85-101 + the dataset shell
 //                          generation_type2.py:180-200 (plant clipping, sensor noise)
 //   tg_ref_window_kernel   MPC/main.py:28-47,51-68
-//   tg_plant_kernel        generation_type1.py:70-84 (open-loop integration with clipping)
+//   tg_plant_kernel        generation_type1.py:70-84 (open-loop integration with clipping; per-trajectory plant parameters)
 //   tg_noise_kernel / tg_philox_kernel   Philox4x32-10 sensor-noise stream
 //   tg_fma_peak_kernel     FMA micro-benchmark (roofline denominator)
 #include <algorithm>
@@ -57,6 +57,7 @@ struct LoopArgs {
     long long *iters_total;
     int ppc;   // problems per CTA
     const tg_ctrl_spec *ctrl;   // [B] per-trajectory settings: read by the ctrl instances only (appended last, like StepArgs::ctrl)
+    const double *plant;        // [B][TG_NPARAMS] per-trajectory plant parameters or null (appended last for the same reason)
 };
 
 // ------------------------------------------------------------------------------------------------ warp-per-problem kernels
@@ -175,7 +176,11 @@ tw_mpc_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLa
     }
 }
 
-template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0), bool CT = false>
+// PT = true: the plant instance.  Trajectory b's plant integrates the row a.plant[b] (tg_closed_loop_params); the controller
+// keeps c.p.  A template flag rather than a run-time branch: the second inlined plant step made the compile-time instances
+// spill more (N = 20: 60 / 84 B of spill stores / loads instead of 48 / 60 B), so the instances a launch without a plant table
+// runs stay as they were.
+template <int W, int S, int NC, bool P1 = false, bool HS = (NC == 0), bool CT = false, bool PT = false>
 __global__ void __launch_bounds__(TW_CTA_THREADS) __maxnreg__(tw_regs<S>())
 tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ WLayout L, const __grid_constant__ LoopArgs a)
 {
@@ -250,7 +255,15 @@ tw_closed_loop_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ 
                 double xs[6];
 #pragma unroll
                 for (int i = 0; i < 6; ++i) xs[i] = sm[LF(x0) + i];
-                tg_plant_step_lanes(c, xs, u0, u1, tid);
+                if constexpr (PT) {   // the trajectory's own plant: row b (global memory, stays in L1 / L2); the controller keeps c.p
+                    const double *__restrict__ pr = a.plant + (size_t)b * TG_NPARAMS;
+                    const bool tab = tg_plant_row_tables(c, pr);
+                    // 1.0 / m is IEEE-rounded in fp64 on the device: the inv_m / inv_Iz tg_create stores for the same m, Iz
+                    tg_plant_step_lanes(c, pr, 1.0 / pr[P_m], 1.0 / pr[P_Iz], tab ? c.tyre_tab : nullptr, tab ? c.atan_tab : nullptr,
+                                        xs, u0, u1, tid);
+                } else {
+                    tg_plant_step_lanes(c, c.p, c.inv_m, c.inv_Iz, c.tyre_tab, c.atan_tab, xs, u0, u1, tid);
+                }
                 if (tid == 0) {
                     double *clean = a.clean + ((size_t)b * (T + 1) + t + 1) * 6;
 #pragma unroll
@@ -303,16 +316,21 @@ __global__ void tg_ref_window_kernel(const __grid_constant__ DevCfg c, const __g
     }
 }
 
-__global__ void tg_plant_kernel(const __grid_constant__ DevCfg c, int B, int T, const double *x0, const double *U, double *X)
+// plant: [B][TG_NPARAMS] per-trajectory parameters or null (every trajectory integrates the handle's c.p)
+__global__ void tg_plant_kernel(const __grid_constant__ DevCfg c, int B, int T, const double *x0, const double *U,
+                                const double *plant, double *X)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
+    const double *__restrict__ pv = plant ? plant + (size_t)b * TG_NPARAMS : c.p;
+    const bool tab = plant ? tg_plant_row_tables(c, pv) : true;
+    const double *tyre_tab = tab ? c.tyre_tab : nullptr, *atan_tab = tab ? c.atan_tab : nullptr;
     double xs[6];
     double *Xo = X + (size_t)b * (T + 1) * 6;
     for (int i = 0; i < 6; ++i) { xs[i] = x0[6 * (size_t)b + i]; Xo[i] = xs[i]; }
     for (int t = 0; t < T; ++t) {
-        if (c.plant == TG_PLANT_MPC) tg_plant_step(c, xs, U[((size_t)b * T + t) * 2], U[((size_t)b * T + t) * 2 + 1]);
-        else tg_plant_step_gen(c, xs, U[((size_t)b * T + t) * 2], U[((size_t)b * T + t) * 2 + 1]);
+        if (c.plant == TG_PLANT_MPC) tg_plant_step(c, pv, xs, U[((size_t)b * T + t) * 2], U[((size_t)b * T + t) * 2 + 1]);
+        else tg_plant_step_gen(c, pv, tyre_tab, atan_tab, xs, U[((size_t)b * T + t) * 2], U[((size_t)b * T + t) * 2 + 1]);
         for (int i = 0; i < 6; ++i) Xo[6 * (size_t)(t + 1) + i] = xs[i];
     }
 }
@@ -420,6 +438,7 @@ typedef void (*TwLoopKernel)(DevCfg, WLayout, LoopArgs);
 struct TwKernels {
     TwStepKernel step, step_p1;
     TwLoopKernel loop, loop_p1;
+    TwLoopKernel loop_pt, loop_pt_p1;   // the same loop kernels with per-trajectory plant parameters (PT)
 };
 // what a launch of one set of instances needs: the kernels, the shared memory per problem, and the most problems per CTA
 // (0: one problem does not fit)
@@ -474,10 +493,12 @@ static TwKernels tw_instance()
     if constexpr (!(HS && NC > 0 && W <= 2)) {
         k.step = tw_mpc_step_kernel<W, S, NC, false, HS, CT>;
         k.loop = tw_closed_loop_kernel<W, S, NC, false, HS, CT>;
+        k.loop_pt = tw_closed_loop_kernel<W, S, NC, false, HS, CT, true>;
     }
     if constexpr (W <= 2 && (NC == 0 || HS)) {
         k.step_p1 = tw_mpc_step_kernel<W, S, NC, true, HS, CT>;
         k.loop_p1 = tw_closed_loop_kernel<W, S, NC, true, HS, CT>;
+        k.loop_pt_p1 = tw_closed_loop_kernel<W, S, NC, true, HS, CT, true>;
     }
     return k;
 }
@@ -522,7 +543,8 @@ static int make_tw_launch(const tg_handle *h, const TwKernels &k, size_t smem, T
     if (h->W > 1) p = std::min(p, TW_BAR_STEP - TW_BAR_PROB);
     while (p > 1 && (size_t)p * smem > h->smem_optin) p -= 1;
     out.ppc_max = p;
-    for (const void *f : {(const void *)k.step, (const void *)k.step_p1, (const void *)k.loop, (const void *)k.loop_p1}) {
+    for (const void *f : {(const void *)k.step, (const void *)k.step_p1, (const void *)k.loop, (const void *)k.loop_p1,
+                          (const void *)k.loop_pt, (const void *)k.loop_pt_p1}) {
         if (!f) continue;
         CK(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
         CK(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -859,6 +881,13 @@ int tg_closed_loop_ctrl(tg_handle *h, int B, int T, const double *x0, const doub
                         const tg_ctrl_spec *ctrl, const double *brk, const double *coef, int64_t traj_id0, double *clean,
                         double *noisy, double *U, int32_t *status_counts, int64_t *iters_total)
 {
+    return tg_closed_loop_params(h, B, T, x0, u0, spec, ctrl, nullptr, brk, coef, traj_id0, clean, noisy, U, status_counts, iters_total);
+}
+
+int tg_closed_loop_params(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                          const tg_ctrl_spec *ctrl, const double *plant, const double *brk, const double *coef, int64_t traj_id0,
+                          double *clean, double *noisy, double *U, int32_t *status_counts, int64_t *iters_total)
+{
     if (!h || B < 0 || T < 0 || (B > 0 && (!x0 || !u0 || !spec || !clean || !noisy || (T > 0 && !U)))) return fail(TG_ERR_INVALID, "bad argument");
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
@@ -867,16 +896,40 @@ int tg_closed_loop_ctrl(tg_handle *h, int B, int T, const double *x0, const doub
     a.B = B; a.T = T; a.x0 = x0; a.u0 = u0; a.spec = spec; a.brk = brk; a.coef = coef; a.traj_id0 = traj_id0;
     a.clean = clean; a.noisy = noisy; a.U = U; a.status_counts = status_counts; a.iters_total = (long long *)iters_total;
     a.ctrl = ctrl;
-    const TwLaunch &t = ctrl ? h->tw_ctrl : h->tw;
-    return launch_tw(h, t, t.k.loop, t.k.loop_p1, a);
+    a.plant = plant;
+    const TwLaunch &t = ctrl ? h->tw_ctrl : h->tw;   // a plant table alone keeps the handle's own (compile-time-horizon) instances
+    return plant ? launch_tw(h, t, t.k.loop_pt, t.k.loop_pt_p1, a) : launch_tw(h, t, t.k.loop, t.k.loop_p1, a);
+}
+
+// the rules of a plant table (include/trajgen.h): TG_ERR_INVALID naming the first bad row and field
+int tg_check_plant_params(int B, const double *plant)
+{
+    static const char *const names[TG_NPARAMS] = {"Cm1", "Cm2", "Cr0", "Cr2", "Br", "Cr", "Dr", "Bf", "Cf", "Df", "m", "Iz", "lf",
+                                                  "lr", "g", "maxAlpha", "vx_zero"};
+    if (B < 0) return fail(TG_ERR_INVALID, "bad argument: B < 0");
+    if (B > 0 && !plant) return fail(TG_ERR_INVALID, "bad argument: plant is null");
+    for (int b = 0; b < B; ++b) {
+        const double *r = plant + (size_t)b * TG_NPARAMS;
+        auto bad = [&](int i, const char *why) { return fail(TG_ERR_INVALID, "plant row " + std::to_string(b) + ": " + names[i] + " " + why); };
+        for (int i = 0; i < TG_NPARAMS; ++i)
+            if (!std::isfinite(r[i])) return bad(i, "must be finite");
+        for (int i : {P_m, P_Iz, P_vx_zero, P_maxAlpha})
+            if (!(r[i] > 0.0)) return bad(i, "must be > 0");
+    }
+    return TG_OK;
 }
 
 int tg_plant_rollout(tg_handle *h, int B, int T, const double *x0, const double *U, double *X)
 {
+    return tg_plant_rollout_params(h, B, T, x0, U, nullptr, X);
+}
+
+int tg_plant_rollout_params(tg_handle *h, int B, int T, const double *x0, const double *U, const double *plant, double *X)
+{
     if (!h || B < 0 || T < 0 || (B > 0 && (!x0 || !X || (T > 0 && !U)))) return fail(TG_ERR_INVALID, "bad argument");
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
-    tg_plant_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(h->dc, B, T, x0, U, X);
+    tg_plant_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(h->dc, B, T, x0, U, plant, X);
     h->launches += 1;
     CK(cudaGetLastError());
     return TG_OK;
@@ -974,15 +1027,17 @@ static int openloop_check(tg_handle *h, int B, int T, const double *x0, const vo
 extern "C++" {
 template <int KIND, typename Rules>
 static int openloop_launch(tg_handle *h, int B, int T, const double *x0, const Rules &rules, uint64_t ctrl_seed_base,
-                           int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes)
+                           int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
 {
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
     OpenLoopArgs a;
     a.B = B; a.T = T; a.x0 = x0; a.traj_id0 = traj_id0; a.ctrl_seed_base = ctrl_seed_base;
-    a.clean = clean; a.noisy = noisy; a.U = U; a.modes = (signed char *)modes;
+    a.clean = clean; a.noisy = noisy; a.U = U; a.modes = (signed char *)modes; a.plant = plant;
     const int per_cta = 32 * TG_OL_WARPS;
-    tg_openloop_kernel<KIND, Rules><<<(B + per_cta - 1) / per_cta, per_cta, TG_OL_WARPS * TG_OL_TILE * sizeof(double), h->stream>>>(h->dc, rules, a);
+    const size_t smem = TG_OL_WARPS * TG_OL_TILE * sizeof(double);
+    if (plant) tg_openloop_kernel<KIND, Rules, true><<<(B + per_cta - 1) / per_cta, per_cta, smem, h->stream>>>(h->dc, rules, a);
+    else tg_openloop_kernel<KIND, Rules, false><<<(B + per_cta - 1) / per_cta, per_cta, smem, h->stream>>>(h->dc, rules, a);
     h->launches += 1;
     CK(cudaGetLastError());
     return TG_OK;
@@ -991,6 +1046,12 @@ static int openloop_launch(tg_handle *h, int B, int T, const double *x0, const R
 
 int tg_openloop_type1(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules, uint64_t ctrl_seed_base,
                       int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes)
+{
+    return tg_openloop_type1_params(h, B, T, x0, rules, ctrl_seed_base, traj_id0, nullptr, clean, noisy, U, modes);
+}
+
+int tg_openloop_type1_params(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules, uint64_t ctrl_seed_base,
+                             int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
 {
     int rc = openloop_check(h, B, T, x0, rules, clean, noisy, U);
     if (rc != TG_OK) return rc;
@@ -1005,11 +1066,17 @@ int tg_openloop_type1(tg_handle *h, int B, int T, const double *x0, const tg_typ
         const double every = std::max(1.0, std::nearbyint(r.checkpoint_s[0] / Ts));
         if (std::ceil(n_tr / every) + 1 > TG_OL_MAX_KNOTS) return fail(TG_ERR_UNSUPPORTED, "type-1 rules: more than 16 spline knots in the transient");
     }
-    return openloop_launch<1>(h, B, T, x0, r, ctrl_seed_base, traj_id0, clean, noisy, U, modes);
+    return openloop_launch<1>(h, B, T, x0, r, ctrl_seed_base, traj_id0, plant, clean, noisy, U, modes);
 }
 
 int tg_openloop_type2(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
                       int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes)
+{
+    return tg_openloop_type2_params(h, B, T, x0, rules, ctrl_seed_base, traj_id0, nullptr, clean, noisy, U, modes);
+}
+
+int tg_openloop_type2_params(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
+                             int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
 {
     int rc = openloop_check(h, B, T, x0, rules, clean, noisy, U);
     if (rc != TG_OK) return rc;
@@ -1018,7 +1085,7 @@ int tg_openloop_type2(tg_handle *h, int B, int T, const double *x0, const tg_typ
     for (int i = 0; i < 4; ++i) { if (!(r.p_modes[i] >= 0)) return fail(TG_ERR_INVALID, "type-2 rules: negative probability"); tot4 += r.p_modes[i]; }
     for (int i = 0; i < 2; ++i) { if (!(r.p_after_turn[i] >= 0)) return fail(TG_ERR_INVALID, "type-2 rules: negative probability"); tot2 += r.p_after_turn[i]; }
     if (!(tot4 > 0) || !(tot2 > 0) || !(r.seg_s[0] > 0) || r.seg_s[1] < r.seg_s[0]) return fail(TG_ERR_INVALID, "type-2 rules: bad range");
-    return openloop_launch<2>(h, B, T, x0, r, ctrl_seed_base, traj_id0, clean, noisy, U, modes);
+    return openloop_launch<2>(h, B, T, x0, r, ctrl_seed_base, traj_id0, plant, clean, noisy, U, modes);
 }
 
 // ---- estimator physics (tg_estimator.cuh)
@@ -1257,8 +1324,18 @@ int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const
                              int64_t traj_id0, double *clean, double *noisy, double *U, int32_t *status_counts,
                              int64_t *iters_total)
 {
+    return tg_closed_loop_params_host(h, B, T, x0, u0, spec, ctrl, nullptr, brk, n_breaks, coef, n_coef, traj_id0, clean, noisy, U,
+                                      status_counts, iters_total);
+}
+
+int tg_closed_loop_params_host(tg_handle *h, int B, int T, const double *x0, const double *u0, const tg_ref_spec *spec,
+                               const tg_ctrl_spec *ctrl, const double *plant, const double *brk, int64_t n_breaks,
+                               const double *coef, int64_t n_coef, int64_t traj_id0, double *clean, double *noisy, double *U,
+                               int32_t *status_counts, int64_t *iters_total)
+{
     if (!h || B < 0 || T < 0 || (B > 0 && (!x0 || !u0 || !spec || !clean || !noisy || (T > 0 && !U)))) return fail(TG_ERR_INVALID, "bad argument");
     if (ctrl) { const int rc = tg_check_ctrl(B, ctrl, bounded_states(h)); if (rc != TG_OK) return rc; }
+    if (plant) { const int rc = tg_check_plant_params(B, plant); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     {   // the scenario table is host memory here: reject what would send the device out of bounds
         const int64_t n_tab = (brk && coef) ? (n_breaks < n_coef ? n_breaks : n_coef) : 0;
@@ -1283,8 +1360,9 @@ int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const
     // of the rows after the kernel disappears.  Pageable buffers are staged through the device arena.
     double *a_cl = (double *)pinned_device_alias(clean), *a_no = (double *)pinned_device_alias(noisy), *a_U = (double *)pinned_device_alias(U);
     const bool direct = a_cl && a_no && (a_U || !s_U);
-    const size_t s_ct = ctrl ? (size_t)B * sizeof(tg_ctrl_spec) : 0;
-    const size_t total = PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + (direct ? 0 : 2 * PAD(s_cl) + PAD(s_U)) + PAD(s_sc) + PAD(s_it) + PAD(s_ct) + 4096;
+    const size_t s_ct = ctrl ? (size_t)B * sizeof(tg_ctrl_spec) : 0, s_pl = plant ? (size_t)B * TG_NPARAMS * b8 : 0;
+    const size_t total = PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + (direct ? 0 : 2 * PAD(s_cl) + PAD(s_U)) + PAD(s_sc) + PAD(s_it) + PAD(s_ct) +
+                         PAD(s_pl) + 4096;
     int rc = ensure_dstage(h, total);
     if (rc != TG_OK) return rc;
     Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
@@ -1296,11 +1374,13 @@ int tg_closed_loop_ctrl_host(tg_handle *h, int B, int T, const double *x0, const
     int32_t *d_sc = (int32_t *)ar.take(s_sc);
     long long *d_it = (long long *)ar.take(s_it);
     tg_ctrl_spec *d_ct = ctrl ? (tg_ctrl_spec *)ar.take(s_ct) : nullptr;
+    double *d_pl = plant ? (double *)ar.take(s_pl) : nullptr;
     H2D(d_x0, x0, s_x0); H2D(d_u0, u0, s_u0); H2D(d_sp, spec, s_sp);
     if (s_bk) H2D(d_bk, brk, s_bk);
     if (s_cf) H2D(d_cf, coef, s_cf);
     if (ctrl) H2D(d_ct, ctrl, s_ct);
-    rc = tg_closed_loop_ctrl(h, B, T, d_x0, d_u0, d_sp, d_ct, d_bk, d_cf, traj_id0, d_cl, d_no, d_U, d_sc, (int64_t *)d_it);
+    if (plant) H2D(d_pl, plant, s_pl);
+    rc = tg_closed_loop_params(h, B, T, d_x0, d_u0, d_sp, d_ct, d_pl, d_bk, d_cf, traj_id0, d_cl, d_no, d_U, d_sc, (int64_t *)d_it);
     if (rc != TG_OK) return rc;
     if (!direct) {
         D2H(clean, d_cl, s_cl); D2H(noisy, d_no, s_cl);
@@ -1337,15 +1417,17 @@ int tg_make_scenarios_host(tg_handle *h, int B, int64_t traj_id0, const tg_scena
 
 extern "C++" {
 template <typename Rules, typename Fn>
-static int openloop_host(tg_handle *h, int B, int T, const double *x0, const Rules *rules, double *clean, double *noisy, double *U,
-                         int8_t *modes, size_t n_modes, Fn &&run)
+static int openloop_host(tg_handle *h, int B, int T, const double *x0, const Rules *rules, const double *plant, double *clean,
+                         double *noisy, double *U, int8_t *modes, size_t n_modes, Fn &&run)
 {
     if (!h || B < 0 || T < 1 || !rules || (B > 0 && !x0)) return fail(TG_ERR_INVALID, "bad argument (T >= 1 required)");
+    if (plant) { const int rc = tg_check_plant_params(B, plant); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
     const size_t b8 = sizeof(double);
     const size_t s_x0 = (size_t)B * 6 * b8, s_cl = (size_t)B * (T + 1) * 6 * b8, s_U = (size_t)B * T * 2 * b8;
-    const size_t total = PAD(s_x0) + 2 * PAD(s_cl) + PAD(s_U) + PAD(n_modes) + 4096;
+    const size_t s_pl = plant ? (size_t)B * TG_NPARAMS * b8 : 0;
+    const size_t total = PAD(s_x0) + 2 * PAD(s_cl) + PAD(s_U) + PAD(n_modes) + PAD(s_pl) + 4096;
     int rc = ensure_dstage(h, total);
     if (rc != TG_OK) return rc;
     Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
@@ -1353,8 +1435,10 @@ static int openloop_host(tg_handle *h, int B, int T, const double *x0, const Rul
     double *d_cl = clean ? (double *)ar.take(s_cl) : nullptr, *d_no = noisy ? (double *)ar.take(s_cl) : nullptr;
     double *d_U = U ? (double *)ar.take(s_U) : nullptr;
     int8_t *d_m = modes ? (int8_t *)ar.take(n_modes) : nullptr;
+    double *d_pl = plant ? (double *)ar.take(s_pl) : nullptr;
     H2D(d_x0, x0, s_x0);
-    rc = run(d_x0, d_cl, d_no, d_U, d_m);
+    if (plant) H2D(d_pl, plant, s_pl);
+    rc = run(d_x0, d_pl, d_cl, d_no, d_U, d_m);
     if (rc != TG_OK) return rc;
     if (clean) D2H(clean, d_cl, s_cl);
     if (noisy) D2H(noisy, d_no, s_cl);
@@ -1368,18 +1452,30 @@ static int openloop_host(tg_handle *h, int B, int T, const double *x0, const Rul
 int tg_openloop_type1_host(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules, uint64_t ctrl_seed_base,
                            int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes)
 {
-    return openloop_host(h, B, T, x0, rules, clean, noisy, U, modes, (size_t)(B > 0 ? B : 0),
-                         [&](double *dx, double *dc, double *dn, double *dU, int8_t *dm) {
-                             return tg_openloop_type1(h, B, T, dx, rules, ctrl_seed_base, traj_id0, dc, dn, dU, dm);
+    return tg_openloop_type1_params_host(h, B, T, x0, rules, ctrl_seed_base, traj_id0, nullptr, clean, noisy, U, modes);
+}
+
+int tg_openloop_type1_params_host(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules, uint64_t ctrl_seed_base,
+                                  int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
+{
+    return openloop_host(h, B, T, x0, rules, plant, clean, noisy, U, modes, (size_t)(B > 0 ? B : 0),
+                         [&](double *dx, double *dp, double *dc, double *dn, double *dU, int8_t *dm) {
+                             return tg_openloop_type1_params(h, B, T, dx, rules, ctrl_seed_base, traj_id0, dp, dc, dn, dU, dm);
                          });
 }
 
 int tg_openloop_type2_host(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
                            int64_t traj_id0, double *clean, double *noisy, double *U, int8_t *modes)
 {
-    return openloop_host(h, B, T, x0, rules, clean, noisy, U, modes, (size_t)(B > 0 ? B : 0) * (size_t)(T > 0 ? T : 0),
-                         [&](double *dx, double *dc, double *dn, double *dU, int8_t *dm) {
-                             return tg_openloop_type2(h, B, T, dx, rules, ctrl_seed_base, traj_id0, dc, dn, dU, dm);
+    return tg_openloop_type2_params_host(h, B, T, x0, rules, ctrl_seed_base, traj_id0, nullptr, clean, noisy, U, modes);
+}
+
+int tg_openloop_type2_params_host(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
+                                  int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
+{
+    return openloop_host(h, B, T, x0, rules, plant, clean, noisy, U, modes, (size_t)(B > 0 ? B : 0) * (size_t)(T > 0 ? T : 0),
+                         [&](double *dx, double *dp, double *dc, double *dn, double *dU, int8_t *dm) {
+                             return tg_openloop_type2_params(h, B, T, dx, rules, ctrl_seed_base, traj_id0, dp, dc, dn, dU, dm);
                          });
 }
 

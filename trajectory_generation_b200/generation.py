@@ -11,7 +11,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from .mpc import BatchedMPC, Params  # noqa: F401
+from .mpc import BatchedMPC, Params, _plant_table, _plant_arg  # noqa: F401
 
 PATH_PARABOLA, PATH_SINE, PATH_SPLINE, PATH_ARC = 0, 1, 2, 3
 VREF_HOLD, VREF_CONST, VREF_RAMP, VREF_TRAPEZOID, VREF_SINE = 0, 1, 2, 3, 4
@@ -189,6 +189,15 @@ class ClosedLoopGenerator(BatchedMPC):
     def __init__(self, device=0, warm_start=True, **kwargs):
         super().__init__(device=device, warm_start=warm_start, **kwargs)
 
+    def plant_table(self, B, **columns):
+        """A [B, 17] table of per-trajectory plant parameters for ``generate`` / ``plant_rollout`` (C-contiguous fp64, columns in
+        PARAM_ORDER).  Every row starts as this handle's ``params``; a keyword named as in PARAM_ORDER sets a column to a scalar or
+        a [B] array, e.g. ``plant_table(B, m=0.041 * rng.uniform(0.8, 1.2, B))``.  Only the plant (the ground truth) integrates
+        the table; the controller keeps the handle's model.  Rows that keep Bf, Cf, Br, Cr and maxAlpha keep the handle's tyre
+        tables; rows that change them evaluate the tyre curve with libdevice (include/trajgen.h).  Checked: raises ValueError
+        naming the first bad row and column."""
+        return _plant_table(self.cfg.params, B, columns)
+
     @staticmethod
     def alloc_result(B, T, pinned=True):
         """result buffers of one generate() call: dict(clean[B,T+1,6], noisy[B,T+1,6], U[B,T,2], status_counts[B,6],
@@ -200,7 +209,7 @@ class ClosedLoopGenerator(BatchedMPC):
     #: generate() streams batches whose result rows exceed this many bytes through two page-locked chunk buffers
     STREAM_BYTES = 1 << 30
 
-    def generate(self, x0, u0, scenarios, T, traj_id0=0, out=None, pinned=True, chunk=None, ctrl=None):
+    def generate(self, x0, u0, scenarios, T, traj_id0=0, out=None, pinned=True, chunk=None, ctrl=None, plant_params=None):
         """x0[B,6], u0[B,2], scenarios (len B), T steps -> dict(clean[B,T+1,6], noisy[B,T+1,6], U[B,T,2],
         status_counts[B,6], iters_total[B]).  Row 0 of clean is x0; noise seed = base + traj_id0 + i.
         The result arrays are page-locked by default (``pinned``), so the kernel writes its rows straight into them
@@ -209,24 +218,28 @@ class ClosedLoopGenerator(BatchedMPC):
         a batch whose rows exceed STREAM_BYTES (or any batch when ``chunk`` is given) is generated in chunks through two
         cached page-locked chunk buffers (generate_chunks) and gathered into ordinary arrays by host threads while the next
         chunk computes.  ``ctrl``: a [B] table of per-trajectory weights and bounds (``ctrl_table``), held for all T steps;
-        None = the handle's settings for every trajectory."""
+        None = the handle's settings for every trajectory.  ``plant_params``: a [B, 17] table of per-trajectory plant
+        parameters (``plant_table``): trajectory b's ground truth integrates row b while its controller keeps the handle's model;
+        None = the handle's params for every plant."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B, T = x0.shape[0], int(T)
         u0 = self._arr(np.asarray(u0, float).reshape(-1, 2), (B, 2))
         if len(scenarios) != B:
             raise ValueError("one scenario per trajectory required")
         ctrl = None if ctrl is None else self._ctrl_arg(ctrl, B)
+        plant_params = _plant_arg(plant_params, B)
         row_bytes = (2 * (T + 1) * 6 + T * 2) * 8
         if out is None and (chunk is not None or (pinned and B * row_bytes > self.STREAM_BYTES)):
-            return self._generate_streamed(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl)
+            return self._generate_streamed(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl, plant_params=plant_params)
         spec = np.ascontiguousarray(scenarios.spec)
         brk, coef = scenarios.tables()
         if out is None:
             out = self.alloc_result(B, T, pinned)
         elif out["clean"].shape != (B, T + 1, 6) or out["U"].shape != (B, T, 2):
             raise ValueError("`out` was allocated for another batch size / horizon")
-        _lib.check(_lib.load().tg_closed_loop_ctrl_host(
-            self._h, B, T, _lib.ptr(x0), _lib.ptr(u0), spec.ctypes.data, _lib.ptr(ctrl), _lib.ptr(brk) if len(brk) else None,
+        _lib.check(_lib.load().tg_closed_loop_params_host(
+            self._h, B, T, _lib.ptr(x0), _lib.ptr(u0), spec.ctypes.data, _lib.ptr(ctrl), _lib.ptr(plant_params),
+            _lib.ptr(brk) if len(brk) else None,
             len(brk), _lib.ptr(coef) if len(coef) else None, len(coef), int(traj_id0),
             _lib.ptr(out["clean"]), _lib.ptr(out["noisy"]), _lib.ptr(out["U"]), _lib.ptr(out["status_counts"]),
             _lib.ptr(out["iters_total"])))
@@ -247,17 +260,18 @@ class ClosedLoopGenerator(BatchedMPC):
             self._chunk_key = key
         return self._chunk_bufs
 
-    def generate_chunks(self, x0, u0, scenarios, T, traj_id0=0, chunk=None, ctrl=None):
+    def generate_chunks(self, x0, u0, scenarios, T, traj_id0=0, chunk=None, ctrl=None, plant_params=None):
         """Iterator over a large batch: yields (lo, hi, res) with res = the result dict of trajectories lo .. hi - 1 as views of
         one of two page-locked chunk buffers.  The GPU computes chunk k + 1 (a host thread sits in tg_closed_loop_host, which
         releases the GIL) while the caller consumes chunk k; a yielded view stays valid until the caller asks for the
-        next-but-one chunk.  ``chunk`` defaults to 8192 trajectories (1.1 GB of rows at T = 1200).  ``ctrl`` ([B] table, see
-        ``generate``) is sliced with the scenarios."""
+        next-but-one chunk.  ``chunk`` defaults to 8192 trajectories (1.1 GB of rows at T = 1200).  ``ctrl`` and
+        ``plant_params`` ([B] tables, see ``generate``) are sliced with the scenarios."""
         from concurrent.futures import ThreadPoolExecutor
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         u0 = np.ascontiguousarray(np.asarray(u0, float).reshape(-1, 2))
         B, T = x0.shape[0], int(T)
         ctrl = None if ctrl is None else self._ctrl_arg(ctrl, B)   # checked before the first chunk is launched
+        plant_params = _plant_arg(plant_params, B)
         chunk = int(chunk) if chunk else 8192
         nb = min(chunk, B)
         bufs = self._chunk_buffers(nb, T)
@@ -267,7 +281,8 @@ class ClosedLoopGenerator(BatchedMPC):
             lo = los[k]; hi = min(lo + chunk, B)
             res = {k_: v[:hi - lo] for k_, v in bufs[k % 2].items()}
             ClosedLoopGenerator.generate(self, x0[lo:hi], u0[lo:hi], scenarios.slice(lo, hi), T, traj_id0 + lo, out=res,
-                                         ctrl=None if ctrl is None else ctrl[lo:hi])
+                                         ctrl=None if ctrl is None else ctrl[lo:hi],
+                                         plant_params=None if plant_params is None else plant_params[lo:hi])
             return lo, hi, res
 
         with ThreadPoolExecutor(1) as ex:
@@ -278,12 +293,12 @@ class ClosedLoopGenerator(BatchedMPC):
                     fut = ex.submit(run, k + 1)          # into the buffer the caller released when it asked for this chunk
                 yield item
 
-    def _generate_streamed(self, x0, u0, scenarios, T, traj_id0, chunk, n_copy_threads=4, ctrl=None):
+    def _generate_streamed(self, x0, u0, scenarios, T, traj_id0, chunk, n_copy_threads=4, ctrl=None, plant_params=None):
         from concurrent.futures import ThreadPoolExecutor
         B = x0.shape[0]
         out = self.alloc_result(B, T, pinned=False)
         with ThreadPoolExecutor(n_copy_threads) as pool:
-            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl):
+            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl, plant_params=plant_params):
                 jobs = []
                 step = max(1, (hi - lo + n_copy_threads - 1) // n_copy_threads)
                 for a in range(0, hi - lo, step):        # ndarray copies release the GIL: first touch + copy on several cores
@@ -296,12 +311,13 @@ class ClosedLoopGenerator(BatchedMPC):
         return out
 
     def generate_to_csv(self, x0, u0, scenarios, T, clean_path, noisy_path, traj_id0=0, chunk=8192, keep=False, n_threads=0,
-                        csv_ids=None, ctrl=None):
+                        csv_ids=None, ctrl=None, plant_params=None):
         """generate() in chunks of ``chunk`` trajectories with the dataset files written as it goes (the reference holds
         every DataFrame in RAM and writes once at the end, generation_type2.py:166,216-218,319-322): while the GPU computes
         chunk k + 1 into one set of pinned buffers, the host formats chunk k from the other (tg_write_csv, all cores,
         appending).  ``csv_ids``: write only the first csv_ids trajectories to the files (BASELINE config 5: CSV for the
-        first 5 000 ids, the rest stays binary).  ``ctrl``: per-trajectory settings as in ``generate``.  Returns
+        first 5 000 ids, the rest stays binary).  ``ctrl``, ``plant_params``: per-trajectory tables as in ``generate`` (the
+        files do not record the plant table: the caller keeps it).  Returns
         dict(status_counts[B,6], iters_total[B]) (+ the rows if ``keep``)."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B, T = x0.shape[0], int(T)
@@ -312,7 +328,7 @@ class ClosedLoopGenerator(BatchedMPC):
         from concurrent.futures import ThreadPoolExecutor
         with ThreadPoolExecutor(1) as writer:                # one writer: chunks are appended in order
             pending = []
-            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl):
+            for lo, hi, res in self.generate_chunks(x0, u0, scenarios, T, traj_id0, chunk, ctrl=ctrl, plant_params=plant_params):
                 out["status_counts"][lo:hi] = res["status_counts"]; out["iters_total"][lo:hi] = res["iters_total"]
                 if keep:
                     for k_ in ("clean", "noisy", "U"):
@@ -354,15 +370,17 @@ class ClosedLoopGenerator(BatchedMPC):
                                              bufs[3].ptr if bufs[3] else None, int(t_index), op.ptr, ov.ptr))
         return self._from_device(op, (B, N + 1, 3)), self._from_device(ov, (B, N + 1))
 
-    def plant_rollout(self, x0, U):
-        """K4 tap: open-loop Euler integration with the configured plant (generation_type1.py:70-84)."""
+    def plant_rollout(self, x0, U, plant_params=None):
+        """K4 tap: open-loop Euler integration with the configured plant (generation_type1.py:70-84); ``plant_params``: a
+        [B, 17] table (``plant_table``) of per-trajectory vehicles, None = the handle's params."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B = x0.shape[0]
         U = np.ascontiguousarray(np.asarray(U, float))
         T = U.shape[1]
-        bx, bu = self._on_device([x0, U])
+        plant_params = _plant_arg(plant_params, B)
+        bx, bu, bp = self._on_device([x0, U, plant_params])
         oX = _lib.DeviceBuffer(B * (T + 1) * 6 * 8, self._h)
-        _lib.check(_lib.load().tg_plant_rollout(self._h, B, T, bx.ptr, bu.ptr, oX.ptr))
+        _lib.check(_lib.load().tg_plant_rollout_params(self._h, B, T, bx.ptr, bu.ptr, bp.ptr if bp else None, oX.ptr))
         return self._from_device(oX, (B, T + 1, 6))
 
     def sensor_noise_normals(self, traj_id0, n_traj, n_rows):

@@ -63,6 +63,45 @@ def make_config(Ts=0.02, N=20, params=None, q_c=6.0, q_phi=0.5, q_vx=0.5, R=None
 
 
 
+def check_plant_table(table):
+    """The rules of a per-trajectory plant table (include/trajgen.h, tg_check_plant_params) for a C-contiguous [B, 17] fp64 array
+    whose columns follow PARAM_ORDER: every entry finite, m, Iz, vx_zero and maxAlpha > 0.  Raises ValueError naming the first
+    bad row and column, as the C entry points do.  Returns the table."""
+    t = np.asarray(table)
+    if t.dtype != np.float64 or t.ndim != 2 or t.shape[1] != _lib.TG_NPARAMS or not t.flags["C_CONTIGUOUS"]:
+        raise ValueError(f"plant table: expected a C-contiguous [B, {_lib.TG_NPARAMS}] float64 array (columns in PARAM_ORDER), "
+                         f"got {t.dtype} {t.shape}")
+    L = _lib.load()
+    if L.tg_check_plant_params(t.shape[0], _lib.ptr(t)) != 0:
+        raise ValueError(L.tg_last_error().decode())
+    return table
+
+
+def _plant_table(params, B, columns):
+    """[B, 17] plant table whose rows start as ``params`` (17 values in PARAM_ORDER); columns by name take a scalar or a [B] array"""
+    B = int(B)
+    t = np.empty((B, _lib.TG_NPARAMS))
+    t[:] = np.asarray(params[:], float)
+    for k, v in columns.items():
+        if k not in _lib.PARAM_ORDER:
+            raise TypeError(f"unknown plant parameter {k!r} (names: {', '.join(_lib.PARAM_ORDER)})")
+        v = np.asarray(v, float)
+        if v.ndim > 1 or (v.ndim == 1 and v.shape[0] != B):
+            raise ValueError(f"plant parameter {k}: expected a scalar or {B} values, got shape {v.shape}")
+        t[:, _lib.PARAM_ORDER.index(k)] = v
+    return check_plant_table(t)
+
+
+def _plant_arg(table, B):
+    """a caller's plant table, checked (None stays None)"""
+    if table is None:
+        return None
+    t = np.asarray(table)
+    if t.ndim != 2 or t.shape[0] != B:
+        raise ValueError(f"plant_params: expected {B} rows, got shape {t.shape}")
+    return check_plant_table(np.ascontiguousarray(t) if t.dtype == np.float64 else t)
+
+
 def check_ctrl_table(table, bounded):
     """The rules of include/trajgen.h::tg_ctrl_spec for every row of ``table`` (CTRL_SPEC_DTYPE), checked by the library's
     tg_check_ctrl; ``bounded[6]`` says which state components the handle bounds.  Raises ValueError naming the first bad row

@@ -13,7 +13,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from .mpc import PLANT_GEN1, PLANT_GEN2, make_config
+from .mpc import PLANT_GEN1, PLANT_GEN2, make_config, _plant_table, _plant_arg
 from .generation import X0_RANGES_TYPE1, X0_RANGES_TYPE2, sample_x0
 
 TYPE1_MODES = ("straight", "sinusoid")                                # generation_type1.py:108
@@ -95,11 +95,18 @@ class OpenLoopGenerator:
         """the generator's own initial-state ranges (generation_type1.py:260-265 / generation_type2.py:171-174)."""
         return sample_x0(num_traj, seed, X0_RANGES_TYPE1 if self.kind == "type1" else X0_RANGES_TYPE2)
 
-    def generate(self, x0, T, traj_id0=0, want=("clean", "noisy", "U", "modes")):
+    def plant_table(self, B, **columns):
+        """A [B, 17] table of per-trajectory plant parameters for ``generate`` (see ClosedLoopGenerator.plant_table): rows start as
+        this handle's params, keywords named as in PARAM_ORDER set a column to a scalar or a [B] array.  Checked."""
+        return _plant_table(self.cfg.params, B, columns)
+
+    def generate(self, x0, T, traj_id0=0, want=("clean", "noisy", "U", "modes"), plant_params=None):
         """x0[B,6], T steps -> dict(clean[B,T+1,6], noisy[B,T+1,6], U[B,T,2], modes): modes[B] (type 1: 0 straight,
-        1 sinusoid) or modes[B,T] (type 2: index into TYPE2_MODES)."""
+        1 sinusoid) or modes[B,T] (type 2: index into TYPE2_MODES).  ``plant_params``: a [B, 17] table (``plant_table``) with
+        which trajectory b's ground truth is integrated; None = the handle's params."""
         x0 = np.ascontiguousarray(np.asarray(x0, float).reshape(-1, 6))
         B, T = x0.shape[0], int(T)
+        plant_params = _plant_arg(plant_params, B)
         out = {}
         if "clean" in want:
             out["clean"] = np.empty((B, T + 1, 6))
@@ -109,16 +116,18 @@ class OpenLoopGenerator:
             out["U"] = np.empty((B, T, 2))
         if "modes" in want:
             out["modes"] = np.zeros(B if self.kind == "type1" else (B, T), dtype=np.int8)
-        fn = getattr(_lib.load(), f"tg_openloop_{self.kind}_host")
+        fn = getattr(_lib.load(), f"tg_openloop_{self.kind}_params_host")
         _lib.check(fn(self._h, B, T, _lib.ptr(x0), ctypes.byref(self.rules), self.ctrl_seed_base, int(traj_id0),
-                      _lib.ptr(out.get("clean")), _lib.ptr(out.get("noisy")), _lib.ptr(out.get("U")), _lib.ptr(out.get("modes"))))
+                      _lib.ptr(plant_params), _lib.ptr(out.get("clean")), _lib.ptr(out.get("noisy")), _lib.ptr(out.get("U")), _lib.ptr(out.get("modes"))))
         return out
 
-    def generate_device(self, x0_dev, B, T, clean_dev=None, noisy_dev=None, U_dev=None, modes_dev=None, traj_id0=0):
-        """device-pointer form (asynchronous on the handle's stream): tg_openloop_type{1,2}."""
-        fn = getattr(_lib.load(), f"tg_openloop_{self.kind}")
+    def generate_device(self, x0_dev, B, T, clean_dev=None, noisy_dev=None, U_dev=None, modes_dev=None, traj_id0=0,
+                        plant_dev=None):
+        """device-pointer form (asynchronous on the handle's stream): tg_openloop_type{1,2}_params.  ``plant_dev``: device
+        pointer of a [B, 17] plant table or None; its rules (check_plant_table) are the caller's to keep."""
+        fn = getattr(_lib.load(), f"tg_openloop_{self.kind}_params")
         _lib.check(fn(self._h, int(B), int(T), x0_dev, ctypes.byref(self.rules), self.ctrl_seed_base, int(traj_id0),
-                      clean_dev, noisy_dev, U_dev, modes_dev))
+                      plant_dev, clean_dev, noisy_dev, U_dev, modes_dev))
 
     def synchronize(self):
         _lib.check(_lib.load().tg_synchronize(self._h))
