@@ -1241,10 +1241,6 @@ int tg_memcpy_d2h(tg_handle *h, void *dst, const void *src, int64_t bytes)
 }
 
 // ---- host-buffer entry points: stage through one device arena, copies on the handle's stream
-struct Arena {
-    char *base; size_t off, cap;
-    void *take(size_t bytes) { size_t o = (off + 255) & ~(size_t)255; off = o + bytes; return (off <= cap) ? base + o : nullptr; }
-};
 static int ensure_dstage(tg_handle *h, size_t bytes)
 {
     if (bytes <= h->dstage_bytes) return TG_OK;
@@ -1253,9 +1249,57 @@ static int ensure_dstage(tg_handle *h, size_t bytes)
     h->dstage_bytes = bytes;
     return TG_OK;
 }
-#define PAD(x) (((size_t)(x) + 255) & ~(size_t)255)
-#define H2D(dst, src, bytes) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->stream))
-#define D2H(dst, src, bytes) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->stream))
+
+// The buffers of one *_host call, each listed once: in() before the launch, out() after it.  stage() sizes the arena from
+// the list, points each device pointer at its slot and enqueues the host-to-device copies; finish() enqueues the
+// device-to-host copies and synchronises.  A null host pointer or zero bytes gives a null device pointer and no copy, so an
+// optional output the caller leaves out is one the kernel does not store.  Slots start on 256-byte boundaries (the open-loop
+// kernels store double2).
+extern "C++" {
+class HostStage {
+public:
+    explicit HostStage(tg_handle *h) : h_(h) {}
+    template <typename T> void in(T *&dev, const T *host, size_t bytes) { add(dev, const_cast<T *>(host), bytes, true); }
+    // alias: where the kernel stores straight into the caller's (pinned) buffer; nothing is staged or copied then
+    template <typename T> void out(T *&dev, T *host, size_t bytes, T *alias = nullptr)
+    {
+        if (alias) dev = alias;
+        else add(dev, host, bytes, false);
+    }
+    int stage()
+    {
+        const int rc = ensure_dstage(h_, end_);
+        if (rc != TG_OK) return rc;
+        for (const Buf &b : bufs_) {
+            char *p = (char *)h_->dstage + b.off;
+            b.set(b.dev, p);
+            if (b.in) CK(cudaMemcpyAsync(p, b.host, b.bytes, cudaMemcpyHostToDevice, h_->stream));
+        }
+        return TG_OK;
+    }
+    int finish()
+    {
+        for (const Buf &b : bufs_)
+            if (!b.in) CK(cudaMemcpyAsync(b.host, (char *)h_->dstage + b.off, b.bytes, cudaMemcpyDeviceToHost, h_->stream));
+        CK(cudaStreamSynchronize(h_->stream));
+        return TG_OK;
+    }
+
+private:
+    struct Buf { void *dev; void (*set)(void *, char *); void *host; size_t bytes, off; bool in; };
+    template <typename T> static void set_ptr(void *dev, char *p) { *static_cast<T **>(dev) = reinterpret_cast<T *>(p); }
+    template <typename T> void add(T *&dev, T *host, size_t bytes, bool in)
+    {
+        dev = nullptr;
+        if (!host || !bytes) return;
+        bufs_.push_back({&dev, &set_ptr<T>, host, bytes, end_, in});
+        end_ = (end_ + bytes + 255) & ~(size_t)255;
+    }
+    tg_handle *h_;
+    std::vector<Buf> bufs_;
+    size_t end_ = 0;
+};
+}  // extern "C++"
 
 int tg_mpc_step_host(tg_handle *h, int B, const double *x0, const double *u_prev, const double *path_ref, const double *vref,
                      double *u_cmd, int32_t *status, int32_t *iters, double *objective, double *U_opt, double *X_opt, double *y_opt)
@@ -1273,34 +1317,27 @@ int tg_mpc_step_ctrl_host(tg_handle *h, int B, const double *x0, const double *u
     CK(cudaSetDevice(h->device));
     const int N = h->dc.N, n = h->dc.n, m = h->dc.m;
     const size_t b8 = sizeof(double);
-    const size_t s_x0 = (size_t)B * 6 * b8, s_up = (size_t)B * 2 * b8, s_pr = (size_t)B * (N + 1) * 3 * b8, s_vr = (size_t)B * (N + 1) * b8;
-    const size_t s_uc = (size_t)B * 2 * b8, s_i = (size_t)B * 4, s_ob = (size_t)B * b8, s_U = (size_t)B * n * b8, s_X = (size_t)B * (N + 1) * 6 * b8, s_y = (size_t)B * m * b8;
-    const size_t s_ct = ctrl ? (size_t)B * sizeof(tg_ctrl_spec) : 0;
-    const size_t total = PAD(s_x0) + PAD(s_up) + PAD(s_pr) + PAD(s_vr) + PAD(s_uc) + 2 * PAD(s_i) + PAD(s_ob) + PAD(s_U) + PAD(s_X) + PAD(s_y) + PAD(s_ct) + 4096;
-    int rc = ensure_dstage(h, total);
+    double *d_x0, *d_up, *d_pr, *d_vr, *d_uc, *d_ob, *d_U, *d_X, *d_y;
+    int32_t *d_st, *d_it;
+    tg_ctrl_spec *d_ct;
+    HostStage s(h);
+    s.in(d_x0, x0, (size_t)B * 6 * b8);
+    s.in(d_up, u_prev, (size_t)B * 2 * b8);
+    s.in(d_pr, path_ref, (size_t)B * (N + 1) * 3 * b8);
+    s.in(d_vr, vref, (size_t)B * (N + 1) * b8);
+    s.in(d_ct, ctrl, (size_t)B * sizeof(tg_ctrl_spec));
+    s.out(d_uc, u_cmd, (size_t)B * 2 * b8);
+    s.out(d_st, status, (size_t)B * 4);
+    s.out(d_it, iters, (size_t)B * 4);
+    s.out(d_ob, objective, (size_t)B * b8);
+    s.out(d_U, U_opt, (size_t)B * n * b8);
+    s.out(d_X, X_opt, (size_t)B * (N + 1) * 6 * b8);
+    s.out(d_y, y_opt, (size_t)B * m * b8);
+    int rc = s.stage();
     if (rc != TG_OK) return rc;
-    Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
-    double *d_x0 = (double *)ar.take(s_x0), *d_up = (double *)ar.take(s_up), *d_pr = (double *)ar.take(s_pr);
-    double *d_vr = vref ? (double *)ar.take(s_vr) : nullptr;
-    double *d_uc = (double *)ar.take(s_uc);
-    int32_t *d_st = (int32_t *)ar.take(s_i), *d_it = (int32_t *)ar.take(s_i);
-    double *d_ob = (double *)ar.take(s_ob);
-    double *d_U = U_opt ? (double *)ar.take(s_U) : nullptr, *d_X = X_opt ? (double *)ar.take(s_X) : nullptr, *d_y = y_opt ? (double *)ar.take(s_y) : nullptr;
-    tg_ctrl_spec *d_ct = ctrl ? (tg_ctrl_spec *)ar.take(s_ct) : nullptr;
-    H2D(d_x0, x0, s_x0); H2D(d_up, u_prev, s_up); H2D(d_pr, path_ref, s_pr);
-    if (vref) H2D(d_vr, vref, s_vr);
-    if (ctrl) H2D(d_ct, ctrl, s_ct);
     rc = tg_mpc_step_ctrl(h, B, d_x0, d_up, d_pr, d_vr, d_ct, d_uc, d_st, d_it, d_ob, d_U, d_X, d_y);
     if (rc != TG_OK) return rc;
-    D2H(u_cmd, d_uc, s_uc);
-    if (status) D2H(status, d_st, s_i);
-    if (iters) D2H(iters, d_it, s_i);
-    if (objective) D2H(objective, d_ob, s_ob);
-    if (U_opt) D2H(U_opt, d_U, s_U);
-    if (X_opt) D2H(X_opt, d_X, s_X);
-    if (y_opt) D2H(y_opt, d_y, s_y);
-    CK(cudaStreamSynchronize(h->stream));
-    return TG_OK;
+    return s.finish();
 }
 
 // device alias of a pinned (cudaHostAlloc'ed / registered) host buffer, or null for pageable memory
@@ -1352,44 +1389,35 @@ int tg_closed_loop_params_host(tg_handle *h, int B, int T, const double *x0, con
     }
     CK(cudaSetDevice(h->device));
     const size_t b8 = sizeof(double);
-    const size_t s_x0 = (size_t)B * 6 * b8, s_u0 = (size_t)B * 2 * b8, s_sp = (size_t)B * sizeof(tg_ref_spec);
-    const size_t s_bk = (size_t)(n_breaks > 0 ? n_breaks : 0) * b8, s_cf = (size_t)(n_coef > 0 ? n_coef : 0) * 4 * b8;
-    const size_t s_cl = (size_t)B * (T + 1) * 6 * b8, s_U = (size_t)B * T * 2 * b8, s_sc = (size_t)B * TG_NUM_STATUS * 4, s_it = (size_t)B * 8;
+    const size_t s_cl = (size_t)B * (T + 1) * 6 * b8;
     // Rows leave the SM at ~1 GB/s (112 B per MPC step), far below what PCIe carries, so when the caller's result buffers
     // are pinned the kernel stores straight into them (posted writes overlap the computation) and the device-to-host copy
     // of the rows after the kernel disappears.  Pageable buffers are staged through the device arena.
     double *a_cl = (double *)pinned_device_alias(clean), *a_no = (double *)pinned_device_alias(noisy), *a_U = (double *)pinned_device_alias(U);
-    const bool direct = a_cl && a_no && (a_U || !s_U);
-    const size_t s_ct = ctrl ? (size_t)B * sizeof(tg_ctrl_spec) : 0, s_pl = plant ? (size_t)B * TG_NPARAMS * b8 : 0;
-    const size_t total = PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + (direct ? 0 : 2 * PAD(s_cl) + PAD(s_U)) + PAD(s_sc) + PAD(s_it) + PAD(s_ct) +
-                         PAD(s_pl) + 4096;
-    int rc = ensure_dstage(h, total);
+    const bool direct = a_cl && a_no && (a_U || T == 0);
+    double *d_x0, *d_u0, *d_bk, *d_cf, *d_cl, *d_no, *d_U, *d_pl;
+    tg_ref_spec *d_sp;
+    int32_t *d_sc;
+    int64_t *d_it;
+    tg_ctrl_spec *d_ct;
+    HostStage s(h);
+    s.in(d_x0, x0, (size_t)B * 6 * b8);
+    s.in(d_u0, u0, (size_t)B * 2 * b8);
+    s.in(d_sp, spec, (size_t)B * sizeof(tg_ref_spec));
+    s.in(d_bk, brk, (size_t)(n_breaks > 0 ? n_breaks : 0) * b8);
+    s.in(d_cf, coef, (size_t)(n_coef > 0 ? n_coef : 0) * 4 * b8);
+    s.in(d_ct, ctrl, (size_t)B * sizeof(tg_ctrl_spec));
+    s.in(d_pl, plant, (size_t)B * TG_NPARAMS * b8);
+    s.out(d_cl, clean, s_cl, direct ? a_cl : nullptr);
+    s.out(d_no, noisy, s_cl, direct ? a_no : nullptr);
+    s.out(d_U, U, (size_t)B * T * 2 * b8, direct ? a_U : nullptr);
+    s.out(d_sc, status_counts, (size_t)B * TG_NUM_STATUS * 4);
+    s.out(d_it, iters_total, (size_t)B * 8);
+    int rc = s.stage();
     if (rc != TG_OK) return rc;
-    Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
-    double *d_x0 = (double *)ar.take(s_x0), *d_u0 = (double *)ar.take(s_u0);
-    tg_ref_spec *d_sp = (tg_ref_spec *)ar.take(s_sp);
-    double *d_bk = s_bk ? (double *)ar.take(s_bk) : nullptr, *d_cf = s_cf ? (double *)ar.take(s_cf) : nullptr;
-    double *d_cl = direct ? a_cl : (double *)ar.take(s_cl), *d_no = direct ? a_no : (double *)ar.take(s_cl);
-    double *d_U = direct ? a_U : (double *)ar.take(s_U ? s_U : 8);
-    int32_t *d_sc = (int32_t *)ar.take(s_sc);
-    long long *d_it = (long long *)ar.take(s_it);
-    tg_ctrl_spec *d_ct = ctrl ? (tg_ctrl_spec *)ar.take(s_ct) : nullptr;
-    double *d_pl = plant ? (double *)ar.take(s_pl) : nullptr;
-    H2D(d_x0, x0, s_x0); H2D(d_u0, u0, s_u0); H2D(d_sp, spec, s_sp);
-    if (s_bk) H2D(d_bk, brk, s_bk);
-    if (s_cf) H2D(d_cf, coef, s_cf);
-    if (ctrl) H2D(d_ct, ctrl, s_ct);
-    if (plant) H2D(d_pl, plant, s_pl);
-    rc = tg_closed_loop_params(h, B, T, d_x0, d_u0, d_sp, d_ct, d_pl, d_bk, d_cf, traj_id0, d_cl, d_no, d_U, d_sc, (int64_t *)d_it);
+    rc = tg_closed_loop_params(h, B, T, d_x0, d_u0, d_sp, d_ct, d_pl, d_bk, d_cf, traj_id0, d_cl, d_no, d_U, d_sc, d_it);
     if (rc != TG_OK) return rc;
-    if (!direct) {
-        D2H(clean, d_cl, s_cl); D2H(noisy, d_no, s_cl);
-        if (s_U) D2H(U, d_U, s_U);
-    }
-    if (status_counts) D2H(status_counts, d_sc, s_sc);
-    if (iters_total) D2H(iters_total, d_it, s_it);
-    CK(cudaStreamSynchronize(h->stream));
-    return TG_OK;
+    return s.finish();
 }
 
 int tg_make_scenarios_host(tg_handle *h, int B, int64_t traj_id0, const tg_scenario_rules *rules, double *x0, double *u0,
@@ -1401,51 +1429,48 @@ int tg_make_scenarios_host(tg_handle *h, int B, int64_t traj_id0, const tg_scena
     if (!x0 || !u0 || !spec || !spl_breaks || !spl_coef) return fail(TG_ERR_INVALID, "null output");
     CK(cudaSetDevice(h->device));
     const size_t P = (size_t)rules->spl_knots - 1;
-    const size_t s_x0 = (size_t)B * 48, s_u0 = (size_t)B * 16, s_sp = (size_t)B * sizeof(tg_ref_spec), s_bk = (size_t)B * P * 8, s_cf = s_bk * 4;
-    rc = ensure_dstage(h, PAD(s_x0) + PAD(s_u0) + PAD(s_sp) + PAD(s_bk) + PAD(s_cf) + 4096);
+    double *d_x0, *d_u0, *d_bk, *d_cf;
+    tg_ref_spec *d_sp;
+    HostStage s(h);
+    s.out(d_x0, x0, (size_t)B * 48);
+    s.out(d_u0, u0, (size_t)B * 16);
+    s.out(d_sp, spec, (size_t)B * sizeof(tg_ref_spec));
+    s.out(d_bk, spl_breaks, (size_t)B * P * 8);
+    s.out(d_cf, spl_coef, (size_t)B * P * 32);
+    rc = s.stage();
     if (rc != TG_OK) return rc;
-    Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
-    double *d_x0 = (double *)ar.take(s_x0), *d_u0 = (double *)ar.take(s_u0);
-    tg_ref_spec *d_sp = (tg_ref_spec *)ar.take(s_sp);
-    double *d_bk = (double *)ar.take(s_bk), *d_cf = (double *)ar.take(s_cf);
     rc = tg_make_scenarios(h, B, traj_id0, rules, d_x0, d_u0, d_sp, d_bk, d_cf);
     if (rc != TG_OK) return rc;
-    D2H(x0, d_x0, s_x0); D2H(u0, d_u0, s_u0); D2H(spec, d_sp, s_sp); D2H(spl_breaks, d_bk, s_bk); D2H(spl_coef, d_cf, s_cf);
-    CK(cudaStreamSynchronize(h->stream));
-    return TG_OK;
+    return s.finish();
 }
 
 extern "C++" {
-template <typename Rules, typename Fn>
-static int openloop_host(tg_handle *h, int B, int T, const double *x0, const Rules *rules, const double *plant, double *clean,
-                         double *noisy, double *U, int8_t *modes, size_t n_modes, Fn &&run)
+template <typename Rules>
+static int openloop_host(int (*launch)(tg_handle *, int, int, const double *, const Rules *, uint64_t, int64_t, const double *,
+                                       double *, double *, double *, int8_t *),
+                         tg_handle *h, int B, int T, const double *x0, const Rules *rules, uint64_t ctrl_seed_base,
+                         int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes,
+                         size_t n_modes)
 {
     if (!h || B < 0 || T < 1 || !rules || (B > 0 && !x0)) return fail(TG_ERR_INVALID, "bad argument (T >= 1 required)");
     if (plant) { const int rc = tg_check_plant_params(B, plant); if (rc != TG_OK) return rc; }
     if (B == 0) return TG_OK;
     CK(cudaSetDevice(h->device));
-    const size_t b8 = sizeof(double);
-    const size_t s_x0 = (size_t)B * 6 * b8, s_cl = (size_t)B * (T + 1) * 6 * b8, s_U = (size_t)B * T * 2 * b8;
-    const size_t s_pl = plant ? (size_t)B * TG_NPARAMS * b8 : 0;
-    const size_t total = PAD(s_x0) + 2 * PAD(s_cl) + PAD(s_U) + PAD(n_modes) + PAD(s_pl) + 4096;
-    int rc = ensure_dstage(h, total);
+    const size_t b8 = sizeof(double), s_cl = (size_t)B * (T + 1) * 6 * b8;
+    double *d_x0, *d_pl, *d_cl, *d_no, *d_U;
+    int8_t *d_m;
+    HostStage s(h);
+    s.in(d_x0, x0, (size_t)B * 6 * b8);
+    s.out(d_cl, clean, s_cl);
+    s.out(d_no, noisy, s_cl);
+    s.out(d_U, U, (size_t)B * T * 2 * b8);
+    s.out(d_m, modes, n_modes);
+    s.in(d_pl, plant, (size_t)B * TG_NPARAMS * b8);
+    int rc = s.stage();
     if (rc != TG_OK) return rc;
-    Arena ar{(char *)h->dstage, 0, h->dstage_bytes};
-    double *d_x0 = (double *)ar.take(s_x0);
-    double *d_cl = clean ? (double *)ar.take(s_cl) : nullptr, *d_no = noisy ? (double *)ar.take(s_cl) : nullptr;
-    double *d_U = U ? (double *)ar.take(s_U) : nullptr;
-    int8_t *d_m = modes ? (int8_t *)ar.take(n_modes) : nullptr;
-    double *d_pl = plant ? (double *)ar.take(s_pl) : nullptr;
-    H2D(d_x0, x0, s_x0);
-    if (plant) H2D(d_pl, plant, s_pl);
-    rc = run(d_x0, d_pl, d_cl, d_no, d_U, d_m);
+    rc = launch(h, B, T, d_x0, rules, ctrl_seed_base, traj_id0, d_pl, d_cl, d_no, d_U, d_m);
     if (rc != TG_OK) return rc;
-    if (clean) D2H(clean, d_cl, s_cl);
-    if (noisy) D2H(noisy, d_no, s_cl);
-    if (U) D2H(U, d_U, s_U);
-    if (modes) D2H(modes, d_m, n_modes);
-    CK(cudaStreamSynchronize(h->stream));
-    return TG_OK;
+    return s.finish();
 }
 }  // extern "C++"
 
@@ -1458,10 +1483,8 @@ int tg_openloop_type1_host(tg_handle *h, int B, int T, const double *x0, const t
 int tg_openloop_type1_params_host(tg_handle *h, int B, int T, const double *x0, const tg_type1_rules *rules, uint64_t ctrl_seed_base,
                                   int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
 {
-    return openloop_host(h, B, T, x0, rules, plant, clean, noisy, U, modes, (size_t)(B > 0 ? B : 0),
-                         [&](double *dx, double *dp, double *dc, double *dn, double *dU, int8_t *dm) {
-                             return tg_openloop_type1_params(h, B, T, dx, rules, ctrl_seed_base, traj_id0, dp, dc, dn, dU, dm);
-                         });
+    return openloop_host(tg_openloop_type1_params, h, B, T, x0, rules, ctrl_seed_base, traj_id0, plant, clean, noisy, U, modes,
+                         (size_t)(B > 0 ? B : 0));
 }
 
 int tg_openloop_type2_host(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
@@ -1473,10 +1496,8 @@ int tg_openloop_type2_host(tg_handle *h, int B, int T, const double *x0, const t
 int tg_openloop_type2_params_host(tg_handle *h, int B, int T, const double *x0, const tg_type2_rules *rules, uint64_t ctrl_seed_base,
                                   int64_t traj_id0, const double *plant, double *clean, double *noisy, double *U, int8_t *modes)
 {
-    return openloop_host(h, B, T, x0, rules, plant, clean, noisy, U, modes, (size_t)(B > 0 ? B : 0) * (size_t)(T > 0 ? T : 0),
-                         [&](double *dx, double *dp, double *dc, double *dn, double *dU, int8_t *dm) {
-                             return tg_openloop_type2_params(h, B, T, dx, rules, ctrl_seed_base, traj_id0, dp, dc, dn, dU, dm);
-                         });
+    return openloop_host(tg_openloop_type2_params, h, B, T, x0, rules, ctrl_seed_base, traj_id0, plant, clean, noisy, U, modes,
+                         (size_t)(B > 0 ? B : 0) * (size_t)(T > 0 ? T : 0));
 }
 
 }  // extern "C"
